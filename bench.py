@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the batched Gaussian-BP hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): lazaridis_2014 admixture graph, clique
 tree (17 clusters / 16 sepsets / 32 messages per calibration), full
@@ -17,7 +17,14 @@ One step =  beliefs <- factors (init_beliefs_reset_fromfactors!),
 for all B replicates of the rank.  `value` times that with the factors
 resident in HBM; `e2e` times the public host-buffer API per step:
 pinned host tip data -> H2D -> assignfactors (K1) -> calibrate -> integratebelief
--> D2H of the log-likelihoods.
+-> D2H of the log-likelihoods.  The timed region is exactly `--steps` steps.
+
+`--dump-outputs DIR` writes what the last timed step of the headline workload computed, as DIR/<name>.npy
+(float64): `loglik` [B] (per-replicate log-likelihood at the root), or for the loopy workloads `factored_energy`
+[B, 3] (average energy, approximate entropy, factored energy); with N > 1 also `gathered` [N * B], the
+per-element results of all ranks in rank order.  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.  Outputs beyond 64 MB in all are cut to a fixed, seeded sample of rows (the
+row indices in DIR/<name>_rows.npy).
 
 `--impl reference`: the reference is Julia (not in this image), so the
 reference arm is the C/OpenMP restatement of the reference's algorithm
@@ -38,6 +45,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "clique-tree calibrations/sec (batched replicates)"
 SEED = 0xB200
+DUMP_BYTES = 64 << 20
 
 
 class C2:
@@ -534,7 +542,28 @@ class Ctx:
         return [float(x) for x in t]
 
 
-def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_region_s):
+def dump_outputs(outdir, arrays):
+    """Writes every array as <outdir>/<name>.npy in float64, all files together at most DUMP_BYTES.  If the arrays
+    do not fit, each keeps a fixed, seeded sample of its rows, whose indices go to <name>_rows.npy (float64, exact
+    below 2^53)."""
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BYTES - 2 * 4096 * len(arrays)  # room for the .npy headers of two files per array
+    for name, a in arrays.items():
+        rows_path = os.path.join(outdir, name + "_rows.npy")
+        if total > budget:
+            # half the budget for the sampled rows, at most as much again for their indices (a row is >= 8 bytes)
+            keep = max(1, int(a.shape[0] * budget / (2 * total)))
+            rows = np.sort(np.random.default_rng(SEED).choice(a.shape[0], size=keep, replace=False))
+            np.save(rows_path, rows.astype(np.float64))
+            a = a[rows]
+        elif os.path.exists(rows_path):
+            os.remove(rows_path)  # left by an earlier, sampled dump: these rows are all there is now
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
+def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap):
     """One workload on this rank's GPU: device-resident arm (value, roofline), end-to-end arm (host buffers), CPU
     check on a bounded sample (rank 0 of a single-GPU run).  Returns the dict of the JSON line (rank 0) or None."""
     import pgbp_b200
@@ -682,27 +711,14 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
     for _ in range(warm):
         step()
     barrier()
-    # Inner repeats: the timed region is `steps` x `inner` passes, long enough (>= min_region_s) that one launch
-    # hiccup or a clock ramp cannot decide the number; everything below is reported per pass.
-    pe0, pe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    pe0.record(stream)
-    for _ in range(3):
-        step()
-    pe1.record(stream)
-    barrier()
-    t_probe = pe0.elapsed_time(pe1) / 3 * 1e-3
-    # (15 % margin: the three probe passes run a little slower than the steady state)
-    inner = int(min(256, max(1, np.ceil(1.15 * min_region_s / max(steps * t_probe, 1e-9)))))
-    inner = int(ctx.max_over_ranks([inner])[0])
-    nsteps = steps * inner
     sampler = ClockSampler(local) if (rank == 0 and headline) else None
     bt.launch_count(reset=True)
-    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(nsteps)]
+    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     t0 = time.perf_counter()
     e0.record(stream)
-    for k in range(nsteps):
+    for k in range(steps):
         step(evs[k])
     e1.record(stream)
     barrier()
@@ -712,7 +728,7 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
     ms_msgs = sum(a.elapsed_time(b) for a, b in evs)
     clocks = sampler.stop(t0, t1) if sampler else None
     ms_total, ms_msgs = ctx.max_over_ranks([ms_total, ms_msgs])
-    value = world * B * upe * nsteps / (ms_total * 1e-3)
+    value = world * B * upe * steps / (ms_total * 1e-3)
     st = bt.status()
     assert (st == 0).all(), "numerical failure inside the timed region"
     # the gathered vector of the LAST step: every rank's results in rank order; it must equal an NCCL all-gather of
@@ -731,12 +747,18 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
         dist.all_gather_into_tensor(ref_all, mine)  # NCCL cross-check of the peer-written window
         assert np.array_equal(ref_all.cpu().numpy().reshape(world, wld)[:, :B], win[:, :B]), "peer-gathered window != NCCL all_gather"
         gather_checked = "window of every rank == NCCL all_gather of the same values (bitwise)"
+        gathered_last = win[:, :B]
     else:
         loglik_dev = d_norms[klast][:B].cpu().numpy()
         if world > 1:
-            mine = gathered[klast].view(world, ld)[rank, :B].cpu().numpy()
-            assert np.array_equal(mine, loglik_dev)
+            gathered_last = gathered[klast].view(world, ld)[:, :B].cpu().numpy()
+            assert np.array_equal(gathered_last[rank], loglik_dev)
             gather_checked = "own slice of the NCCL-gathered vector == local result (bitwise)"
+    if headline and args.dump_outputs and rank == 0:
+        outs = {"factored_energy": d_fe.view(3, ld)[:, :B].T.cpu().numpy()} if loopy else {"loglik": loglik_dev}
+        if world > 1:
+            outs["gathered"] = gathered_last.reshape(-1)
+        dump_outputs(args.dump_outputs, outs)
 
     # ---- end-to-end arm: public host-buffer API, pinned host inputs, D2H of the result -------
     # Every step = one synchronous sequence of public calls on one batch: H2D of that step's inputs
@@ -744,7 +766,7 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
     # fit in HBM the steps alternate between batches driven by their own host threads (the ABI allows
     # distinct batches on distinct threads): the H2D / D2H of one step overlaps the kernels of the others.
     big = params if w.key == "c4" else tips
-    e2e_steps = min(nsteps, e2e_steps_cap)
+    e2e_steps = min(steps, e2e_steps_cap)
     d_params = d_tips = None  # the device-resident arm's input copies are not needed any more (c5s: 20 GB)
     step = finish = None
     torch.cuda.empty_cache()
@@ -822,7 +844,7 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
         return None
 
     # ---- roofline of the dominant kernel family (k_message*): ALGORITHMIC bytes / device time -----------
-    achieved = bytes_unit * B * nsteps / (ms_msgs * 1e-3) / 1e9
+    achieved = bytes_unit * B * steps / (ms_msgs * 1e-3) / 1e9
     traffic = None
     tp = os.path.join(ROOT, "profiles", "traffic.json")
     if os.path.exists(tp):
@@ -834,10 +856,10 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
                 "basis": "algorithmic-bytes roofline: SURVEY 8(d) bytes of every message / CUDA-event time of the message "
                          "kernels; the lazy sepset zero, L2 hits on lines written by the previous level and (c2s) shared J "
                          "rows make the DRAM traffic smaller than the algorithmic count, see dram_gbs_from_traffic",
-                "dram_gbs_from_traffic": (traffic * nsteps / (ms_msgs * 1e-3) / 1e9) if traffic else None,
+                "dram_gbs_from_traffic": (traffic * steps / (ms_msgs * 1e-3) / 1e9) if traffic else None,
                 "algorithmic_bytes_per_unit_per_element": bytes_unit,
                 "algorithmic_flops_per_unit_per_element": flops_unit,
-                "fp64_gflops_achieved": flops_unit * B * nsteps / (ms_msgs * 1e-3) / 1e9,
+                "fp64_gflops_achieved": flops_unit * B * steps / (ms_msgs * 1e-3) / 1e9,
                 "share_of_step": ms_msgs / ms_total}
 
     # ---- CPU baseline + parity of the results (rank 0, N = 1 only) -------------------------------------
@@ -857,11 +879,11 @@ def measure(w, args, ctx, steps, headline, cpu_seconds, e2e_steps_cap, min_regio
 
     line = {
         "metric": METRIC, "value": value, "unit": w.unit, "n_gpus": world, "steps": steps,
-        "warmup": warm, "ms_per_step": ms_total / nsteps, "higher_is_better": True,
+        "warmup": warm, "ms_per_step": ms_total / steps, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": make_config(w, B, world),
-        "timing": {"inner_repeats": inner, "passes_timed": nsteps, "timed_region_ms": ms_total,
-                   "note": "steps x inner_repeats passes inside one CUDA-event pair (max over ranks); ms_per_step is per pass"
+        "timing": {"passes_timed": steps, "timed_region_ms": ms_total,
+                   "note": "`steps` passes inside one CUDA-event pair (max over ranks); ms_per_step is per pass"
                            + ("; device-resident passes start from the factors resident in HBM (factor assignment, K1, is "
                               "outside this arm and inside e2e)" if w.key in ("c2", "c2s", "c3", "c3l") else "")},
         "gather": {"kind": gather_kind, "checked": gather_checked} if world > 1 else None,
@@ -896,7 +918,7 @@ def run_gpu(args):
     ctx = Ctx(args)
     t_start = time.perf_counter()
     w = WORKLOADS[args.workload]()
-    line = measure(w, args, ctx, args.steps, True, args.cpu_seconds, 10 ** 9 if args.workload in ("c2", "c2s") else 5, 0.5)
+    line = measure(w, args, ctx, args.steps, True, args.cpu_seconds, 10 ** 9 if args.workload in ("c2", "c2s") else 5)
     # The other BASELINE configurations, each measured the same way at reduced step counts, so that the driver's
     # own run holds them too (configs[3] = the north-star target: 10k-tip network, p = 8, 4,096 parameter vectors).
     others = {}
@@ -911,7 +933,7 @@ def run_gpu(args):
             ctx.torch.cuda.empty_cache()
             try:
                 ww = WORKLOADS[key]()
-                ln = measure(ww, args, ctx, k_steps, False, cpu_s, 4, 0.0)
+                ln = measure(ww, args, ctx, k_steps, False, cpu_s, 4)
                 if ctx.rank == 0:
                     others[key] = compact(ln)
                 del ww
@@ -931,7 +953,7 @@ def run_gpu(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="batch elements per GPU (default: the workload's)")
@@ -952,7 +974,13 @@ def main():
     ap.add_argument("--coop", type=int, default=None, help="medium-shape kernel: -1 auto, 1 shared-memory, 8 cooperative, 0 generic")
     ap.add_argument("--graph", type=int, default=None, help="CUDA-graph replay of calibrate (-1 auto, 0 off, 1 on)")
     ap.add_argument("--walk", type=int, default=None, help="kernel strategy override: 0 level-parallel, 1 walk kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the results of the last timed step of the "
+                    "headline workload to DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed; the reference arm has no such step")
     if args.impl == "reference":
         run_reference(args)
     else:
