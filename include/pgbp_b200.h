@@ -291,6 +291,27 @@ int32_t pgbp_integrate_device(pgbp_batch* batch, int32_t belief, double* d_mu_so
  * takes from every cluster (integratebelief! + inv(b.J), src/calibration.jl:462-463) */
 int32_t pgbp_integrate_cov(pgbp_batch* batch, int32_t belief, double* mu, double* cov, double* norm);
 
+/* Posterior (conditional) moments of variable subsets -- ancestral state reconstruction.  Query q is the marginal
+ * Gaussian of belief q_belief[q] on its scope positions q_pos[q_off[q] .. q_off[q+1]) (k_q distinct positions in
+ * [0, m), any order): mu = (J^-1 h)[pos] and cov = (J^-1)[pos, pos], i.e. integratebelief!
+ * (src/beliefupdates.jl:168-200) + inv(J) restricted to the subset, the node moments the reference reads in
+ * test/test_calibration.jl:47-105 and test/test_exactBM.jl:20-52.  Each belief is factorised once per element
+ * however many queries name it; entries are bit-identical to the same entries of pgbp_integrate_cov.  On a loopy
+ * graph the result is the belief's approximate marginal.  Sepset beliefs are allowed.
+ * mu [B][sum k_q] and cov [B][sum k_q^2] (column-major k_q x k_q per query, queries in order); cov may be NULL.
+ * Per element: J not positive definite -> status PGBP_STATUS(0x7ffffe, pivot) and NaN in every output of that
+ * belief; all-zero (J, h) -> +Inf in every mean and covariance output of that belief (integratebelief's mean;
+ * pgbp_integrate_cov leaves its covariance undefined there).
+ * PGBP_EINVAL: nq < 1, a null required pointer, a belief out of range, q_off decreasing, a position outside [0, m)
+ * or repeated within a query, or (host variant) more than 65535*32 mean or covariance columns. */
+int32_t pgbp_marginal_moments(pgbp_batch* batch, int32_t nq, const int32_t* q_belief, const int32_t* q_off,
+                              const int32_t* q_pos, double* mu, double* cov);
+/* same into device SoA arrays, enqueue only: d_mu rows [sum k_q][ld], d_cov rows [sum k_q(k_q+1)/2][ld] (query q's
+ * packed upper triangle, (r <= c) -> c(c+1)/2 + r, after those of queries < q; the layout of pgbp_device_view);
+ * d_cov may be NULL */
+int32_t pgbp_marginal_moments_device(pgbp_batch* batch, int32_t nq, const int32_t* q_belief, const int32_t* q_off,
+                                     const int32_t* q_pos, double* d_mu, double* d_cov);
+
 /* factored_energy (src/score.jl:151-154,162-182): out [B][3] =
  * (average energy, approximate entropy, factored energy) */
 int32_t pgbp_factored_energy(pgbp_batch* batch, double* out);

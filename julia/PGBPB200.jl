@@ -314,6 +314,35 @@ function integratebelief_cov!(b::BatchedClusterGraphBelief, j::Integer)
     return μ, cov, nrm
 end
 
+# (belief j, positions) queries -> 0-based C arrays (positions are 1-based here, as Julia indices)
+function _marginal_queries(queries)
+    qb = Int32[j - 1 for (j, _) in queries]
+    off = Int32[0]; pos = Int32[]
+    for (_, p) in queries
+        append!(pos, Int32.(p) .- Int32(1)); push!(off, length(pos))
+    end
+    return qb, off, pos
+end
+
+"""
+    marginal_moments!(b, queries) -> [(μ (k,B), cov (k,k,B)) per query]
+
+Posterior moments of position subsets: query `(j, positions)` (1-based belief index and 1-based scope positions) is
+the marginal of belief j on those positions, `μ = (J \\ h)[pos]`, `cov = inv(J)[pos, pos]` (`integratebelief!` +
+`inv(J)`, src/beliefupdates.jl:168-200), for every element; each belief is factorised once however many queries name
+it.  Entries equal those of `integratebelief_cov!` bit for bit.
+"""
+function marginal_moments!(b::BatchedClusterGraphBelief, queries::AbstractVector)
+    qb, off, pos = _marginal_queries(queries)
+    ks = diff(off)
+    μ = Matrix{Float64}(undef, sum(ks), b.B); cov = Matrix{Float64}(undef, sum(ks .^ 2), b.B)
+    GC.@preserve qb off pos μ cov check(ccall((:pgbp_marginal_moments, LIB), Int32,
+        (Ptr{Cvoid}, Int32, Ptr{Int32}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}),
+        b.handle, length(qb), qb, off, pos, μ, cov))
+    m0 = cumsum([0; ks]); c0 = cumsum([0; ks .^ 2])
+    return [(μ[m0[q]+1:m0[q+1], :], reshape(cov[c0[q]+1:c0[q+1], :], ks[q], ks[q], b.B)) for q in eachindex(ks)]
+end
+
 "`factored_energy(beliefs)` -> (3,B) matrix: average energy, approximate entropy, factored energy (src/score.jl:151)"
 function PGBP.factored_energy(b::BatchedClusterGraphBelief)
     out = Matrix{Float64}(undef, 3, b.B)
@@ -440,6 +469,14 @@ function calibrate_async!(b::BatchedClusterGraphBelief, schedule::AbstractVector
 end
 integratebelief_device!(b::BatchedClusterGraphBelief, j::Integer, d_norm::Ptr{Float64}, d_mu::Ptr{Float64}=Ptr{Float64}(C_NULL)) =
     check(ccall((:pgbp_integrate_device, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float64}, Ptr{Float64}), b.handle, j - 1, d_mu, d_norm))
+"`marginal_moments!` into device arrays, enqueue only: μ rows [sum k][ld], cov rows [sum k(k+1)/2][ld] (packed upper per query)"
+function marginal_moments_device!(b::BatchedClusterGraphBelief, queries::AbstractVector, d_mu::Ptr{Float64},
+                                  d_cov::Ptr{Float64}=Ptr{Float64}(C_NULL))
+    qb, off, pos = _marginal_queries(queries)
+    GC.@preserve qb off pos check(ccall((:pgbp_marginal_moments_device, LIB), Int32,
+        (Ptr{Cvoid}, Int32, Ptr{Int32}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}),
+        b.handle, length(qb), qb, off, pos, d_mu, d_cov))
+end
 factored_energy_device!(b::BatchedClusterGraphBelief, d_out::Ptr{Float64}) =
     check(ccall((:pgbp_factored_energy_device, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}), b.handle, d_out))
 "run the batch on an externally owned `cudaStream_t` (e.g. `CUDA.stream().handle`)"

@@ -78,6 +78,8 @@ SIGNATURES = {
     "pgbp_integrate": (i32, [vp, i32, P(f64), P(f64)]),
     "pgbp_integrate_device": (i32, [vp, i32, vp, vp]),
     "pgbp_integrate_cov": (i32, [vp, i32, P(f64), P(f64), P(f64)]),
+    "pgbp_marginal_moments": (i32, [vp, i32, P(i32), P(i32), P(i32), P(f64), P(f64)]),
+    "pgbp_marginal_moments_device": (i32, [vp, i32, P(i32), P(i32), P(i32), vp, vp]),
     "pgbp_factored_energy": (i32, [vp, P(f64)]),
     "pgbp_factored_energy_device": (i32, [vp, vp]),
     "pgbp_regularize_bycluster": (i32, [vp]),

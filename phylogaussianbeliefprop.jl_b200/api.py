@@ -497,6 +497,100 @@ class BatchedClusterGraphBelief:
         self.lib.check(self.lib.pgbp_integrate_cov(self.handle, j - 1, _fptr(mu), _fptr(cov), _fptr(norm)))
         return mu, cov, norm
 
+    @staticmethod
+    def _query_arrays(queries):
+        qb, off, pos = [], [0], []
+        for j, p in queries:
+            qb.append(int(j) - 1)
+            pos.extend(int(x) for x in p)
+            off.append(len(pos))
+        return _ia(qb), _ia(off), _ia(pos or [0]), off
+
+    def marginal_moments(self, queries):
+        """Posterior moments of position subsets of beliefs (pgbp_marginal_moments): `queries` is a list of
+        (belief_j, positions), 1-based belief index, 0-based positions in its scope.  Returns one (mu[B,k], cov[B,k,k])
+        per query -- mu = (J^-1 h)[pos], cov = inv(J)[pos, pos], bit-identical to those entries of
+        integratebelief_cov -- as views into one packed result.  Each belief is factorised once however many queries
+        name it.  All-zero belief: +Inf; J not positive definite: NaN and a status word for that element."""
+        (qa, qp), (oa, op), (pa, pp), off = self._query_arrays(queries)
+        ks = np.diff(off)
+        mu = np.empty((self.B, int(ks.sum())))
+        cov = np.empty((self.B, int((ks * ks).sum())))
+        self.lib.check(self.lib.pgbp_marginal_moments(self.handle, len(ks), qp, op, pp, _fptr(mu), _fptr(cov)))
+        out, m0, c0 = [], 0, 0
+        for k in ks:
+            k = int(k)
+            # column-major k x k per query
+            out.append((mu[:, m0:m0 + k], cov[:, c0:c0 + k * k].reshape(self.B, k, k).transpose(0, 2, 1)))
+            m0 += k
+            c0 += k * k
+        return out
+
+    def marginal_moments_device(self, queries, d_mu_ptr, d_cov_ptr=None):
+        """pgbp_marginal_moments_device, enqueue only: query q's mean into rows [sum_{q'<q} k_q' ...) of the device
+        array d_mu ([sum k][ld] doubles, ld of device_view()), its packed upper covariance triangle into rows
+        [sum_{q'<q} k_q'(k_q'+1)/2 ...) of d_cov ([sum k(k+1)/2][ld]); d_cov may be None."""
+        (qa, qp), (oa, op), (pa, pp), off = self._query_arrays(queries)
+        self.lib.check(self.lib.pgbp_marginal_moments_device(self.handle, len(off) - 1, qp, op, pp,
+                                                             C.c_void_p(int(d_mu_ptr)),
+                                                             C.c_void_p(int(d_cov_ptr)) if d_cov_ptr else None))
+
+    def node_queries(self):
+        """The node-family table's query of every network node with a trait in scope: [(v, traits, belief_j,
+        positions)] with v the 0-based preorder node index, `traits` its in-scope traits (0-based), belief_j its home
+        cluster node_cluster[v] (1-based) and `positions` those traits' positions in the cluster's scope (its own
+        member entry: mem_pos + t, or mem_tpos with partial scopes)."""
+        if getattr(self, "_node_queries", None) is not None:  # the family table is static: computed once per batch
+            return self._node_queries
+        fam = self.plan.families
+        if fam is None:
+            raise ValueError("node moments need the plan's node-family table (ClusterGraphPlan(families=...))")
+        p = self.plan.ntraits
+        tpos = fam.get("mem_tpos")
+        out = []
+        for v in range(int(fam["nnodes"])):
+            a = fam["mem_off"][v]  # the node's own member entry (members are listed child first)
+            if tpos is not None:
+                tp = [int(tpos[a * p + t]) for t in range(p)]
+            else:
+                base = int(fam["mem_pos"][a])
+                tp = [base + t if base >= 0 else -1 for t in range(p)]
+            traits = [t for t in range(p) if tp[t] >= 0]
+            if traits:
+                out.append((v, traits, int(fam["node_cluster"][v]) + 1, [tp[t] for t in traits]))
+        self._node_queries = out
+        return out
+
+    def node_moments(self):
+        """Posterior distribution of every network node given the data (ancestral state reconstruction):
+        (mu[B, nnodes, p], cov[B, nnodes, p, p], in_scope[nnodes, p]) from each node's home cluster (node_queries).
+        Traits out of scope are NaN (in mu and in their covariance rows and columns): every trait of a tip (observed
+        values are evidence, missing ones are integrated out of the tip's edge factor, src/beliefs.jl:833-857), a
+        trait with no data below an internal node, a fixed root.  On a loopy cluster graph the result is the home cluster's
+        approximate (belief-propagation) marginal."""
+        nq = self.node_queries()
+        n, p = int(self.plan.families["nnodes"]), self.plan.ntraits
+        mu = np.full((self.B, n, p), np.nan)
+        cov = np.full((self.B, n, p, p), np.nan)
+        ins = np.zeros((n, p), dtype=bool)
+        if nq:
+            res = self.marginal_moments([(j, pos) for _, _, j, pos in nq])
+            for (v, tr, _, _), (m, c) in zip(nq, res):
+                t = np.asarray(tr)
+                ins[v, t] = True
+                mu[:, v, t] = m
+                cv = cov[:, v]
+                cv[:, t[:, None], t[None, :]] = c
+        return mu, cov, ins
+
+    def node_moments_device(self, d_mu_ptr, d_cov_ptr=None):
+        """node_moments into device arrays, enqueue only: the rows are those of marginal_moments_device for the
+        queries of node_queries(), in that order (sum of in-scope traits rows of d_mu, sum k(k+1)/2 of d_cov)."""
+        nq = self.node_queries()
+        if not nq:
+            raise ValueError("no network node has a trait in scope")
+        self.marginal_moments_device([(j, pos) for _, _, j, pos in nq], d_mu_ptr, d_cov_ptr)
+
     def factored_energy(self):
         """-> [B,3] = (average energy, approximate entropy, factored energy)."""
         out = np.empty((self.B, 3))

@@ -16,7 +16,7 @@ LIBDIR = os.path.join(HERE, "lib")
 # translation units in parallel (pgbp_message_t0.cu with -DPGBP_T0_PART=0,1,2)
 SOURCES = [("pgbp_plan.cu", [], "pgbp_plan"), ("pgbp_batch.cu", [], "pgbp_batch"), ("pgbp_message.cu", [], "pgbp_message"),
            ("pgbp_message_medium.cu", [], "pgbp_message_medium"), ("pgbp_factors.cu", [], "pgbp_factors"),
-           ("pgbp_comm.cu", [], "pgbp_comm"),
+           ("pgbp_comm.cu", [], "pgbp_comm"), ("pgbp_marginals.cu", [], "pgbp_marginals"),
            ("pgbp_message_t0.cu", ["PGBP_T0_PART=0"], "pgbp_message_t0_0"),
            ("pgbp_message_t0.cu", ["PGBP_T0_PART=1"], "pgbp_message_t0_1"),
            ("pgbp_message_t0.cu", ["PGBP_T0_PART=2"], "pgbp_message_t0_2"),

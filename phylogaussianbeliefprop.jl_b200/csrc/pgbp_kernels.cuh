@@ -585,17 +585,11 @@ PGBP_HD void kldiv_thread(const MsgArgs& a, double* kldiv, int msg_index, int64_
   kldiv[(int64_t)md.dmsg * ld + e] = 0.5 * (-trace + quad + ld0 - ld1);
 }
 
-// integratebelief (src/beliefupdates.jl:187-200): mu = J^-1 h,
-// norm = g + (m log2pi - logdet J + h'mu)/2; all-zero (h,J) -> (Inf.., g).
+// ---- integratebelief pieces, shared by integrate_thread and marginal_thread (one arithmetic, bit-identical results)
+// Load the packed J (from stj, pitch ldj) and h of one belief into A / hv; true if every entry is zero.
 template <int MAXM>
-PGBP_HD void integrate_thread(const double* state, int32_t* status, int64_t ld, int64_t e, int64_t jslot,
-                              int64_t hslot, int64_t gslot, int M, double* mu_soa, double* norm, int64_t ld_out,
-                              double* cov_soa = nullptr, const double* stj = nullptr, int64_t ldj = 0) {
-  constexpr int NA = MAXM * (MAXM + 1) / 2;
-  double A[NA > 0 ? NA : 1];
-  double hv[MAXM > 0 ? MAXM : 1];
-  const double* st = state + e;
-  if (!stj) { stj = st; ldj = ld; }  // (shared-precision batches: J rows of the element's group, own array and pitch)
+PGBP_HD bool integrate_load(const double* st, int64_t ld, const double* stj, int64_t ldj, int64_t jslot, int64_t hslot,
+                            int M, double* A, double* hv) {
   const int SM = tri(M);
   bool zero = true;
   for (int q = 0; q < SM; q++) {
@@ -606,23 +600,16 @@ PGBP_HD void integrate_thread(const double* state, int32_t* status, int64_t ld, 
     hv[k] = st[(hslot + k) * ld];
     if (hv[k] != 0.0) zero = false;
   }
-  const double g = st[gslot * ld];
-  if (zero) {
-    if (mu_soa)
-      for (int k = 0; k < M; k++) mu_soa[k * ld_out + e] = INFINITY;
-    norm[e] = g;
-    return;
-  }
+  return zero;
+}
+// Right-looking Cholesky J = U'U in place (A keeps U with 1/U_kk on the diagonal) and forward solve U'w = h in hv.
+// Returns 0, or the 1-based pivot at which J is not positive definite.
+template <int MAXM>
+PGBP_HD int integrate_factor(double* A, double* hv, int M, double* logdet_out, double* ww_out) {
   double logdet = 0.0, ww = 0.0;
   for (int k = 0; k < M; k++) {
     const double d = A[pk(k, k)];
-    if (!(d > 0.0)) {
-      status_fail(status, e, PGBP_STATUS(0x7ffffe, k + 1));
-      if (mu_soa)
-        for (int q = 0; q < M; q++) mu_soa[q * ld_out + e] = NAN;
-      norm[e] = NAN;
-      return;
-    }
+    if (!(d > 0.0)) return k + 1;
     logdet += log(d);
     const double rinv = 1.0 / sqrt(d);
     A[pk(k, k)] = rinv;
@@ -636,32 +623,129 @@ PGBP_HD void integrate_thread(const double* state, int32_t* status, int64_t ld, 
       hv[c] = nfma(akc, wk, hv[c]);
     }
   }
-  norm[e] = g + 0.5 * ((double)M * PGBP_LOG2PI - logdet + ww);
-  if (mu_soa) {
-    for (int k = M - 1; k >= 0; k--) {  // U mu = w
-      double s = hv[k];
-      for (int c = k + 1; c < M; c++) s = nfma(A[pk(k, c)], hv[c], s);
-      hv[k] = s * A[pk(k, k)];
-      mu_soa[k * ld_out + e] = hv[k];
+  *logdet_out = logdet;
+  *ww_out = ww;
+  return 0;
+}
+// Back substitution U mu = w in place in hv; each mu_k is also stored to mu_soa row k when mu_soa is given.
+template <int MAXM>
+PGBP_HD void integrate_solve(const double* A, double* hv, int M, double* mu_soa, int64_t ld_out, int64_t e) {
+  for (int k = M - 1; k >= 0; k--) {
+    double s = hv[k];
+    for (int c = k + 1; c < M; c++) s = nfma(A[pk(k, c)], hv[c], s);
+    hv[k] = s * A[pk(k, k)];
+    if (mu_soa) mu_soa[k * ld_out + e] = hv[k];
+  }
+}
+// inv(J) = V V' with V = U^-1 (the conditional covariance that calibrate_exact_cliquetree! reads with
+// inv(b.J), src/calibration.jl:463).  In place: A holds U with 1/U_kk on the diagonal; columns
+// descending, rows descending, so column c only reads U entries of columns < c and V of column c.
+template <int MAXM>
+PGBP_HD void integrate_invert(double* A, int M) {
+  for (int c = M - 1; c >= 0; c--) {
+    for (int r = c - 1; r >= 0; r--) {
+      double s = A[pk(r, c)] * A[pk(c, c)];
+      for (int k = r + 1; k < c; k++) s = fma(A[pk(r, k)], A[pk(k, c)], s);
+      A[pk(r, c)] = -s * A[pk(r, r)];
     }
   }
+}
+// Entry (i, j), i <= j, of inv(J) = V V' from the V that integrate_invert leaves in A.
+PGBP_HD double integrate_cov_entry(const double* A, int M, int i, int j) {
+  double s = 0.0;
+  for (int k = j; k < M; k++) s = fma(A[pk(i, k)], A[pk(j, k)], s);
+  return s;
+}
+
+// integratebelief (src/beliefupdates.jl:187-200): mu = J^-1 h,
+// norm = g + (m log2pi - logdet J + h'mu)/2; all-zero (h,J) -> (Inf.., g).
+template <int MAXM>
+PGBP_HD void integrate_thread(const double* state, int32_t* status, int64_t ld, int64_t e, int64_t jslot,
+                              int64_t hslot, int64_t gslot, int M, double* mu_soa, double* norm, int64_t ld_out,
+                              double* cov_soa = nullptr, const double* stj = nullptr, int64_t ldj = 0) {
+  constexpr int NA = MAXM * (MAXM + 1) / 2;
+  double A[NA > 0 ? NA : 1];
+  double hv[MAXM > 0 ? MAXM : 1];
+  const double* st = state + e;
+  if (!stj) { stj = st; ldj = ld; }  // (shared-precision batches: J rows of the element's group, own array and pitch)
+  const bool zero = integrate_load<MAXM>(st, ld, stj, ldj, jslot, hslot, M, A, hv);
+  const double g = st[gslot * ld];
+  if (zero) {
+    if (mu_soa)
+      for (int k = 0; k < M; k++) mu_soa[k * ld_out + e] = INFINITY;
+    norm[e] = g;
+    return;
+  }
+  double logdet = 0.0, ww = 0.0;
+  const int pivot = integrate_factor<MAXM>(A, hv, M, &logdet, &ww);
+  if (pivot) {
+    status_fail(status, e, PGBP_STATUS(0x7ffffe, pivot));
+    if (mu_soa)
+      for (int q = 0; q < M; q++) mu_soa[q * ld_out + e] = NAN;
+    norm[e] = NAN;
+    return;
+  }
+  norm[e] = g + 0.5 * ((double)M * PGBP_LOG2PI - logdet + ww);
+  if (mu_soa) integrate_solve<MAXM>(A, hv, M, mu_soa, ld_out, e);
   if (cov_soa) {
-    // inv(J) = V V' with V = U^-1 (the conditional covariance that calibrate_exact_cliquetree! reads with
-    // inv(b.J), src/calibration.jl:463).  In place: A holds U with 1/U_kk on the diagonal; columns
-    // descending, rows descending, so column c only reads U entries of columns < c and V of column c.
-    for (int c = M - 1; c >= 0; c--) {
-      for (int r = c - 1; r >= 0; r--) {
-        double s = A[pk(r, c)] * A[pk(c, c)];
-        for (int k = r + 1; k < c; k++) s = fma(A[pk(r, k)], A[pk(k, c)], s);
-        A[pk(r, c)] = -s * A[pk(r, r)];
-      }
-    }
+    integrate_invert<MAXM>(A, M);
     for (int j = 0; j < M; j++)
-      for (int i = 0; i <= j; i++) {
-        double s = 0.0;
-        for (int k = j; k < M; k++) s = fma(A[pk(i, k)], A[pk(j, k)], s);
-        cov_soa[(int64_t)pk(i, j) * ld_out + e] = s;
-      }
+      for (int i = 0; i <= j; i++) cov_soa[(int64_t)pk(i, j) * ld_out + e] = integrate_cov_entry(A, M, i, j);
+  }
+}
+
+// Posterior moments of position subsets of one belief (pgbp_marginal_moments): the belief is read and factorised
+// once per element, then every query [t0, t1) of it gets mu[pos] and the packed upper triangle of inv(J)[pos, pos],
+// with the arithmetic of integrate_thread (same entries bit for bit).  qtab[4t..4t+3] = (k, offset of the positions
+// in qpos, first mu row, first covariance row).  All-zero (J, h): +Inf everywhere; J not positive definite: status
+// 0x7ffffe and NaN everywhere.
+struct MargDesc {
+  int64_t jslot, hrow;  // J slot (plan layout; the group batch's array for shared-precision batches), first h row
+  int32_t m, t0, t1, pad;
+};
+template <int MAXM>
+PGBP_HD void marginal_thread(const double* state, int32_t* status, int64_t ld, int64_t e, const MargDesc& d,
+                             const int32_t* qtab, const int32_t* qpos, double* mu_soa, double* cov_soa,
+                             int64_t ld_out, const double* stj, int64_t ldj) {
+  constexpr int NA = MAXM * (MAXM + 1) / 2;
+  double A[NA > 0 ? NA : 1];
+  double hv[MAXM > 0 ? MAXM : 1];
+  const double* st = state + e;
+  if (!stj) { stj = st; ldj = ld; }
+  const int M = d.m;
+  double fillv = INFINITY;
+  bool ok = !integrate_load<MAXM>(st, ld, stj, ldj, d.jslot, d.hrow, M, A, hv);
+  if (ok) {
+    double logdet, ww;
+    const int pivot = integrate_factor<MAXM>(A, hv, M, &logdet, &ww);
+    if (pivot) {
+      status_fail(status, e, PGBP_STATUS(0x7ffffe, pivot));
+      fillv = NAN;
+      ok = false;
+    }
+  }
+  if (!ok) {
+    for (int t = d.t0; t < d.t1; t++) {
+      const int k = qtab[4 * t];
+      for (int r = 0; r < k; r++) mu_soa[(int64_t)(qtab[4 * t + 2] + r) * ld_out + e] = fillv;
+      if (cov_soa)
+        for (int r = 0; r < tri(k); r++) cov_soa[(int64_t)(qtab[4 * t + 3] + r) * ld_out + e] = fillv;
+    }
+    return;
+  }
+  integrate_solve<MAXM>(A, hv, M, nullptr, 0, e);
+  if (cov_soa) integrate_invert<MAXM>(A, M);
+  for (int t = d.t0; t < d.t1; t++) {
+    const int k = qtab[4 * t];
+    const int32_t* pos = qpos + qtab[4 * t + 1];
+    const int64_t mr = qtab[4 * t + 2], cr = qtab[4 * t + 3];
+    for (int r = 0; r < k; r++) mu_soa[(mr + r) * ld_out + e] = hv[pos[r]];
+    if (cov_soa)
+      for (int c = 0; c < k; c++)
+        for (int r = 0; r <= c; r++) {
+          const int a = pos[r], b = pos[c];
+          cov_soa[(cr + pk(r, c)) * ld_out + e] = a <= b ? integrate_cov_entry(A, M, a, b) : integrate_cov_entry(A, M, b, a);
+        }
   }
 }
 
