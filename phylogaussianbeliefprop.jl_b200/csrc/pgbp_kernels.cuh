@@ -74,17 +74,6 @@ PGBP_HD void store_flag(const MsgArgs& a, int dmsg, int64_t e, int S, double max
   }
 }
 
-// Register-resident message kernel body, compile-time shape (I >= 1 integrated
-// out, S kept).  marginalize (src/beliefupdates.jl:55-83) -> divide! (:579-587)
-// -> mult! (:483-488) -> residual (:646-647) -> flag (src/beliefs.jl:994-1003).
-//
-// Only J_II (packed), J_IK and h_I stay in registers.  They are factorised in
-// place (right-looking U'U on the I rows): afterwards AI holds U, Bm holds
-// Z' = U^-T J_IK and hI holds w = U^-T h_I.  The kept block is then STREAMED in
-// chunks of PGBP_CHUNK packed entries: the sender's J_KK entry, the sepset's old
-// value and the receiver's old value are all loaded first (3*CHUNK independent
-// loads in flight per thread), then  new = J_KK - z_r.z_c,  delta = new - old,
-// and the three stores.  h and g follow the same pattern.
 // L2 prefetch hint (device only): starts the HBM -> L2 transfer of a line that is read later
 PGBP_HD void l2_prefetch(const void* p) {
 #if defined(__CUDA_ARCH__)
@@ -99,55 +88,95 @@ PGBP_HD double* slot_ptr(char* base, uint32_t slot, uint32_t ld8) {
   return (double*)(base + (uint64_t)slot * (uint64_t)ld8);
 }
 
-template <int CI, int CS>
-PGBP_HD void message_thread_t0(const MsgArgs& a, int msg_index, int64_t e) {
-  constexpr int I = CI, S = CS, M = I + S, SI = I * (I + 1) / 2, SS = S * (S + 1) / 2;
-  const MsgDesc md = a.msgs[msg_index];  // by value: lives in registers, never re-read after a store
-  if (a.status[e] != 0) return;
-  if (a.done && a.done[e]) return;
+// Every slot row a register-class message (I, S) reads, numbered in one fixed order: sender J in gather order
+// [FJ, FH), sender h in [I;K] order [FH, FG), sender g, receiver g, receiver J and h at the sepset's positions
+// [TJ, TH) and [TH, SG), then the old sepset g, J and h [SG, N).  The sepset rows come last because they are not
+// read under PGBP_OPT_SEPZERO: the staged kernel then stages the first SG rows only.
+template <int I, int S>
+struct T0Rows {
+  static constexpr int M = I + S, SMM = M * (M + 1) / 2, SS = S * (S + 1) / 2;
+  static constexpr int FJ = 0, FH = SMM, FG = SMM + M, TG = FG + 1, TJ = TG + 1, TH = TJ + SS, SG = TH + S,
+                       SJ = SG + 1, SH = SJ + SS, N = SH + S;
+  // slot of row n (in the unrolled body n is a compile-time constant and the branches fold away)
+  static PGBP_HD uint32_t slot(const MsgDesc& md, const int32_t* __restrict__ gat, const int32_t* __restrict__ sca, int n) {
+    if (n < FG) return (n < FH ? (uint32_t)md.fJ : (uint32_t)md.fh) + (uint32_t)gat[n];
+    if (n == FG) return (uint32_t)md.fg;
+    if (n == TG) return (uint32_t)md.tg;
+    if (n < SG) return (n < TH ? (uint32_t)md.tJ : (uint32_t)md.th) + (uint32_t)sca[n - TJ];
+    if (n == SG) return (uint32_t)md.sg;
+    return n < SH ? (uint32_t)md.sJ + (uint32_t)(n - SJ) : (uint32_t)md.sh + (uint32_t)(n - SH);
+  }
+};
+
+// Operand sources of message_body_t0: slot(n) is the slot of row n (T0Rows numbering), at(n, slot) its value for
+// this element.  T0Global reads the state array (host emulation, k_walk); the staged kernel's source reads a tile
+// staged in shared memory (pgbp_msg_t0.cuh).
+template <int I, int S>
+struct T0Global {
+  const MsgDesc& md;
+  const int32_t* __restrict__ gat;
+  const int32_t* __restrict__ sca;
+  char* st;
+  uint32_t ld8;
+  PGBP_HD uint32_t slot(int n) const { return T0Rows<I, S>::slot(md, gat, sca, n); }
+  PGBP_HD double at(int, uint32_t s) const { return *slot_ptr(st, s, ld8); }
+};
+
+// Register-resident message kernel body, compile-time shape (I >= 1 integrated
+// out, S kept).  marginalize (src/beliefupdates.jl:55-83) -> divide! (:579-587)
+// -> mult! (:483-488) -> residual (:646-647) -> flag (src/beliefs.jl:994-1003).
+//
+// Only J_II (packed), J_IK and h_I stay in registers.  They are factorised in
+// place (right-looking U'U on the I rows): afterwards AI holds U, Bm holds
+// Z' = U^-T J_IK and hI holds w = U^-T h_I.  The kept block is then STREAMED in
+// chunks of PGBP_CHUNK packed entries: the sender's J_KK entry, the sepset's old
+// value and the receiver's old value are all loaded first (3*CHUNK independent
+// loads in flight per thread), then  new = J_KK - z_r.z_c,  delta = new - old,
+// and the three stores.  h and g follow the same pattern.  Operands come from src
+// (T0Global or a staged tile); results are stored to the state array.
+template <int CI, int CS, class Src>
+PGBP_HD void message_body_t0(const MsgArgs& a, const MsgDesc& md, int64_t e, const Src& src) {
+  constexpr int I = CI, S = CS, SI = I * (I + 1) / 2, SS = S * (S + 1) / 2;
+  using R = T0Rows<I, S>;
   const uint32_t ld8 = (uint32_t)(a.ld * 8);  // (batches with 8*ld >= 2^32 are refused at creation)
   char* st = (char*)(a.state + e);
   char* rs = a.resid ? (char*)(a.resid + e) : nullptr;
-  char* stj = st;
-  const int32_t* __restrict__ gat = a.tab + md.gat;
-  const int32_t* __restrict__ sca = a.tab + md.sca;
-  const uint32_t fJ = (uint32_t)md.fJ, fh = (uint32_t)md.fh, sJ = (uint32_t)md.sJ, sh = (uint32_t)md.sh,
-                 tJ = (uint32_t)md.tJ, th = (uint32_t)md.th, rJ = (uint32_t)md.rJ, rh = (uint32_t)md.rh;
-  constexpr int SMM = M * (M + 1) / 2;
+  const uint32_t sJ = (uint32_t)md.sJ, sh = (uint32_t)md.sh, rJ = (uint32_t)md.rJ, rh = (uint32_t)md.rh;
+  auto ld = [&](int n) { return src.at(n, src.slot(n)); };
   double AI[SI > 0 ? SI : 1];
   double Bm[I * S > 0 ? I * S : 1];  // Bm[k*S + c] = J[I_k, K_c]
   double hI[I > 0 ? I : 1];
 #pragma unroll
   for (int c = 0; c < I; c++) {
 #pragma unroll
-    for (int r = 0; r <= c; r++) AI[pk(r, c)] = *slot_ptr(stj, fJ + gat[pk(r, c)], ld8);
+    for (int r = 0; r <= c; r++) AI[pk(r, c)] = ld(R::FJ + pk(r, c));
   }
 #pragma unroll
   for (int c = 0; c < S; c++) {
 #pragma unroll
-    for (int k = 0; k < I; k++) Bm[k * S + c] = *slot_ptr(stj, fJ + gat[pk(k, I + c)], ld8);
+    for (int k = 0; k < I; k++) Bm[k * S + c] = ld(R::FJ + pk(k, I + c));
   }
 #pragma unroll
-  for (int k = 0; k < I; k++) hI[k] = *slot_ptr(st, fh + gat[SMM + k], ld8);
-  double g = *slot_ptr(st, (uint32_t)md.fg, ld8);
+  for (int k = 0; k < I; k++) hI[k] = ld(R::FH + k);
+  double g = ld(R::FG);
   const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
-  const double sg_old = sz ? 0.0 : *slot_ptr(st, (uint32_t)md.sg, ld8);
-  const double tg_old = *slot_ptr(st, (uint32_t)md.tg, ld8);
+  const double sg_old = sz ? 0.0 : ld(R::SG);
+  const double tg_old = ld(R::TG);
 #ifdef PGBP_T0_PREFETCH
   // everything the streaming phase will read (kept block of the sender, old sepset, old receiver):
   // the HBM -> L2 transfers overlap the factorisation, the chunk loop then waits on L2 only
 #pragma unroll
   for (int q = 0; q < SS; q++) {
     const int c = colof(q), r = q - c * (c + 1) / 2;
-    l2_prefetch(slot_ptr(st, fJ + gat[pk(I + r, I + c)], ld8));
+    l2_prefetch(slot_ptr(st, src.slot(R::FJ + pk(I + r, I + c)), ld8));
     l2_prefetch(slot_ptr(st, sJ + q, ld8));
-    l2_prefetch(slot_ptr(st, tJ + sca[q], ld8));
+    l2_prefetch(slot_ptr(st, src.slot(R::TJ + q), ld8));
   }
 #pragma unroll
   for (int k = 0; k < S; k++) {
-    l2_prefetch(slot_ptr(st, fh + gat[SMM + I + k], ld8));
+    l2_prefetch(slot_ptr(st, src.slot(R::FH + I + k), ld8));
     l2_prefetch(slot_ptr(st, sh + k, ld8));
-    l2_prefetch(slot_ptr(st, th + sca[SS + k], ld8));
+    l2_prefetch(slot_ptr(st, src.slot(R::TH + k), ld8));
   }
 #endif
 
@@ -209,13 +238,13 @@ PGBP_HD void message_thread_t0(const MsgArgs& a, int msg_index, int64_t e) {
     constexpr int q0 = decltype(chc)::value * PGBP_CHUNK;
     constexpr int n = (SS - q0) < PGBP_CHUNK ? (SS - q0) : PGBP_CHUNK;
     double jo[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-    double* ta[PGBP_CHUNK];
+    uint32_t ta[PGBP_CHUNK];
     static_for<n>([&](auto kc) {
       constexpr int k = decltype(kc)::value, q = q0 + k, c = colof(q), r = q - c * (c + 1) / 2;
-      ta[k] = slot_ptr(st, tJ + sca[q], ld8);
-      jo[k] = *slot_ptr(st, fJ + gat[pk(I + r, I + c)], ld8);
-      so[k] = sz ? 0.0 : *slot_ptr(st, sJ + q, ld8);
-      to[k] = *ta[k];
+      ta[k] = src.slot(R::TJ + q);
+      jo[k] = ld(R::FJ + pk(I + r, I + c));
+      so[k] = sz ? 0.0 : ld(R::SJ + q);
+      to[k] = src.at(R::TJ + q, ta[k]);
     });
     static_for<n>([&](auto kc) {
       constexpr int k = decltype(kc)::value, q = q0 + k, c = colof(q), r = q - c * (c + 1) / 2;
@@ -224,20 +253,20 @@ PGBP_HD void message_thread_t0(const MsgArgs& a, int msg_index, int64_t e) {
       for (int i = 0; i < I; i++) nv = nfma(Bm[i * S + r], Bm[i * S + c], nv);
       const double d = nv - so[k];
       *slot_ptr(st, sJ + q, ld8) = nv;
-      *ta[k] = to[k] + d;
+      *slot_ptr(st, ta[k], ld8) = to[k] + d;
       if (rs) *slot_ptr(rs, rJ + q, ld8) = d;
       absmax(maxJ, d);
     });
   });
   {
     double ho[S > 0 ? S : 1], so[S > 0 ? S : 1], to[S > 0 ? S : 1];
-    double* ta[S > 0 ? S : 1];
+    uint32_t ta[S > 0 ? S : 1];
 #pragma unroll
     for (int k = 0; k < S; k++) {
-      ta[k] = slot_ptr(st, th + sca[SS + k], ld8);
-      ho[k] = *slot_ptr(st, fh + gat[SMM + I + k], ld8);
-      so[k] = sz ? 0.0 : *slot_ptr(st, sh + k, ld8);
-      to[k] = *ta[k];
+      ta[k] = src.slot(R::TH + k);
+      ho[k] = ld(R::FH + I + k);
+      so[k] = sz ? 0.0 : ld(R::SH + k);
+      to[k] = src.at(R::TH + k, ta[k]);
     }
 #pragma unroll
     for (int k = 0; k < S; k++) {
@@ -246,7 +275,7 @@ PGBP_HD void message_thread_t0(const MsgArgs& a, int msg_index, int64_t e) {
       for (int i = 0; i < I; i++) nv = nfma(Bm[i * S + k], hI[i], nv);
       const double d = nv - so[k];
       *slot_ptr(st, sh + k, ld8) = nv;
-      *ta[k] = to[k] + d;
+      *slot_ptr(st, ta[k], ld8) = to[k] + d;
       if (rs) *slot_ptr(rs, rh + k, ld8) = d;
       absmax(maxh, d);
     }
@@ -254,6 +283,16 @@ PGBP_HD void message_thread_t0(const MsgArgs& a, int msg_index, int64_t e) {
   *slot_ptr(st, (uint32_t)md.sg, ld8) = g;
   *slot_ptr(st, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
   store_flag(a, md.dmsg, e, S, maxJ, maxh);
+}
+
+// One (message, element) of the register class with operands read from global memory.
+template <int CI, int CS>
+PGBP_HD void message_thread_t0(const MsgArgs& a, int msg_index, int64_t e) {
+  const MsgDesc md = a.msgs[msg_index];  // by value: lives in registers, never re-read after a store
+  if (a.status[e] != 0) return;
+  if (a.done && a.done[e]) return;
+  const T0Global<CI, CS> src{md, a.tab + md.gat, a.tab + md.sca, (char*)(a.state + e), (uint32_t)(a.ld * 8)};
+  message_body_t0<CI, CS>(a, md, e, src);
 }
 
 // Runtime-shape variants share this tail: divide / multiply / residual / flag with

@@ -163,7 +163,7 @@ int launch_medium(pgbp_batch* b, const MsgArgs& a, int n, int I, int S) {
     } else if (M <= PGBP_COOP_MAX) {
       rc = launch_coop<48, 16>(b, a, n);
     } else {
-      rc = launch_message<-1, -1, 64>(b, a, n);
+      rc = launch_message<64>(b, a, n);
     }
   } else if (mode != 0 && M <= PGBP_COOP_MAX) {
     if (M <= 16) rc = (mode == 4) ? launch_coop<16, 4>(b, a, n) : launch_coop<16, 8>(b, a, n);
@@ -171,9 +171,9 @@ int launch_medium(pgbp_batch* b, const MsgArgs& a, int n, int I, int S) {
     else if (M <= 32) rc = launch_coop<32, 8>(b, a, n);
     else rc = launch_coop<48, 16>(b, a, n);  // 16 lanes per element: 2 elements per warp (half sectors)
   } else if (M <= 32) {
-    rc = launch_message<-1, -1, 32>(b, a, n);
+    rc = launch_message<32>(b, a, n);
   } else {
-    rc = launch_message<-1, -1, 64>(b, a, n);
+    rc = launch_message<64>(b, a, n);
   }
   return rc;
 }

@@ -1,4 +1,4 @@
-// One third of the register-resident message kernels (see pgbp_msg_t0.cuh).  -DPGBP_T0_PART=0: i in 1..3,
+// One third of the register-class message kernels (see pgbp_msg_t0.cuh).  -DPGBP_T0_PART=0: i in 1..3,
 // 1: i in 4..6, 2: i in 7..12.
 #include "pgbp_msg_t0.cuh"
 
@@ -25,7 +25,7 @@ namespace pgbp {
 template <int I_, int S_>
 static int try_shape(pgbp_batch* b, const MsgArgs& a, int nmsg, int ci, int cs) {
   if constexpr (I_ >= PGBP_PART_LO && I_ <= PGBP_PART_HI) {
-    if (ci == I_ && cs == S_) return launch_message<I_, S_, 0>(b, a, nmsg);
+    if (ci == I_ && cs == S_) return launch_message_staged<I_, S_>(b, a, nmsg);
   }
   return PGBP_NOT_MINE;
 }
