@@ -74,15 +74,6 @@ PGBP_HD void store_flag(const MsgArgs& a, int dmsg, int64_t e, int S, double max
   }
 }
 
-// L2 prefetch hint (device only): starts the HBM -> L2 transfer of a line that is read later
-PGBP_HD void l2_prefetch(const void* p) {
-#if defined(__CUDA_ARCH__)
-  asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p));
-#else
-  (void)p;
-#endif
-}
-
 // slot k of this element: base + k * (8*ld); 32-bit slot x 32-bit pitch -> one IMAD.WIDE.U32
 PGBP_HD double* slot_ptr(char* base, uint32_t slot, uint32_t ld8) {
   return (double*)(base + (uint64_t)slot * (uint64_t)ld8);
@@ -110,7 +101,7 @@ struct T0Rows {
 
 // Operand sources of message_body_t0: slot(n) is the slot of row n (T0Rows numbering), at(n, slot) its value for
 // this element.  T0Global reads the state array (host emulation, k_walk); the staged kernel's source reads a tile
-// staged in shared memory (pgbp_msg_t0.cuh).
+// staged in shared memory (pgbp_msg_t0.cuh), the tile walk's values loaded before the body runs (pgbp_message.cu).
 template <int I, int S>
 struct T0Global {
   const MsgDesc& md;
@@ -133,15 +124,15 @@ struct T0Global {
 // value and the receiver's old value are all loaded first (3*CHUNK independent
 // loads in flight per thread), then  new = J_KK - z_r.z_c,  delta = new - old,
 // and the three stores.  h and g follow the same pattern.  Operands come from src
-// (T0Global or a staged tile); results are stored to the state array.
-template <int CI, int CS, class Src>
-PGBP_HD void message_body_t0(const MsgArgs& a, const MsgDesc& md, int64_t e, const Src& src) {
+// (T0Global, a staged tile or the tile walk's registers); results are stored to the state array at the
+// destination rows of md (a MsgDesc, or the tile walk's TwDesc: same field names).
+template <int CI, int CS, class Desc, class Src>
+PGBP_HD void message_body_t0(const MsgArgs& a, const Desc& md, int64_t e, const Src& src) {
   constexpr int I = CI, S = CS, SI = I * (I + 1) / 2, SS = S * (S + 1) / 2;
   using R = T0Rows<I, S>;
   const uint32_t ld8 = (uint32_t)(a.ld * 8);  // (batches with 8*ld >= 2^32 are refused at creation)
   char* st = (char*)(a.state + e);
   char* rs = a.resid ? (char*)(a.resid + e) : nullptr;
-  const uint32_t sJ = (uint32_t)md.sJ, sh = (uint32_t)md.sh, rJ = (uint32_t)md.rJ, rh = (uint32_t)md.rh;
   auto ld = [&](int n) { return src.at(n, src.slot(n)); };
   double AI[SI > 0 ? SI : 1];
   double Bm[I * S > 0 ? I * S : 1];  // Bm[k*S + c] = J[I_k, K_c]
@@ -162,23 +153,6 @@ PGBP_HD void message_body_t0(const MsgArgs& a, const MsgDesc& md, int64_t e, con
   const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
   const double sg_old = sz ? 0.0 : ld(R::SG);
   const double tg_old = ld(R::TG);
-#ifdef PGBP_T0_PREFETCH
-  // everything the streaming phase will read (kept block of the sender, old sepset, old receiver):
-  // the HBM -> L2 transfers overlap the factorisation, the chunk loop then waits on L2 only
-#pragma unroll
-  for (int q = 0; q < SS; q++) {
-    const int c = colof(q), r = q - c * (c + 1) / 2;
-    l2_prefetch(slot_ptr(st, src.slot(R::FJ + pk(I + r, I + c)), ld8));
-    l2_prefetch(slot_ptr(st, sJ + q, ld8));
-    l2_prefetch(slot_ptr(st, src.slot(R::TJ + q), ld8));
-  }
-#pragma unroll
-  for (int k = 0; k < S; k++) {
-    l2_prefetch(slot_ptr(st, src.slot(R::FH + I + k), ld8));
-    l2_prefetch(slot_ptr(st, sh + k, ld8));
-    l2_prefetch(slot_ptr(st, src.slot(R::TH + k), ld8));
-  }
-#endif
 
   // "Ji = Jki = hi = 0 if missing data" shortcut, src/beliefupdates.jl:62-66
   bool allzero = true;
@@ -198,7 +172,7 @@ PGBP_HD void message_body_t0(const MsgArgs& a, const MsgDesc& md, int64_t e, con
     for (int k = 0; k < I; k++) {
       const double d = AI[pk(k, k)];
       if (!(d > 0.0)) {  // LAPACK potrf: info = k+1 (also catches NaN)
-        status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, k + 1));
+        status_fail(a.status, e, PGBP_STATUS(a.ref_base + (int32_t)md.ref, k + 1));
         return;
       }
       logdet += log(d);
@@ -252,9 +226,9 @@ PGBP_HD void message_body_t0(const MsgArgs& a, const MsgDesc& md, int64_t e, con
 #pragma unroll
       for (int i = 0; i < I; i++) nv = nfma(Bm[i * S + r], Bm[i * S + c], nv);
       const double d = nv - so[k];
-      *slot_ptr(st, sJ + q, ld8) = nv;
+      *slot_ptr(st, (uint32_t)md.sJ + q, ld8) = nv;  // (md read at the store: the tile walk's is in shared memory)
       *slot_ptr(st, ta[k], ld8) = to[k] + d;
-      if (rs) *slot_ptr(rs, rJ + q, ld8) = d;
+      if (rs) *slot_ptr(rs, (uint32_t)md.rJ + q, ld8) = d;
       absmax(maxJ, d);
     });
   });
@@ -274,15 +248,15 @@ PGBP_HD void message_body_t0(const MsgArgs& a, const MsgDesc& md, int64_t e, con
 #pragma unroll
       for (int i = 0; i < I; i++) nv = nfma(Bm[i * S + k], hI[i], nv);
       const double d = nv - so[k];
-      *slot_ptr(st, sh + k, ld8) = nv;
+      *slot_ptr(st, (uint32_t)md.sh + k, ld8) = nv;
       *slot_ptr(st, ta[k], ld8) = to[k] + d;
-      if (rs) *slot_ptr(rs, rh + k, ld8) = d;
+      if (rs) *slot_ptr(rs, (uint32_t)md.rh + k, ld8) = d;
       absmax(maxh, d);
     }
   }
   *slot_ptr(st, (uint32_t)md.sg, ld8) = g;
   *slot_ptr(st, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
-  store_flag(a, md.dmsg, e, S, maxJ, maxh);
+  store_flag(a, (int)md.dmsg, e, S, maxJ, maxh);
 }
 
 // One (message, element) of the register class with operands read from global memory.

@@ -70,145 +70,91 @@ PGBP_HD void walk_thread(const MsgArgs& a, int nmsg, int64_t e) {
 //  * a message issues ALL its loads (sender, old sepset, old receiver, status) before any arithmetic:
 //    one HBM/L2 round trip per message instead of three;
 //  * registers are capped (launch bounds) so that every block of the batch is resident at once.
-// The arithmetic is statement for statement that of message_thread_t0<I,S> (I = 0 is the streaming copy)
-// => bit-identical results (asserted by tests/test_parity.py and tests/test_fullsize.py).
+// The arithmetic is message_body_t0<I,S> on the loaded values (I = 0 is the streaming copy): results are
+// bit-identical to the per-step kernels by construction.
+
+// Operand source of message_body_t0 in the tile walk: slots from the pre-resolved descriptor, values v[n] loaded
+// by tilewalk_t0 before the body runs.
+template <int I, int S>
+struct T0Tile {
+  using R = T0Rows<I, S>;
+  const TwDesc& d;
+  double v[R::N];
+  PGBP_HD uint32_t slot(int n) const {
+    if (n < R::FH) return d.fJ[n];
+    if (n < R::FG) return d.fh[n - R::FH];
+    if (n == R::FG) return d.fg;
+    if (n == R::TG) return d.tg;
+    if (n < R::TH) return d.tJ[n - R::TJ];
+    if (n < R::SG) return d.th[n - R::TH];
+    if (n == R::SG) return d.sg;
+    return n < R::SH ? d.sJ + (uint32_t)(n - R::SJ) : d.sh + (uint32_t)(n - R::SH);
+  }
+  PGBP_HD double at(int n, uint32_t) const { return v[n]; }
+};
+
+// Loads in the order the body uses them (J_II, J_IK, h_I, g, then the kept entries with their old sepset and
+// receiver values): in row order k_tilewalk spills 1,664 instead of 1,328 bytes at its 64-register cap.
 template <int CI, int CS>
-PGBP_HD void message_thread_tw(const MsgArgs& a, const TwDesc& d, int64_t e) {
-  constexpr int I = CI, S = CS, SI = I * (I + 1) / 2, SS = S * (S + 1) / 2;
+PGBP_HD void tilewalk_t0(const MsgArgs& a, const TwDesc& d, int64_t e) {
+  constexpr int I = CI, S = CS, SS = S * (S + 1) / 2;
+  using R = T0Rows<I, S>;
   const uint32_t ld8 = (uint32_t)(a.ld * 8);
   char* st = (char*)(a.state + e);
-  char* rs = a.resid ? (char*)(a.resid + e) : nullptr;
-  const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
+  const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;  // the body does not read the old sepset then
   const int32_t stat = a.status[e];
   const uint8_t dn = a.done ? a.done[e] : (uint8_t)0;
-  double AI[SI > 0 ? SI : 1], Bm[I * S > 0 ? I * S : 1], hI[I > 0 ? I : 1];
-  double jo[SS > 0 ? SS : 1], sJo[SS > 0 ? SS : 1], tJo[SS > 0 ? SS : 1];
-  double ho[S > 0 ? S : 1], sho[S > 0 ? S : 1], tho[S > 0 ? S : 1];
+  T0Tile<I, S> src{d, {}};
+  auto load = [&](int n) { src.v[n] = *slot_ptr(st, src.slot(n), ld8); };
 #pragma unroll
   for (int c = 0; c < I; c++) {
 #pragma unroll
-    for (int r = 0; r <= c; r++) AI[pk(r, c)] = *slot_ptr(st, d.fJ[pk(r, c)], ld8);
+    for (int r = 0; r <= c; r++) load(R::FJ + pk(r, c));
   }
 #pragma unroll
   for (int c = 0; c < S; c++) {
 #pragma unroll
-    for (int k = 0; k < I; k++) Bm[k * S + c] = *slot_ptr(st, d.fJ[pk(k, I + c)], ld8);
+    for (int k = 0; k < I; k++) load(R::FJ + pk(k, I + c));
   }
 #pragma unroll
-  for (int k = 0; k < I; k++) hI[k] = *slot_ptr(st, d.fh[k], ld8);
-  double g = *slot_ptr(st, d.fg, ld8);
-  const double sg_old = sz ? 0.0 : *slot_ptr(st, d.sg, ld8);
-  const double tg_old = *slot_ptr(st, d.tg, ld8);
+  for (int k = 0; k < I; k++) load(R::FH + k);
+  load(R::FG);
+  if (!sz) load(R::SG);
+  load(R::TG);
 #pragma unroll
   for (int q = 0; q < SS; q++) {
     const int c = colof(q), r = q - c * (c + 1) / 2;
-    jo[q] = *slot_ptr(st, d.fJ[pk(I + r, I + c)], ld8);
-    sJo[q] = sz ? 0.0 : *slot_ptr(st, d.sJ + q, ld8);
-    tJo[q] = *slot_ptr(st, d.tJ[q], ld8);
+    load(R::FJ + pk(I + r, I + c));
+    if (!sz) load(R::SJ + q);
+    load(R::TJ + q);
   }
 #pragma unroll
   for (int k = 0; k < S; k++) {
-    ho[k] = *slot_ptr(st, d.fh[I + k], ld8);
-    sho[k] = sz ? 0.0 : *slot_ptr(st, d.sh + k, ld8);
-    tho[k] = *slot_ptr(st, d.th[k], ld8);
+    load(R::FH + I + k);
+    if (!sz) load(R::SH + k);
+    load(R::TH + k);
   }
   if (stat != 0 || dn) return;
-
-  bool allzero = true;  // src/beliefupdates.jl:62-66
-#pragma unroll
-  for (int q = 0; q < SI; q++)
-    if (!(fabs(AI[q]) <= PGBP_EPS)) allzero = false;
-#pragma unroll
-  for (int q = 0; q < I * S; q++)
-    if (!(fabs(Bm[q]) <= PGBP_EPS)) allzero = false;
-#pragma unroll
-  for (int k = 0; k < I; k++)
-    if (!(fabs(hI[k]) <= PGBP_EPS)) allzero = false;
-  if (!allzero) {
-    double logdet = 0.0, ww = 0.0;
-#pragma unroll
-    for (int k = 0; k < I; k++) {
-      const double dd = AI[pk(k, k)];
-      if (!(dd > 0.0)) {
-        status_fail(a.status, e, PGBP_STATUS(a.ref_base + (int32_t)d.ref, k + 1));
-        return;
-      }
-      logdet += log(dd);
-      const double rinv = 1.0 / sqrt(dd);
-#pragma unroll
-      for (int c = k + 1; c < I; c++) AI[pk(k, c)] *= rinv;
-#pragma unroll
-      for (int c = 0; c < S; c++) Bm[k * S + c] *= rinv;
-      const double wk = hI[k] * rinv;
-      hI[k] = wk;
-      ww = fma(wk, wk, ww);
-#pragma unroll
-      for (int c = k + 1; c < I; c++) {
-        const double akc = AI[pk(k, c)];
-#pragma unroll
-        for (int r = k + 1; r <= c; r++) AI[pk(r, c)] = nfma(AI[pk(k, r)], akc, AI[pk(r, c)]);
-        hI[c] = nfma(akc, wk, hI[c]);
-      }
-#pragma unroll
-      for (int c = 0; c < S; c++) {
-        const double bkc = Bm[k * S + c];
-#pragma unroll
-        for (int r = k + 1; r < I; r++) Bm[r * S + c] = nfma(AI[pk(k, r)], bkc, Bm[r * S + c]);
-      }
-    }
-    g += 0.5 * ((double)I * PGBP_LOG2PI - logdet + ww);
-  } else {
-#pragma unroll
-    for (int q = 0; q < I * S; q++) Bm[q] = 0.0;
-#pragma unroll
-    for (int k = 0; k < I; k++) hI[k] = 0.0;
-  }
-  double maxJ = 0.0, maxh = 0.0;
-#pragma unroll
-  for (int q = 0; q < SS; q++) {
-    const int c = colof(q), r = q - c * (c + 1) / 2;
-    double nv = jo[q];
-#pragma unroll
-    for (int i = 0; i < I; i++) nv = nfma(Bm[i * S + r], Bm[i * S + c], nv);
-    const double dl = nv - sJo[q];
-    *slot_ptr(st, d.sJ + q, ld8) = nv;
-    *slot_ptr(st, d.tJ[q], ld8) = tJo[q] + dl;
-    if (rs) *slot_ptr(rs, d.rJ + q, ld8) = dl;
-    absmax(maxJ, dl);
-  }
-#pragma unroll
-  for (int k = 0; k < S; k++) {
-    double nv = ho[k];
-#pragma unroll
-    for (int i = 0; i < I; i++) nv = nfma(Bm[i * S + k], hI[i], nv);
-    const double dl = nv - sho[k];
-    *slot_ptr(st, d.sh + k, ld8) = nv;
-    *slot_ptr(st, d.th[k], ld8) = tho[k] + dl;
-    if (rs) *slot_ptr(rs, d.rh + k, ld8) = dl;
-    absmax(maxh, dl);
-  }
-  *slot_ptr(st, d.sg, ld8) = g;
-  *slot_ptr(st, d.tg, ld8) = tg_old + (g - sg_old);
-  store_flag(a, (int)d.dmsg, e, S, maxJ, maxh);
+  message_body_t0<CI, CS>(a, d, e, src);
 }
 
 PGBP_HD void tilewalk_message(const MsgArgs& a, const TwDesc& d, int64_t e) {
   switch (d.shape) {
-    case 0 * 8 + 0: message_thread_tw<0, 0>(a, d, e); break;
-    case 0 * 8 + 1: message_thread_tw<0, 1>(a, d, e); break;
-    case 0 * 8 + 2: message_thread_tw<0, 2>(a, d, e); break;
-    case 0 * 8 + 3: message_thread_tw<0, 3>(a, d, e); break;
-    case 0 * 8 + 4: message_thread_tw<0, 4>(a, d, e); break;
-    case 1 * 8 + 0: message_thread_tw<1, 0>(a, d, e); break;
-    case 1 * 8 + 1: message_thread_tw<1, 1>(a, d, e); break;
-    case 1 * 8 + 2: message_thread_tw<1, 2>(a, d, e); break;
-    case 1 * 8 + 3: message_thread_tw<1, 3>(a, d, e); break;
-    case 2 * 8 + 0: message_thread_tw<2, 0>(a, d, e); break;
-    case 2 * 8 + 1: message_thread_tw<2, 1>(a, d, e); break;
-    case 2 * 8 + 2: message_thread_tw<2, 2>(a, d, e); break;
-    case 3 * 8 + 0: message_thread_tw<3, 0>(a, d, e); break;
-    case 3 * 8 + 1: message_thread_tw<3, 1>(a, d, e); break;
-    case 4 * 8 + 0: message_thread_tw<4, 0>(a, d, e); break;
+    case 0 * 8 + 0: tilewalk_t0<0, 0>(a, d, e); break;
+    case 0 * 8 + 1: tilewalk_t0<0, 1>(a, d, e); break;
+    case 0 * 8 + 2: tilewalk_t0<0, 2>(a, d, e); break;
+    case 0 * 8 + 3: tilewalk_t0<0, 3>(a, d, e); break;
+    case 0 * 8 + 4: tilewalk_t0<0, 4>(a, d, e); break;
+    case 1 * 8 + 0: tilewalk_t0<1, 0>(a, d, e); break;
+    case 1 * 8 + 1: tilewalk_t0<1, 1>(a, d, e); break;
+    case 1 * 8 + 2: tilewalk_t0<1, 2>(a, d, e); break;
+    case 1 * 8 + 3: tilewalk_t0<1, 3>(a, d, e); break;
+    case 2 * 8 + 0: tilewalk_t0<2, 0>(a, d, e); break;
+    case 2 * 8 + 1: tilewalk_t0<2, 1>(a, d, e); break;
+    case 2 * 8 + 2: tilewalk_t0<2, 2>(a, d, e); break;
+    case 3 * 8 + 0: tilewalk_t0<3, 0>(a, d, e); break;
+    case 3 * 8 + 1: tilewalk_t0<3, 1>(a, d, e); break;
+    case 4 * 8 + 0: tilewalk_t0<4, 0>(a, d, e); break;
     default: break;  // unreachable: use_tilewalk() admits sender dimensions <= 4 only
   }
 }

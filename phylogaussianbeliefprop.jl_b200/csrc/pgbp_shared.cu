@@ -218,49 +218,67 @@ PGBP_HD void jmsg_body(const JArgs& a, int mi, int64_t g, const W& w, double* A,
     a.calflag[(int64_t)md.dmsg * ld + g] = (S > 0 ? (maxJ / (double)S <= 1e-5) : true) ? 1 : 0;
 }
 
-// h, g part of one message for one element.  CI >= 0: compile-time integrated dimension (w in registers);
-// CI < 0: runtime (thread-local array).
-// CH: kept entries per streaming chunk (3 CH loads in flight per thread).  Measured on B200: CH = 4 beats CH = 8 (254
-// registers): c5s 4,801 vs 4,227 calibrations/s, c2s 137.7 vs 130.9 M/s at that stage; with CH = 4 the kernel is capped
-// at 128 registers for I <= 16 (4 blocks per SM: 166.5 ms per C5S step against 178.6 with 3 and 194.0 with 5)
-// STAGED (device only): the block staged the message's record and its two index tables in dynamic shared memory
-// (k_hmsg); they are read through the shared window (LDS with immediate offsets), not through generic pointers.
-template <int CI, int CH, bool STAGED = false>
-PGBP_HD void hmsg_thread(const HArgs& a, int mi, int64_t e, int reclen = 0) {
-  constexpr int PGBP_HMSG_CHUNK = CH;
-  const MsgDesc& md = a.msgs[mi];  // only the fields used below are loaded; rows fit 32 bits (checked at creation)
-  if (a.status[e] != 0) return;
+// Every slot row the element pass of a message (I, S), M = I + S, reads, numbered in one fixed order: sender h in [I;K]
+// order [0, TH), receiver h at the sepset's positions [TH, FG), sender g, receiver g, then the old sepset g and h
+// [SG, N).  The sepset rows come last because they are not read under PGBP_OPT_SEPZERO: k_hmsg_bulk then stages the
+// first SG rows only.
+struct HRows {
+  int TH, FG, TG, SG, SH, N;
+  PGBP_HD HRows(int M, int S) : TH(M), FG(M + S), TG(M + S + 1), SG(M + S + 2), SH(M + S + 3), N(M + 2 * S + 3) {}
+  PGBP_HD uint32_t slot(const MsgDesc& md, const int32_t* __restrict__ gat, const int32_t* __restrict__ sca, int n) const {
+    if (n < TH) return (uint32_t)md.fh + (uint32_t)gat[n];
+    if (n < FG) return (uint32_t)md.th + (uint32_t)sca[n - TH];
+    if (n == FG) return (uint32_t)md.fg;
+    if (n == TG) return (uint32_t)md.tg;
+    if (n == SG) return (uint32_t)md.sg;
+    return (uint32_t)md.sh + (uint32_t)(n - SH);
+  }
+};
+
+// Operand sources of hmsg_body: fslot(k) and tslot(k) are the slots of rows k and TH + k (HRows numbering),
+// at(n, slot) the value of row n for this element, rec the group's factor record.  HTab reads the state array through
+// the index tables, with tables and record in global memory (host emulation, k_hwalk, k_hmsg) or staged in shared
+// memory by k_hmsg; HBulk reads every row from k_hmsg_bulk's tile.  ahead: the old sepset and receiver values of a
+// chunk are loaded with the sender's before its arithmetic (global memory: 3 CH loads in flight), not at the stores
+// (shared memory: nothing held across the arithmetic -- loaded ahead, k_hmsg_bulk<16> took 9 % longer on one B200).
+struct HTab {
+  static constexpr bool ahead = true;
+  uint32_t fh, th;
+  const int32_t* __restrict__ gat;  // sender positions of [I;K]
+  const int32_t* __restrict__ sca;  // receiver positions of the sepset's variables
+  const double* __restrict__ rec;
+  char* st;
+  uint32_t ld8;
+  PGBP_HD uint32_t fslot(int k) const { return fh + (uint32_t)gat[k]; }
+  PGBP_HD uint32_t tslot(int k) const { return th + (uint32_t)sca[k]; }
+  PGBP_HD double at(int, uint32_t s) const { return *slot_ptr(st, s, ld8); }
+};
+
+// h, g part of one message for one element whose status is 0.  CI >= 0: compile-time integrated dimension (w in
+// registers); CI < 0: runtime (thread-local array).
+// CH: kept entries per streaming chunk (3 CH loads in flight per thread).  Measured on B200 for the thread-per-element
+// kernels: CH = 4 beats CH = 8 (254 registers): c5s 4,801 vs 4,227 calibrations/s, c2s 137.7 vs 130.9 M/s at that
+// stage; with CH = 4 k_hmsg is capped at 128 registers for I <= 16 (4 blocks per SM: 166.5 ms per C5S step against
+// 178.6 with 3 and 194.0 with 5).  k_hmsg_bulk reads its operands from shared memory and takes CH = 8.
+template <int CI, int CH, class Src>
+PGBP_HD void hmsg_body(const HArgs& a, const MsgDesc& md, int64_t e, const Src& src) {
   const int S = md.s;
   const int I = CI >= 0 ? CI : md.mF - S, M = I + S;
+  const HRows R(M, S);
   const uint32_t ld8 = (uint32_t)(a.ld * 8);
   char* st = (char*)(a.state + e);
   char* rs = a.resid ? (char*)(a.resid + e) : nullptr;
-  const uint32_t fh = (uint32_t)md.fh, sh = (uint32_t)md.sh, th = (uint32_t)md.th, rh = (uint32_t)md.rh;
+  const uint32_t sh = (uint32_t)md.sh, rh = (uint32_t)md.rh;
   const uint32_t sg = (uint32_t)md.sg, tg = (uint32_t)md.tg;
-#if !defined(PGBP_HOST_EMUL)
-  extern __shared__ double srec[];
-  const int32_t* stab = (const int32_t*)(srec + reclen);
-  const int32_t* __restrict__ gat = STAGED ? stab : a.tab + md.gat + tri(M);  // sender positions of [I;K]
-  const int32_t* __restrict__ sca = STAGED ? stab + M : a.tab + md.sca + tri(S);  // receiver positions of the sepset's variables
-#else
-  (void)reclen;
-  const int32_t* __restrict__ gat = a.tab + md.gat + tri(M);
-  const int32_t* __restrict__ sca = a.tab + md.sca + tri(S);
-#endif
   const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;  // lazy sepset zero: old sepset h, g are 0, not loaded
-  double g = *slot_ptr(st, (uint32_t)md.fg, ld8);
-  const double sg_old = sz ? 0.0 : *slot_ptr(st, sg, ld8), tg_old = *slot_ptr(st, tg, ld8);
+  double g = src.at(R.FG, (uint32_t)md.fg);
+  const double sg_old = sz ? 0.0 : src.at(R.SG, sg), tg_old = src.at(R.TG, tg);
   double hI[CI > 0 ? CI : (CI == 0 ? 1 : PGBP_MAX_DIM)];
-  const double* __restrict__ rec = nullptr;
+  const double* __restrict__ rec = src.rec;
   bool zeroZ = true;
   if (I > 0) {
-#if !defined(PGBP_HOST_EMUL)
-    if constexpr (STAGED) rec = srec;
-    else
-#endif
-      rec = a.cache + (e / a.gs) * a.stride + a.cache_off[mi];
 #pragma unroll
-    for (int k = 0; k < I; k++) hI[k] = *slot_ptr(st, fh + gat[k], ld8);
+    for (int k = 0; k < I; k++) hI[k] = src.at(k, src.fslot(k));
     const double info = rec[0];
     if (info > 0.0) {  // the factorisation of the group's J_I failed at this pivot
       status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, (int)info));
@@ -292,16 +310,19 @@ PGBP_HD void hmsg_thread(const HArgs& a, int mi, int64_t e, int reclen = 0) {
     }
   }
   double maxh = 0.0;
-  for (int k0 = 0; k0 < S; k0 += PGBP_HMSG_CHUNK) {
-    double nv[PGBP_HMSG_CHUNK], so[PGBP_HMSG_CHUNK], to[PGBP_HMSG_CHUNK];
-    double* tp[PGBP_HMSG_CHUNK];
+  for (int k0 = 0; k0 < S; k0 += CH) {
+    double nv[CH], so[CH], to[CH];
+    uint32_t ta[CH];
+    auto load_old = [&](int j) {  // receiver slot, old sepset and receiver values of kept entry k0 + j
+      ta[j] = src.tslot(k0 + j);
+      so[j] = sz ? 0.0 : src.at(R.SH + k0 + j, sh + k0 + j);
+      to[j] = src.at(R.TH + k0 + j, ta[j]);
+    };
 #pragma unroll
-    for (int j = 0; j < PGBP_HMSG_CHUNK; j++)
+    for (int j = 0; j < CH; j++)
       if (k0 + j < S) {
-        tp[j] = slot_ptr(st, th + sca[k0 + j], ld8);
-        nv[j] = *slot_ptr(st, fh + gat[I + k0 + j], ld8);
-        so[j] = sz ? 0.0 : *slot_ptr(st, sh + k0 + j, ld8);
-        to[j] = *tp[j];
+        nv[j] = src.at(I + k0 + j, src.fslot(I + k0 + j));
+        if constexpr (Src::ahead) load_old(j);
       }
     if (!zeroZ) {
       const double* row = rec + 2 + I;
@@ -309,17 +330,18 @@ PGBP_HD void hmsg_thread(const HArgs& a, int mi, int64_t e, int reclen = 0) {
       for (int i = 0; i < I; i++) {
         const double wi = hI[i];
 #pragma unroll
-        for (int j = 0; j < PGBP_HMSG_CHUNK; j++)
+        for (int j = 0; j < CH; j++)
           if (k0 + j < S) nv[j] = nfma(row[(I - 1 - i) + k0 + j], wi, nv[j]);
         row += M - 1 - i;
       }
     }
 #pragma unroll
-    for (int j = 0; j < PGBP_HMSG_CHUNK; j++)
+    for (int j = 0; j < CH; j++)
       if (k0 + j < S) {
+        if constexpr (!Src::ahead) load_old(j);
         const double d = nv[j] - so[j];
         *slot_ptr(st, sh + k0 + j, ld8) = nv[j];
-        *tp[j] = to[j] + d;
+        *slot_ptr(st, ta[j], ld8) = to[j] + d;
         if (rs) *slot_ptr(rs, rh + k0 + j, ld8) = d;
         absmax(maxh, d);
       }
@@ -328,6 +350,17 @@ PGBP_HD void hmsg_thread(const HArgs& a, int mi, int64_t e, int reclen = 0) {
   *slot_ptr(st, tg, ld8) = tg_old + (g - sg_old);
   if ((a.opts & PGBP_CAL_RESIDNORM) && a.calflag)
     a.calflag[(int64_t)md.dmsg * a.ld + e] = (S > 0 ? (maxh / sqrt((double)S) <= 1e-5) : true) ? 1 : 0;
+}
+
+// One (message, element) of the element pass with tables and record read from global memory.
+template <int CI>
+PGBP_HD void hmsg_thread(const HArgs& a, int mi, int64_t e) {
+  const MsgDesc& md = a.msgs[mi];  // only the fields used are loaded; rows fit 32 bits (checked at creation)
+  if (a.status[e] != 0) return;
+  const int S = md.s, M = CI >= 0 ? CI + S : md.mF;
+  const double* rec = M > S ? a.cache + (e / a.gs) * a.stride + a.cache_off[mi] : nullptr;
+  hmsg_body<CI, 4>(a, md, e, HTab{(uint32_t)md.fh, (uint32_t)md.th, a.tab + md.gat + tri(M), a.tab + md.sca + tri(S), rec,
+                                   (char*)(a.state + e), (uint32_t)(a.ld * 8)});
 }
 
 #ifndef PGBP_HOST_EMUL
@@ -362,8 +395,8 @@ __global__ void __launch_bounds__(NT) k_jmsg(JArgs a, int maxM) {
 #ifndef PGBP_HMSG_MINB
 #define PGBP_HMSG_MINB 4  // resident blocks per SM of the element pass for I <= 16 (register cap 128)
 #endif
-template <int CI, int CH>
-__global__ void __launch_bounds__(128, (CH <= 4 ? (CI >= 0 && CI <= 16 ? PGBP_HMSG_MINB : 3) : 2)) k_hmsg(HArgs a, int reclen) {
+template <int CI>
+__global__ void __launch_bounds__(128, (CI >= 0 && CI <= 16 ? PGBP_HMSG_MINB : 3)) k_hmsg(HArgs a, int reclen) {
   extern __shared__ double srec[];
   const int64_t e0 = (int64_t)blockIdx.x * blockDim.x;
   const int64_t e = e0 + threadIdx.x;
@@ -384,8 +417,16 @@ __global__ void __launch_bounds__(128, (CH <= 4 ? (CI >= 0 && CI <= 16 ? PGBP_HM
     }
   }
   if (e >= a.B) return;
-  if (staged) hmsg_thread<CI, CH, true>(a, blockIdx.y, e, reclen);
-  else hmsg_thread<CI, CH, false>(a, blockIdx.y, e);
+  if (!staged) {
+    hmsg_thread<CI>(a, blockIdx.y, e);
+    return;
+  }
+  // record and tables through the shared window (LDS with immediate offsets), not through generic pointers
+  const MsgDesc& md = a.msgs[blockIdx.y];
+  if (a.status[e] != 0) return;
+  const int32_t* stab = (const int32_t*)(srec + reclen);
+  hmsg_body<CI, 4>(a, md, e, HTab{(uint32_t)md.fh, (uint32_t)md.th, stab, stab + md.mF, srec, (char*)(a.state + e),
+                                  (uint32_t)(a.ld * 8)});
 }
 
 // Element pass with bulk-copy staging: the wide levels of big graphs (C5: 420k messages x 1,536 replicates) are a
@@ -396,20 +437,26 @@ __global__ void __launch_bounds__(128, (CH <= 4 ? (CI >= 0 && CI <= 16 ? PGBP_HM
 // g) is a contiguous 1 KB segment of the batch-innermost layout, so thread n issues ONE cp.async.bulk for row n, the
 // factor record arrives by a bulk copy too, and all of them (67 rows = 69 KB for an (I,S) = (16,16) message) are in
 // flight at once on one mbarrier, without holding a register.  Three blocks per SM keep ~200 KB in flight.  The
-// arithmetic (element = thread, operands from shared memory, conflict-free) repeats hmsg_thread operation by
-// operation: bit-identical results.
+// arithmetic is hmsg_body with operands from shared memory (element = thread, conflict-free): bit-identical results.
+struct HBulk {
+  static constexpr bool ahead = false;
+  const double* rec;
+  const double* r;         // this element's column of the tile: row n at r[128 n]
+  const uint32_t* sl;      // slot of every staged row
+  int th;
+  PGBP_HD uint32_t fslot(int k) const { return sl[k]; }
+  PGBP_HD uint32_t tslot(int k) const { return sl[th + k]; }
+  PGBP_HD double at(int n, uint32_t) const { return r[n * 128]; }
+};
 template <int CI>
 __global__ void __launch_bounds__(128, (CI <= 16 ? 3 : 2)) k_hmsg_bulk(HArgs a, int reclen) {
   extern __shared__ __align__(128) double sm[];
   __shared__ __align__(8) unsigned long long mbar;
-  constexpr int I = CI;
   const int tid = threadIdx.x;
   const MsgDesc& md = a.msgs[blockIdx.y];
-  const int S = md.s, M = I + S;
-  const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
-  const int nrows = M + S + 2 + (sz ? 0 : S + 1);
-  // rows: [0, M) sender h in [I;K] order | [M, M+S) target h | M+S: sender g | M+S+1: target g | (unless sz) M+S+2:
-  // sepset g | M+S+3+k: sepset h
+  const int S = md.s, M = CI + S;
+  const HRows R(M, S);
+  const int nrows = (a.opts & PGBP_OPT_SEPZERO) ? R.SG : R.N;
   const int64_t e0 = (int64_t)blockIdx.x * 128, e = e0 + tid;
   const int64_t left = a.ld - e0;
   const uint32_t rowbytes = (uint32_t)(left < 128 ? left : 128) * 8u;
@@ -427,13 +474,7 @@ __global__ void __launch_bounds__(128, (CI <= 16 ? 3 : 2)) k_hmsg_bulk(HArgs a, 
     const int32_t* __restrict__ gat = a.tab + md.gat + tri(M);
     const int32_t* __restrict__ sca = a.tab + md.sca + tri(S);
     for (int n = tid; n < nrows; n += 128) {
-      uint32_t slot;
-      if (n < M) slot = (uint32_t)md.fh + (uint32_t)gat[n];
-      else if (n < M + S) slot = (uint32_t)md.th + (uint32_t)sca[n - M];
-      else if (n == M + S) slot = (uint32_t)md.fg;
-      else if (n == M + S + 1) slot = (uint32_t)md.tg;
-      else if (n == M + S + 2) slot = (uint32_t)md.sg;
-      else slot = (uint32_t)md.sh + (uint32_t)(n - (M + S + 3));
+      const uint32_t slot = R.slot(md, gat, sca, n);
       sslot[n] = slot;
       bulk_g2s(rows + (size_t)n * 128, tileb + (uint64_t)slot * (uint64_t)ld8, rowbytes, &mbar);
     }
@@ -442,79 +483,7 @@ __global__ void __launch_bounds__(128, (CI <= 16 ? 3 : 2)) k_hmsg_bulk(HArgs a, 
   __syncthreads();       // sslot
   mbar_wait(&mbar, 0);   // every row and the record have landed (no thread leaves the block before that)
   if (stat != 0) return;
-  char* st = (char*)(a.state + e);
-  char* rs = a.resid ? (char*)(a.resid + e) : nullptr;
-  const double* rec = sm;
-  const double* r = rows + tid;
-  double g = r[(M + S) * 128];
-  const double tg_old = r[(M + S + 1) * 128], sg_old = sz ? 0.0 : r[(M + S + 2) * 128];
-  double hI[I];
-#pragma unroll
-  for (int k = 0; k < I; k++) hI[k] = r[k * 128];
-  bool zeroZ = true;
-  const double info = rec[0];
-  if (info > 0.0) {
-    status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, (int)info));
-    return;
-  }
-  if (info < 0.0) {
-    bool hz = true;
-#pragma unroll
-    for (int k = 0; k < I; k++)
-      if (!(fabs(hI[k]) <= PGBP_EPS)) hz = false;
-    if (!hz) {
-      status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, 1));
-      return;
-    }
-  } else {
-    zeroZ = false;
-    double ww = 0.0;
-    const double* row = rec + 2 + I;
-#pragma unroll
-    for (int k = 0; k < I; k++) {
-      const double wk = hI[k] * rec[2 + k];
-      hI[k] = wk;
-      ww = fma(wk, wk, ww);
-#pragma unroll
-      for (int c = k + 1; c < I; c++) hI[c] = nfma(row[c - k - 1], wk, hI[c]);
-      row += M - 1 - k;
-    }
-    g += 0.5 * ((double)I * PGBP_LOG2PI - rec[1] + ww);
-  }
-  double maxh = 0.0;
-  constexpr int CH = 8;
-  for (int k0 = 0; k0 < S; k0 += CH) {
-    double nv[CH];
-#pragma unroll
-    for (int j = 0; j < CH; j++)
-      if (k0 + j < S) nv[j] = r[(I + k0 + j) * 128];
-    if (!zeroZ) {
-      const double* row = rec + 2 + I;
-#pragma unroll
-      for (int i = 0; i < I; i++) {
-        const double wi = hI[i];
-#pragma unroll
-        for (int j = 0; j < CH; j++)
-          if (k0 + j < S) nv[j] = nfma(row[(I - 1 - i) + k0 + j], wi, nv[j]);
-        row += M - 1 - i;
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < CH; j++)
-      if (k0 + j < S) {
-        const int k = k0 + j;
-        const double so = sz ? 0.0 : r[(M + S + 3 + k) * 128];
-        const double d = nv[j] - so;
-        *slot_ptr(st, (uint32_t)md.sh + k, ld8) = nv[j];
-        *slot_ptr(st, sslot[M + k], ld8) = r[(M + k) * 128] + d;
-        if (rs) *slot_ptr(rs, (uint32_t)md.rh + k, ld8) = d;
-        absmax(maxh, d);
-      }
-  }
-  *slot_ptr(st, (uint32_t)md.sg, ld8) = g;
-  *slot_ptr(st, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
-  if ((a.opts & PGBP_CAL_RESIDNORM) && a.calflag)
-    a.calflag[(int64_t)md.dmsg * a.ld + e] = (S > 0 ? (maxh / sqrt((double)S) <= 1e-5) : true) ? 1 : 0;
+  hmsg_body<CI, 8>(a, md, e, HBulk{sm, rows + tid, sslot, M});
 }
 #endif
 
@@ -561,12 +530,12 @@ __global__ void __launch_bounds__(32 * PGBP_SW_WIDE) k_jwalk(JArgs a, const int3
 }
 
 // (one out-of-line body per shape: inlined into one switch the nine small shapes cost 2 KB of spills and a 1 KB frame)
-template <int CI, int CH>
-__device__ __noinline__ void hmsg_call(const HArgs& a, int m, int64_t e) { hmsg_thread<CI, CH>(a, m, e); }
+template <int CI>
+__device__ __noinline__ void hmsg_call(const HArgs& a, int m, int64_t e) { hmsg_thread<CI>(a, m, e); }
 
 // SMALL: every message of the run integrates at most 8 variables (C2-like graphs): exact small shapes, 128 registers,
 // four resident blocks per SM; otherwise the I = 0 / 16 / 32 shapes of the p = 16 workloads at 255 registers.
-template <int CH, bool SMALL>
+template <bool SMALL>
 __global__ void __launch_bounds__(128, (SMALL ? 4 : 1)) k_hwalk(HArgs a, const int32_t* __restrict__ step_off, int s0, int s1,
                                                   const unsigned* flags, unsigned* hcount, unsigned* done_blocks, int64_t G) {
   __shared__ unsigned need;
@@ -595,22 +564,22 @@ __global__ void __launch_bounds__(128, (SMALL ? 4 : 1)) k_hwalk(HArgs a, const i
         const int I = a.msgs[m].mF - a.msgs[m].s;
         if constexpr (SMALL) {
           switch (I) {
-            case 0: hmsg_call<0, CH>(a, m, e); break;
-            case 1: hmsg_call<1, CH>(a, m, e); break;
-            case 2: hmsg_call<2, CH>(a, m, e); break;
-            case 3: hmsg_call<3, CH>(a, m, e); break;
-            case 4: hmsg_call<4, CH>(a, m, e); break;
-            case 5: hmsg_call<5, CH>(a, m, e); break;
-            case 6: hmsg_call<6, CH>(a, m, e); break;
-            case 7: hmsg_call<7, CH>(a, m, e); break;
-            default: hmsg_call<8, CH>(a, m, e); break;
+            case 0: hmsg_call<0>(a, m, e); break;
+            case 1: hmsg_call<1>(a, m, e); break;
+            case 2: hmsg_call<2>(a, m, e); break;
+            case 3: hmsg_call<3>(a, m, e); break;
+            case 4: hmsg_call<4>(a, m, e); break;
+            case 5: hmsg_call<5>(a, m, e); break;
+            case 6: hmsg_call<6>(a, m, e); break;
+            case 7: hmsg_call<7>(a, m, e); break;
+            default: hmsg_call<8>(a, m, e); break;
           }
         } else {
           switch (I) {
-            case 0: hmsg_call<0, CH>(a, m, e); break;
-            case 16: hmsg_thread<16, CH>(a, m, e); break;
-            case 32: hmsg_thread<32, CH>(a, m, e); break;
-            default: hmsg_thread<-1, CH>(a, m, e); break;
+            case 0: hmsg_call<0>(a, m, e); break;
+            case 16: hmsg_thread<16>(a, m, e); break;
+            case 32: hmsg_thread<32>(a, m, e); break;
+            default: hmsg_thread<-1>(a, m, e); break;
           }
         }
       }
@@ -662,26 +631,18 @@ static int launch_jmsg(pgbp_batch* b, JArgs a, int nmsg, int maxM, pgbp_stream_t
   return 0;
 }
 
-static int hmsg_chunk() {  // PGBP_HMSG_CHUNK=8 selects the wider streaming chunk of the element pass (tuning knob; default 4)
-  static const int v = [] { const char* e = getenv("PGBP_HMSG_CHUNK"); return (e && atoi(e) == 8) ? 8 : 4; }();
-  return v;
-}
-static bool hmsg_bulk() {  // PGBP_HMSG_BULK=0: the thread-per-element kernel everywhere (A/B switch)
-  static const bool v = [] { const char* e = getenv("PGBP_HMSG_BULK"); return !(e && atoi(e) == 0); }();
-  return v;
-}
 template <int CI>
 static int launch_hmsg_t(pgbp_batch* b, const HArgs& a, int nmsg, int reclen) {
 #ifdef PGBP_HOST_EMUL
   (void)reclen;
   for (int m = 0; m < nmsg; m++)
-    for (int64_t e = 0; e < a.B; e++) hmsg_thread<CI, 4>(a, m, e);
+    for (int64_t e = 0; e < a.B; e++) hmsg_thread<CI>(a, m, e);
 #else
   dim3 grid((unsigned)((a.B + 127) / 128), (unsigned)nmsg);
   if constexpr (CI == 8 || CI == 12 || CI == 16 || CI == 24 || CI == 32) {
     // bulk-copy staging (k_hmsg_bulk): every block of 128 elements inside one group, 16-byte aligned rows, one
     // message shape per launch (reclen > 0), and the rows of a message fit the shared memory of an SM
-    if (hmsg_bulk() && reclen > 0 && (a.gs % 128 == 0 || a.gs >= a.B) && a.ld % 2 == 0 && a.B >= 64) {
+    if (reclen > 0 && (a.gs % 128 == 0 || a.gs >= a.B) && a.ld % 2 == 0 && a.B >= 64) {
       const int S = (int)((reclen - 2 - CI - (CI * (CI - 1)) / 2) / CI);  // jrec_len(I, S) solved for S
       const int reclen16 = (reclen + 15) / 16 * 16;
       const int nrows = CI + 3 * S + 3;
@@ -697,8 +658,7 @@ static int launch_hmsg_t(pgbp_batch* b, const HArgs& a, int nmsg, int reclen) {
   }
   if (reclen * 8 > 40 * 1024) reclen = 0;  // (records beyond the default dynamic shared memory: global loads)
   const size_t smem = reclen ? sizeof(double) * (size_t)reclen + sizeof(int32_t) * 2 * PGBP_MAX_DIM : 0;
-  if (hmsg_chunk() == 4) k_hmsg<CI, 4><<<grid, 128, smem, b->stream>>>(a, reclen);
-  else k_hmsg<CI, 8><<<grid, 128, smem, b->stream>>>(a, reclen);
+  k_hmsg<CI><<<grid, 128, smem, b->stream>>>(a, reclen);
 #endif
   b->launches++;
   return check_launch("k_hmsg");
@@ -886,10 +846,9 @@ int shared_run_traversal(pgbp_batch* b, int tree, int dir, uint32_t opts, int32_
       }
       int maxI = 0;
       for (int k = tv.step_off[g.step]; k < tv.step_off[s1]; k++) maxI = std::max(maxI, tv.msgs[k].mF - tv.msgs[k].s);
-#define PGBP_HWALK(CH_, SM_) k_hwalk<CH_, SM_><<<grid, 128, 0, b->stream>>>(c, b->jb->d_step_off[td], g.step, s1, b->d_walkflags[td], b->d_walkcount[td], b->d_walkcount[td] + 1, b->ngroups)
-      if (maxI <= 8) PGBP_HWALK(4, true);
-      else if (hmsg_chunk() == 4) PGBP_HWALK(4, false);
-      else PGBP_HWALK(8, false);
+#define PGBP_HWALK(SM_) k_hwalk<SM_><<<grid, 128, 0, b->stream>>>(c, b->jb->d_step_off[td], g.step, s1, b->d_walkflags[td], b->d_walkcount[td], b->d_walkcount[td] + 1, b->ngroups)
+      if (maxI <= 8) PGBP_HWALK(true);
+      else PGBP_HWALK(false);
 #undef PGBP_HWALK
       b->launches++;
       PGBP_TRY(check_launch("k_hwalk"));

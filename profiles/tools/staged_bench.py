@@ -1,16 +1,20 @@
 """Parent build against this tree's build of the CUDA library, on one GPU, in one session.
 
     python profiles/tools/staged_bench.py --out DIR --lib parent=PATH --lib new=PATH [--lib NAME=PATH ...]
-                                          [--runs 3] [--default-runs]
+                                          [--runs 3] [--workloads c2:700,c3:30,...] [--dumps c2,c4,c3]
+                                          [--no-profile] [--default-runs]
 
 Every library is an already built libpgbp_b200.so (phylogaussianbeliefprop.jl_b200/build.py); nothing is compiled
 here.  The first --lib is the baseline.  Written to DIR:
   card.csv                  nvidia-smi name, power limit and maximum SM clock, read in the same session
-  c2_<lib>_<k>.json         bench.py --steps 700 --no-others --no-cpu, libraries alternated, k = 1..runs
+  <w>_<lib>_<k>.json        bench.py --workload w --steps K --no-others --no-cpu for every w:K of --workloads (default
+                            c2:700), libraries alternated, k = 1..runs
   dump_<w>_<lib>/           bench.py --dump-outputs for --dumps (default c2, c4, c3; same seeded inputs)
   kernels_<lib>.txt / .json torch.profiler per-kernel device time of one C2 step (after warm-up), own process
+                            (unless --no-profile)
   default_<lib>.json        (--default-runs) the default bench.py run: other_workloads block and CPU check
-  summary.json              medians, spreads, ratios against the baseline, byte-identity of every dump
+  summary.json              per workload: medians, spreads, ratios against the baseline and whether each median lies
+                            within the baseline's min..max; byte-identity of every dump
 Run `--profile-c2 FILE` alone to profile one C2 step with the library PGBP_B200_LIB selects.
 """
 import argparse
@@ -96,7 +100,9 @@ def main():
     ap.add_argument("--lib", action="append", default=[])
     ap.add_argument("--runs", type=int, default=3)
     ap.add_argument("--default-runs", action="store_true")
+    ap.add_argument("--workloads", default="c2:700", help="timed workloads, name:steps, comma-separated")
     ap.add_argument("--dumps", default="c2,c4,c3", help="workloads whose outputs are dumped and compared")
+    ap.add_argument("--no-profile", action="store_true", help="skip the per-kernel profile of one C2 step")
     ap.add_argument("--profile-c2")
     args = ap.parse_args()
     if args.profile_c2:
@@ -113,27 +119,34 @@ def main():
                           capture_output=True, text=True)
     open(os.path.join(out, "card.csv"), "w").write(card.stdout + card.stderr)
     py = sys.executable
-    summary = {"card": card.stdout.strip().splitlines(), "libraries": dict(libs), "c2": {}, "dumps": {}}
-    vals = {n: [] for n, _ in libs}
+    workloads = [(w, int(k)) for w, k in (x.split(":") for x in args.workloads.split(",") if x)]
+    summary = {"card": card.stdout.strip().splitlines(), "libraries": {n: os.path.relpath(p, ROOT) for n, p in libs},
+               "dumps": {}}
+    vals = {(w, n): [] for w, _ in workloads for n, _ in libs}
     for k in range(1, args.runs + 1):
-        for n, p in libs:
-            f = os.path.join(out, "c2_%s_%d.json" % (n, k))
-            rc = run([py, "bench.py", "--steps", "700", "--no-others", "--no-cpu"], p, f, f[:-5] + ".err")
-            j = last_json(f)
-            if rc == 0 and j:
-                vals[n].append(j["value"])
+        for w, steps in workloads:
+            for n, p in libs:
+                f = os.path.join(out, "%s_%s_%d.json" % (w, n, k))
+                rc = run([py, "bench.py", "--workload", w, "--steps", str(steps), "--no-others", "--no-cpu"], p, f,
+                         f[:-5] + ".err")
+                j = last_json(f)
+                if rc == 0 and j:
+                    vals[(w, n)].append(j["value"])
     base = libs[0][0]
-    for n, _ in libs:
-        v = vals[n]
-        summary["c2"][n] = {"values": v, "median": statistics.median(v) if v else None,
-                            "min": min(v) if v else None, "max": max(v) if v else None}
-    bm = summary["c2"][base]["median"]
-    for n, _ in libs:
-        s = summary["c2"][n]
-        if bm and s["median"]:
-            s["median_over_baseline"] = s["median"] / bm
-            s["min_over_baseline_max"] = s["min"] / summary["c2"][base]["max"]
-    steps = {"c2": 20, "c4": 3, "c3": 2}
+    for w, _ in workloads:
+        summary[w] = {}
+        for n, _ in libs:
+            v = vals[(w, n)]
+            summary[w][n] = {"values": v, "median": statistics.median(v) if v else None,
+                             "min": min(v) if v else None, "max": max(v) if v else None}
+        b = summary[w][base]
+        for n, _ in libs:
+            s = summary[w][n]
+            if b["median"] and s["median"]:
+                s["median_over_baseline"] = s["median"] / b["median"]
+                s["min_over_baseline_max"] = s["min"] / b["max"]
+                s["median_within_baseline_spread"] = b["min"] <= s["median"] <= b["max"]
+    steps = {"c2": 20, "c4": 3, "c3": 2, "c3l": 2, "c2s": 20, "c5s": 1}
     for w in filter(None, args.dumps.split(",")):
         st = steps[w]
         for n, p in libs:
@@ -149,6 +162,8 @@ def main():
                 open(os.path.join(ref, x), "rb").read() == open(os.path.join(dd, x), "rb").read() for x in names)
             summary["dumps"]["%s_%s" % (w, n)] = {"files": names, "byte_identical": same}
     for n, p in libs:
+        if args.no_profile:
+            break
         f = os.path.join(out, "kernels_%s.txt" % n)
         run([py, os.path.abspath(__file__), "--profile-c2", f], p, f + ".log", f + ".err")
     if args.default_runs:
@@ -169,7 +184,7 @@ def main():
                         w: (v / dflt[base]["other_workloads"][w]) if v and dflt[base]["other_workloads"].get(w) else None
                         for w, v in dflt[n]["other_workloads"].items()}
     json.dump(summary, open(os.path.join(out, "summary.json"), "w"), indent=1)
-    print(json.dumps(summary["c2"]))
+    print(json.dumps({w: summary[w] for w, _ in workloads}))
     print(json.dumps(summary["dumps"]))
 
 
