@@ -271,6 +271,12 @@ def assignfactors(beliefs, model, tbl, taxa, prenodes, node2cluster, node2family
             cols = [be.nodelabel.index(q) for q in i_inscope]
             var_inscope = be.inscope[:, cols]
             keep_index = np.flatnonzero(var_inscope.T.ravel())  # 0-based, column-major
+            # DELIBERATE DEVIATION from src/beliefs.jl:845-857: a parent's out-of-scope trait t is observed
+            # below no child of it, so the child's trait t is gone already (marginalised above, or by
+            # absorbleaf); under Brownian motion the child's other traits depend on the parents' trait t
+            # not at all, and its rows of (h, J) are zero in exact arithmetic.  They are dropped, not
+            # marginalised: the reference factorises their roundoff (~1e-14 on short edges), which adds
+            # ~ -log(1e-14)/2 per trait to g, or fails on a negative pivot.
             if not node2fixed[ni - 1]:
                 kc = keep_index[keep_index < p]
                 integ_ch = np.setdiff1d(np.arange(p), kc)
@@ -278,14 +284,11 @@ def assignfactors(beliefs, model, tbl, taxa, prenodes, node2cluster, node2family
                 h, J, g = marginalize(h, J, g, keep_ch, integ_ch)
                 if any(not node2fixed[q - 1] for q in nf[1:]):
                     nkc = kc.size
-                    keep_pa = keep_index[keep_index >= p]
-                    integ_pa = np.setdiff1d(np.arange(p, p * len(i_inscope)), keep_pa)
-                    keep_pa = keep_pa - (p - nkc)
-                    integ_pa = integ_pa - (p - nkc)
-                    h, J, g = marginalize(h, J, g, np.concatenate([np.arange(nkc), keep_pa]), integ_pa)
+                    keep_pa = keep_index[keep_index >= p] - (p - nkc)
+                    keep = np.concatenate([np.arange(nkc), keep_pa])
+                    h, J = h[keep], J[np.ix_(keep, keep)]
             else:
-                integ = np.setdiff1d(np.arange(h.size), keep_index)
-                h, J, g = marginalize(h, J, g, keep_index, integ)
+                h, J = h[keep_index], J[np.ix_(keep_index, keep_index)]
         # mult! (src/beliefupdates.jl:483-488)
         be.h[factorind] += h
         be.J[np.ix_(factorind, factorind)] += J

@@ -265,7 +265,7 @@ struct AssignBody {
 //   heterogeneousmodels.jl:119-150, evomodels.jl:377-396)
 //   -> absorbleaf!: absorb the observed traits of a leaf, marginalise its missing ones (beliefupdates.jl:266-274)
 //   -> absorbevidence! of a fixed root among the parents (beliefs.jl:828-831)
-//   -> marginalise the out-of-scope traits: child first, then parents (beliefs.jl:836-857)
+//   -> marginalise the child's out-of-scope traits, drop the parents' (beliefs.jl:836-857; see below)
 //   -> mult! into the cluster at the scope positions (beliefs.jl:858).
 // The working factor is a dense packed-upper matrix over the live variables in thread-local memory
 // (<= PGBP_SCOPED_MAXN variables): this path is about coverage, not speed.  marginalize() keeps the
@@ -467,7 +467,12 @@ struct AssignScoped {
         }
         if (anyroot) f.absorb(sel, val);
       }
-      // out-of-scope traits (src/beliefs.jl:836-857): child first, then parents
+      // out-of-scope traits (src/beliefs.jl:836-857): child first, then parents.  A parent's out-of-scope
+      // trait t is observed below none of its children, so the child's trait t is gone by stage 1 (stage 0 or
+      // absorbleaf!); under Brownian motion the child's other traits do not depend on the parents' trait t, and
+      // its rows of (h, J) are zero in exact arithmetic.  Stage 1 drops them: the reference marginalises them,
+      // which factorises their roundoff (~1e-14 on short edges) and adds ~ -log(1e-14)/2 per trait to g, or
+      // fails on a negative pivot.
       for (int stage = 0; stage < 2; stage++) {
         bool any = false;
         for (int i = 0; i < f.n; i++) {
@@ -476,6 +481,7 @@ struct AssignScoped {
           any = any || sel[i];
         }
         if (!any) continue;
+        if (stage == 1) { f.compact_keep(sel); continue; }
         const int info = f.marginalize(sel);
         if (info) { status_fail(gen.status, e, PGBP_STATUS(0x7ffff9, info)); st[gsl * ld] = NAN; return; }
       }
