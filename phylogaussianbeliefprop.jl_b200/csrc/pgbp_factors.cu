@@ -362,21 +362,128 @@ struct ScopedFactor {
   }
 };
 
+// Sources of the family factors of the scoped K1 body: Brownian motion from the prepared theta rows (ThetaPrep), the
+// univariate Ornstein-Uhlenbeck model from its (sigma2, alpha, theta, mu, v) records.  For parameter set ip:
+//   fail(ip)                    0, or the status word of an invalid parameter set
+//   root(ip, f)                 the root prior over f's p variables (f.h is zero on entry); false: the factor is 1
+//   family(ip, F, k0, nm, f)    the full factor of one node family over (child, parents) x traits (f.h is zero on
+//                               entry); 0 or a status word
+//   mu(ip, t)                   the root prior mean of trait t, which is the value of a fixed root
+struct ScopedBM {
+  const double* theta;  // SoA [rows][ldp]
+  int64_t ldp;
+  ThetaRows tr;
+  PGBP_HD double th(int64_t ip, int row) const { return theta[ip + (int64_t)row * ldp]; }
+  PGBP_HD int32_t fail(int64_t ip) const {
+    const double kind = th(ip, tr.kind());
+    return kind < 0.0 ? PGBP_STATUS(0x7ffffd, (int)(-kind)) : 0;
+  }
+  PGBP_HD bool root(int64_t ip, ScopedFactor& f) const {
+    if (th(ip, tr.kind()) != 1.0) return false;  // fixed root, or improper prior
+    const int p = tr.p;
+    for (int cc = 0; cc < p; cc++) {
+      for (int r = 0; r <= cc; r++) f.A[pk(r, cc)] = th(ip, tr.rootP() + cc * p + r);
+      f.h[cc] = th(ip, tr.rooth() + cc);
+    }
+    f.g = th(ip, tr.rootg());
+    return true;
+  }
+  PGBP_HD int32_t family(int64_t ip, const FamDev& F, int k0, int nm, ScopedFactor& f) const {
+    const int p = tr.p, pp = p * p;
+    double j[PGBP_MAX_TRAITS * PGBP_MAX_TRAITS], w[PGBP_MAX_TRAITS * PGBP_MAX_TRAITS];
+    bool samecolor = true;
+    for (int k = k0 + 2; k < k0 + nm; k++) if (F.mem_color[k] != F.mem_color[k0 + 1]) samecolor = false;
+    if (samecolor) {
+      const int col = F.mem_color[k0 + 1];
+      double t0 = 0.0;
+      if (nm == 2) t0 = F.mem_length[k0 + 1];
+      else for (int k = k0 + 1; k < k0 + nm; k++) t0 += F.mem_gamma[k] * F.mem_gamma[k] * F.mem_length[k];
+      for (int q = 0; q < pp; q++) j[q] = th(ip, tr.P(col) + q) / t0;
+      f.g = th(ip, tr.g0(col)) - 0.5 * p * log(t0);
+    } else {
+      for (int q = 0; q < pp; q++) w[q] = 0.0;
+      for (int k = k0 + 1; k < k0 + nm; k++) {
+        const double fk = F.mem_gamma[k] * F.mem_gamma[k] * F.mem_length[k];
+        const int col = F.mem_color[k];
+        for (int q = 0; q < pp; q++) w[q] += fk * th(ip, tr.R(col) + q);
+      }
+      double ldv;
+      const int info = spd_inverse_logdet(w, j, p, &ldv);
+      if (info) return PGBP_STATUS(0x7ffffc, info);
+      f.g = -0.5 * (p * PGBP_LOG2PI + ldv);
+    }
+    for (int b2 = 0; b2 < nm; b2++) {
+      const double cb = b2 == 0 ? 1.0 : (nm == 2 ? -1.0 : -F.mem_gamma[k0 + b2]);
+      for (int a2 = 0; a2 <= b2; a2++) {
+        const double ca = a2 == 0 ? 1.0 : (nm == 2 ? -1.0 : -F.mem_gamma[k0 + a2]);
+        const double cab = ca * cb;
+        for (int tb = 0; tb < p; tb++)
+          for (int ta = 0; ta < (a2 == b2 ? tb + 1 : p); ta++) f.A[pk(a2 * p + ta, b2 * p + tb)] = cab * j[tb * p + ta];
+      }
+    }
+    return 0;
+  }
+  PGBP_HD double mu(int64_t ip, int t) const { return th(ip, tr.mu() + t); }
+};
+
+// The univariate OU factor of AssignOU before any evidence: with c = (1, -gamma_1 q_1, ..), j = 1 / var,
+//   J = j c c',  h = j omega c,  g = -(log 2pi + log var)/2 - j omega^2 / 2  (src/evomodels/evomodels.jl:214-245)
+struct ScopedOU {
+  const double* params;  // [np][5]: sigma2, alpha, theta, mu, v
+  PGBP_HD int32_t fail(int64_t ip) const {
+    const double* th = params + 5 * ip;
+    return !(th[0] > 0.0) || !(th[1] > 0.0) ? PGBP_STATUS(0x7ffffd, 1) : 0;
+  }
+  PGBP_HD bool root(int64_t ip, ScopedFactor& f) const {
+    const double mu = params[5 * ip + 3], v = params[5 * ip + 4];
+    if (v == 0.0 || v == INFINITY) return false;
+    const double jr = 1.0 / v;
+    f.A[0] = jr;
+    f.h[0] = jr * mu;
+    f.g = 0.5 * (-PGBP_LOG2PI + log(jr) - mu * (jr * mu));
+    return true;
+  }
+  PGBP_HD int32_t family(int64_t ip, const FamDev& F, int k0, int nm, ScopedFactor& f) const {
+    const double* th = params + 5 * ip;
+    const double sigma2 = th[0], alpha = th[1], theta = th[2];
+    const double gamma2 = sigma2 / (2.0 * alpha);
+    double cf[PGBP_MAX_FAMILY];
+    double var = 0.0, omega = 0.0;
+    cf[0] = 1.0;
+    for (int a = 1; a < nm; a++) {
+      const double t = F.mem_length[k0 + a], gam = nm == 2 ? 1.0 : F.mem_gamma[k0 + a];
+      const double q = exp(-alpha * t);
+      var += gam * gam * (gamma2 * (1.0 - q * q));
+      omega += gam * ((1.0 - q) * theta);
+      cf[a] = -(gam * q);
+    }
+    const double j = 1.0 / var;
+    for (int b = 0; b < nm; b++) {
+      f.h[b] = cf[b] * (j * omega);
+      for (int a = 0; a <= b; a++) f.A[pk(a, b)] = (cf[a] * cf[b]) * j;
+    }
+    f.g = -0.5 * (PGBP_LOG2PI + log(var)) - 0.5 * (omega * (j * omega));
+    return 0;
+  }
+  PGBP_HD double mu(int64_t ip, int) const { return params[5 * ip + 3]; }
+};
+
+// gen: the family tables, tip data, output, status and pairing (its theta fields are read through Src only)
+template <class Src>
 struct AssignScoped {
   AssignBody gen;
   const int32_t* mem_tpos;     // [#members * p]
   const uint8_t* tip_missing;  // [ntips * p]
+  Src src;
   int y0 = 0;
   PGBP_HD void operator()(int64_t e, int y) const { run(e, y + y0); }
   PGBP_HD void run(int64_t e, int c) const {
     const FamDev& F = gen.F;
-    const ThetaRows& tr = gen.tr;
-    const int p = F.p, pp = p * p;
-    const int64_t ld = gen.ld, ldp = gen.ldp, ldd = gen.ldd;
+    const int p = F.p;
+    const int64_t ld = gen.ld, ldd = gen.ldd;
     int64_t ip, idd;
     if (gen.pairing == PGBP_PAIR_PRODUCT) { ip = e / gen.nd; idd = e % gen.nd; }
     else { ip = gen.np == 1 ? 0 : e; idd = gen.nd == 1 ? 0 : e; }
-    const double* th = gen.theta + ip;
     const double* td = gen.tip + idd;
     double* st = gen.state + e;
     const bool lead = gen.gs == 0;
@@ -385,13 +492,12 @@ struct AssignScoped {
     if (lead) for (int q = 0; q < tri(m); q++) st[(js + q) * ld] = 0.0;
     for (int q = 0; q < m; q++) st[(hs + q) * ld] = 0.0;
     double g = 0.0;
-    const double kind = th[(int64_t)tr.kind() * ldp];
-    if (kind < 0.0) {
-      if (c == 0) status_fail(gen.status, e, PGBP_STATUS(0x7ffffd, (int)(-kind)));
+    const int32_t bad = src.fail(ip);
+    if (bad) {
+      if (c == 0) status_fail(gen.status, e, bad);
       st[gsl * ld] = NAN;
       return;
     }
-    double j[PGBP_MAX_TRAITS * PGBP_MAX_TRAITS], w[PGBP_MAX_TRAITS * PGBP_MAX_TRAITS];
     ScopedFactor f;
     bool sel[PGBP_SCOPED_MAXN];
     double val[PGBP_SCOPED_MAXN];
@@ -401,43 +507,10 @@ struct AssignScoped {
       f.n = nm * p;
       for (int i = 0; i < f.n; i++) { f.h[i] = 0.0; f.id[i] = (int16_t)i; }
       if (nm == 1) {  // root family (src/beliefs.jl:803-807)
-        if (F.mem_pos[k0] < 0 || kind != 1.0) continue;  // fixed root, or improper prior: factor == 1
-        for (int cc = 0; cc < p; cc++) {
-          for (int r = 0; r <= cc; r++) f.A[pk(r, cc)] = th[(int64_t)(tr.rootP() + cc * p + r) * ldp];
-          f.h[cc] = th[(int64_t)(tr.rooth() + cc) * ldp];
-        }
-        f.g = th[(int64_t)tr.rootg() * ldp];
+        if (F.mem_pos[k0] < 0 || !src.root(ip, f)) continue;  // fixed root, or improper prior: factor == 1
       } else {
-        bool samecolor = true;
-        for (int k = k0 + 2; k < k0 + nm; k++) if (F.mem_color[k] != F.mem_color[k0 + 1]) samecolor = false;
-        if (samecolor) {
-          const int col = F.mem_color[k0 + 1];
-          double t0 = 0.0;
-          if (nm == 2) t0 = F.mem_length[k0 + 1];
-          else for (int k = k0 + 1; k < k0 + nm; k++) t0 += F.mem_gamma[k] * F.mem_gamma[k] * F.mem_length[k];
-          for (int q = 0; q < pp; q++) j[q] = th[(int64_t)(tr.P(col) + q) * ldp] / t0;
-          f.g = th[(int64_t)tr.g0(col) * ldp] - 0.5 * p * log(t0);
-        } else {
-          for (int q = 0; q < pp; q++) w[q] = 0.0;
-          for (int k = k0 + 1; k < k0 + nm; k++) {
-            const double fk = F.mem_gamma[k] * F.mem_gamma[k] * F.mem_length[k];
-            const int col = F.mem_color[k];
-            for (int q = 0; q < pp; q++) w[q] += fk * th[(int64_t)(tr.R(col) + q) * ldp];
-          }
-          double ldv;
-          const int info = spd_inverse_logdet(w, j, p, &ldv);
-          if (info) { status_fail(gen.status, e, PGBP_STATUS(0x7ffffc, info)); st[gsl * ld] = NAN; return; }
-          f.g = -0.5 * (p * PGBP_LOG2PI + ldv);
-        }
-        for (int b2 = 0; b2 < nm; b2++) {
-          const double cb = b2 == 0 ? 1.0 : (nm == 2 ? -1.0 : -F.mem_gamma[k0 + b2]);
-          for (int a2 = 0; a2 <= b2; a2++) {
-            const double ca = a2 == 0 ? 1.0 : (nm == 2 ? -1.0 : -F.mem_gamma[k0 + a2]);
-            const double cab = ca * cb;
-            for (int tb = 0; tb < p; tb++)
-              for (int ta = 0; ta < (a2 == b2 ? tb + 1 : p); ta++) f.A[pk(a2 * p + ta, b2 * p + tb)] = cab * j[tb * p + ta];
-          }
-        }
+        const int32_t info = src.family(ip, F, k0, nm, f);
+        if (info) { status_fail(gen.status, e, info); st[gsl * ld] = NAN; return; }
         // absorbleaf!: observed traits of the leaf, then its missing traits
         const int row = F.node_datarow[v];
         const bool child_fixed = F.mem_pos[k0] < 0;
@@ -462,7 +535,7 @@ struct AssignScoped {
         for (int i = 0; i < f.n; i++) {
           const int a2 = f.id[i] / p, t = f.id[i] % p;
           sel[i] = a2 >= 1 && F.mem_pos[k0 + a2] < 0;
-          val[i] = sel[i] ? th[(int64_t)(tr.mu() + t) * ldp] : 0.0;
+          val[i] = sel[i] ? src.mu(ip, t) : 0.0;
           anyroot = anyroot || sel[i];
         }
         if (anyroot) f.absorb(sel, val);
@@ -472,7 +545,9 @@ struct AssignScoped {
       // absorbleaf!); under Brownian motion the child's other traits do not depend on the parents' trait t, and
       // its rows of (h, J) are zero in exact arithmetic.  Stage 1 drops them: the reference marginalises them,
       // which factorises their roundoff (~1e-14 on short edges) and adds ~ -log(1e-14)/2 per trait to g, or
-      // fails on a negative pivot.
+      // fails on a negative pivot.  Under the univariate OU model (p = 1) a parent is out of scope only if its
+      // child is too; the child was marginalised in stage 0, which leaves the parent's (h, J) entries as
+      // roundoff of zero and nothing else, so dropping them is exact there as well.
       for (int stage = 0; stage < 2; stage++) {
         bool any = false;
         for (int i = 0; i < f.n; i++) {
@@ -1418,7 +1493,8 @@ static int assign_launch(pgbp_batch* b, pgbp::DevTables* dt, double* out, int32_
   AssignBody body{fd, dt->theta, dt->ldp, dt->tip, dt->ldd, out, b->status, b->ld, nparamsets, ndatasets, pairing, tr};
   body.gs = b->group_size;
   if (F.scoped)  // trait-level scopes (missing data): the reference's absorb / marginalise sequence
-    return launch_generic(b, "k_assign_scoped", b->B, p->nclusters, AssignScoped{body, dt->mem_tpos, dt->tip_missing});
+    return launch_generic(b, "k_assign_scoped", b->B, p->nclusters,
+                          AssignScoped<ScopedBM>{body, dt->mem_tpos, dt->tip_missing, ScopedBM{dt->theta, dt->ldp, tr}});
   // shared-precision batches: cache of the family precision blocks, written by the group pass (this function called
   // on the group batch: b->jparent set) and read by the element pass (b->jb set)
   double* juc = nullptr;
@@ -1502,11 +1578,21 @@ int32_t pgbp_assign_factors_ou(pgbp_batch* b, const double* params, int64_t npar
     b->B = saveB;
     PGBP_TRY(rc);
   }
-  FamDev fd{dt->node_cluster, dt->mem_off, dt->mem_pos, dt->mem_length, dt->mem_gamma, dt->mem_color,
-            dt->node_datarow, dt->clu_off, dt->clu_node, dt->jslot, dt->hslot, dt->gslot, dt->dim, 1, 1, F.root_fixed};
-  AssignOU body{fd, b->scratch, dt->tip, dt->ldd, b->state, b->status, b->ld, nparamsets, ndatasets, pairing};
-  body.gs = b->group_size;
-  PGBP_TRY(launch_generic(b, "k_assign_ou", b->B, p->nclusters, body));
+  // K1 on the element batch, or on the group batch of a shared-precision batch (gs == 0: it assigns the J rows)
+  auto launch = [&](pgbp_batch* bb, DevTables* t, int64_t nd, int64_t gs) -> int {
+    FamDev fd{t->node_cluster, t->mem_off, t->mem_pos, t->mem_length, t->mem_gamma, t->mem_color,
+              t->node_datarow, t->clu_off, t->clu_node, t->jslot, t->hslot, t->gslot, t->dim, 1, 1, F.root_fixed};
+    if (F.scoped) {  // trait-level scopes (missing data): the reference's absorb / marginalise sequence
+      AssignBody gen{fd, nullptr, 0, dt->tip, dt->ldd, bb->state, bb->status, bb->ld, nparamsets, nd, pairing, ThetaRows{1, 1}};
+      gen.gs = gs;
+      return launch_generic(bb, "k_assign_scoped", bb->B, p->nclusters,
+                            AssignScoped<ScopedOU>{gen, t->mem_tpos, t->tip_missing, ScopedOU{b->scratch}});
+    }
+    AssignOU body{fd, b->scratch, dt->tip, dt->ldd, bb->state, bb->status, bb->ld, nparamsets, nd, pairing};
+    body.gs = gs;
+    return launch_generic(bb, "k_assign_ou", bb->B, p->nclusters, body);
+  };
+  PGBP_TRY(launch(b, dt, ndatasets, b->group_size));
   b->lazy_factors.pending = false;  // (the OU parameters live in scratch memory: eager snapshot)
   b->lazy_factors.valid = false;
   if (b->jb) {  // shared-precision batch: J rows once per group in the group batch (see assign_enqueue)
@@ -1514,11 +1600,8 @@ int32_t pgbp_assign_factors_ou(pgbp_batch* b, const double* params, int64_t npar
     jb->stream = b->stream;
     DevTables* jdt;
     PGBP_TRY(get_tables(jb, &jdt));
-    FamDev jfd{jdt->node_cluster, jdt->mem_off, jdt->mem_pos, jdt->mem_length, jdt->mem_gamma, jdt->mem_color,
-               jdt->node_datarow, jdt->clu_off, jdt->clu_node, jdt->jslot, jdt->hslot, jdt->gslot, jdt->dim, 1, 1, F.root_fixed};
     const int64_t jnd = pairing == PGBP_PAIR_PRODUCT ? ndatasets / b->group_size : 1;
-    AssignOU jbody{jfd, b->scratch, dt->tip, dt->ldd, jb->state, jb->status, jb->ld, nparamsets, jnd, pairing};
-    PGBP_TRY(launch_generic(jb, "k_assign_ou", jb->B, p->nclusters, jbody));
+    PGBP_TRY(launch(jb, jdt, jnd, 0));
     jb->lazy_factors.pending = false;
     jb->lazy_factors.valid = false;
     PGBP_TRY(batch_zero_sepsets(b, false));
