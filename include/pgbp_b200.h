@@ -263,6 +263,48 @@ int32_t pgbp_assign_factors_device(pgbp_batch* batch, int32_t ncolors, const dou
 int32_t pgbp_assign_factors_ou(pgbp_batch* batch, const double* params, int64_t nparamsets,
                                const double* tipdata, int64_t ndatasets, int32_t pairing);
 
+/* ---------------------------------------------------------------- forward simulation
+ * Trait replicates simulated down the network on the device (parametric bootstrap, power studies, coverage checks):
+ * the output `tipdata` is the record layout pgbp_assign_factors[_device] reads, so simulate -> assign -> calibrate ->
+ * integrate needs no tip data on the host.  Requires plan.families plus mem_parent, one entry per family member
+ * (aligned with mem_off / mem_length): the 0-based preorder index of a parent member, -1 for the child's own entry.
+ * Nodes are visited in preorder; replicate r of parameter record theta draws, for node v:
+ *  - root (v = 0): V == 0 -> x_0 = mu;  proper V -> x_0 = mu + chol_lower(V) z_0;  any diag(V) == Inf (improper) ->
+ *    nothing to draw: status PGBP_STATUS(0x7ffff7, 1) and NaN outputs.
+ *  - PGBP_MODEL_BM (params as pgbp_assign_factors, ncolors rates): K1's factor.  One parent: coefficient 1,
+ *    Sigma = t R_c;  >= 2 parents: mean sum_k gamma_k x_pa_k, Sigma = sum_k gamma_k^2 t_k R_{c_k}.  When every parent
+ *    edge has one colour L = sqrt(t0) chol_lower(R_c), else L = chol_lower(Sigma);  x_v = mean + L z_v, and x_v = mean
+ *    (no draw) when t0 == 0.  A rate or V that is not positive definite: status PGBP_STATUS(0x7ffffd, pivot) (a mixed-
+ *    colour Sigma: PGBP_STATUS(0x7ffffc, pivot), as in K1).
+ *  - PGBP_MODEL_OU (records (sigma2, alpha, theta, mu, v), ntraits == ncolors == 1): q_k = exp(-alpha t_k),
+ *    mean sum_k gamma_k (q_k x_pa_k + (1 - q_k) theta), variance sum_k gamma_k^2 sigma2 / (2 alpha) (1 - q_k^2)
+ *    (gamma = 1 for one parent; 1 - q and 1 - q^2 formed with expm1).  sigma2 <= 0, alpha <= 0 or NaN: status
+ *    PGBP_STATUS(0x7ffffd, 1).
+ *  - normals: Philox4x32-10, key (seed & 0xffffffff, seed >> 32) (seed read as unsigned), counter
+ *    (v, k, r & 0xffffffff, r >> 32) for the trait pair k (traits 2k, 2k+1) of node v;
+ *    u1 = ((x0 >> 5) 2^26 + (x1 >> 6) + 1) 2^-53, u2 = ((x2 >> 5) 2^26 + (x3 >> 6)) 2^-53, rho = sqrt(-2 log u1),
+ *    z_2k = rho cos(6.283185307179586 u2), z_2k+1 = rho sin(6.283185307179586 u2).
+ * Element e is replicate r = first_replicate + e and its values depend on (seed, r, v, k) only: chunking, launch shape
+ * and batch size change nothing, a batch of one at first_replicate = r reproduces element r of a larger batch, and
+ * ranks sharding a run with first_replicate = rank * B_rank together equal one single-GPU run.  Element e uses
+ * parameter record min(e, nparamsets - 1), nparamsets in {1, B} (1 on a shared-precision batch).
+ * Outputs (either may be NULL, not both): tipdata [B][ntips][p] by node_datarow, NaN where the plan's tip_missing is
+ * set (feeds a missing-data plan directly); nodes [B][nnodes][p] in preorder, every node's value (also the true value
+ * of missing tip traits).  Status words are recorded like every other call's (pgbp_get_status).
+ * PGBP_ESTATE: no family table.  PGBP_EINVAL: unknown model; OU with ntraits != 1 or ncolors != 1; ncolors below the
+ * table's colours; nparamsets not in {1, B} or > 1 on a shared-precision batch; a parent index out of range or not
+ * smaller than its child's; a non-root node without parents; a tip with children; first_replicate < 0; both outputs
+ * NULL. */
+#define PGBP_MODEL_BM 0
+#define PGBP_MODEL_OU 1
+int32_t pgbp_simulate(pgbp_batch* batch, int32_t model, int32_t ncolors, const int32_t* mem_parent,
+                      const double* params, int64_t nparamsets, int64_t seed, int64_t first_replicate,
+                      double* tipdata, double* nodes);
+/* same with DEVICE params and outputs, enqueue only */
+int32_t pgbp_simulate_device(pgbp_batch* batch, int32_t model, int32_t ncolors, const int32_t* mem_parent,
+                             const double* d_params, int64_t nparamsets, int64_t seed, int64_t first_replicate,
+                             double* d_tipdata, double* d_nodes);
+
 /* ---------------------------------------------------------------- message passing */
 #define PGBP_CAL_POSTORDER 1u       /* propagate_1traversal_postorder! (src/calibration.jl:111-135) */
 #define PGBP_CAL_PREORDER 2u        /* propagate_1traversal_preorder!  (src/calibration.jl:137-161) */

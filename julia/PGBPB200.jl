@@ -125,7 +125,7 @@ and the library runs the reference's absorb / marginalise sequence per node fami
 function familiestable(prenodes, node2cluster, node2family, node2fixed, beliefs, taxa; edgecolor = e -> 0, rootfixed::Bool, tbl = nothing)
     p = beliefs[1].ntraits
     mem_off = Int32[0]; mem_pos = Int32[]; mem_len = Float64[]; mem_gam = Float64[]; mem_col = Int32[]; row = Int32[]
-    mem_tpos = Int32[]; partial = false
+    mem_tpos = Int32[]; mem_par = Int32[]; partial = false
     for (v, node) in enumerate(prenodes)
         be = beliefs[node2cluster[v]]
         nd = vec(sum(be.inscope, dims=1)); cs = cumsum(vcat(0, nd))
@@ -141,6 +141,7 @@ function familiestable(prenodes, node2cluster, node2family, node2fixed, beliefs,
                     if be.inscope[t, jj]; push!(mem_tpos, run); run += 1 else push!(mem_tpos, -1) end
                 end
             end
+            push!(mem_par, k == 1 ? -1 : q - 1)   # simulate!: 0-based preorder index of a parent, -1 for the child
             if k == 1
                 push!(mem_len, 0.0); push!(mem_gam, 1.0); push!(mem_col, 0)
             else
@@ -158,7 +159,7 @@ function familiestable(prenodes, node2cluster, node2family, node2fixed, beliefs,
     (nnodes = Int32(length(prenodes)), ntips = Int32(length(taxa)), root_fixed = Int32(rootfixed),
      node_cluster = Int32.(node2cluster .- 1), mem_off = mem_off, mem_pos = mem_pos, mem_length = mem_len,
      mem_gamma = mem_gam, mem_color = mem_col, node_datarow = row,
-     mem_tpos = scoped ? mem_tpos : Int32[], tip_missing = scoped ? miss : UInt8[])
+     mem_tpos = scoped ? mem_tpos : Int32[], tip_missing = scoped ? miss : UInt8[], mem_parent = mem_par)
 end
 
 mutable struct Plan
@@ -461,6 +462,48 @@ assignfactors_device!(b::BatchedClusterGraphBelief, d_params::Ptr{Float64}, npar
                       ndatasets::Integer; ncolors::Integer=1, pairing::Symbol=:zip) =
     check(ccall((:pgbp_assign_factors_device, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Float64}, Int64, Ptr{Float64}, Int64, Int32),
                 b.handle, ncolors, d_params, nparamsets, d_tipdata, ndatasets, pairing === :product ? PAIR_PRODUCT : PAIR_ZIP))
+
+const MODEL_BM = Int32(0)
+const MODEL_OU = Int32(1)
+function _mem_parent(b::BatchedClusterGraphBelief)
+    f = b.plan.arrays.families
+    (f === nothing || !haskey(f, :mem_parent)) && error("simulate! needs mem_parent in the plan's families table (familiestable)")
+    f
+end
+
+"""
+    simulate!(b, params::Matrix{Float64}, seed::Integer; first_replicate=0, model=:bm, ncolors=1, nodes=false)
+
+Trait replicates simulated down the network on the device (parametric bootstrap): element e is replicate
+`first_replicate + e` of `seed` and depends on nothing else.  `params`: (len, nparamsets) records of `assignfactors!`
+(`model = :bm`) or (σ2, α, θ, μ, v) (`model = :ou`), nparamsets in {1, B}.  Returns the tip data (p, ntips, B) that
+`assignfactors!` takes (NaN where the plan's tip is missing), and with `nodes = true` also every node's value
+(p, nnodes, B), preorder.
+"""
+function simulate!(b::BatchedClusterGraphBelief, params::Matrix{Float64}, seed::Integer; first_replicate::Integer=0,
+                   model::Symbol=:bm, ncolors::Integer=1, nodes::Bool=false)
+    f = _mem_parent(b)
+    p = Int(b.plan.arrays.ntraits)
+    tip = Array{Float64,3}(undef, p, f.ntips, b.B)
+    nd = Array{Float64,3}(undef, p, nodes ? f.nnodes : 0, b.B)
+    GC.@preserve params tip nd check(ccall((:pgbp_simulate, LIB), Int32,
+        (Ptr{Cvoid}, Int32, Int32, Ptr{Int32}, Ptr{Float64}, Int64, Int64, Int64, Ptr{Float64}, Ptr{Float64}),
+        b.handle, model === :ou ? MODEL_OU : MODEL_BM, ncolors, f.mem_parent, params, size(params, 2),
+        reinterpret(Int64, UInt64(seed)), first_replicate, tip, nodes ? pointer(nd) : Ptr{Float64}(C_NULL)))
+    nodes ? (tip, nd) : tip
+end
+
+"`simulate!` with device records and outputs (`CUDA.CuArray` pointers; either output may be C_NULL), enqueue only"
+function simulate_device!(b::BatchedClusterGraphBelief, d_params::Ptr{Float64}, nparamsets::Integer, seed::Integer,
+                          d_tipdata::Ptr{Float64}, d_nodes::Ptr{Float64}=Ptr{Float64}(C_NULL); first_replicate::Integer=0,
+                          model::Symbol=:bm, ncolors::Integer=1)
+    f = _mem_parent(b)
+    GC.@preserve f check(ccall((:pgbp_simulate_device, LIB), Int32,
+        (Ptr{Cvoid}, Int32, Int32, Ptr{Int32}, Ptr{Float64}, Int64, Int64, Int64, Ptr{Float64}, Ptr{Float64}),
+        b.handle, model === :ou ? MODEL_OU : MODEL_BM, ncolors, f.mem_parent, d_params, nparamsets,
+        reinterpret(Int64, UInt64(seed)), first_replicate, d_tipdata, d_nodes))
+end
+
 function calibrate_async!(b::BatchedClusterGraphBelief, schedule::AbstractVector, niter::Integer=1; auto::Bool=false,
                           update_residualnorm::Bool=true, direction::UInt32=CAL_BOTH)
     ids = Int32[treeid(b, spt) for spt in schedule]

@@ -72,6 +72,8 @@ SIGNATURES = {
     "pgbp_assign_factors": (i32, [vp, i32, P(f64), i64, P(f64), i64, i32]),
     "pgbp_assign_factors_ou": (i32, [vp, P(f64), i64, P(f64), i64, i32]),
     "pgbp_assign_factors_device": (i32, [vp, i32, vp, i64, vp, i64, i32]),
+    "pgbp_simulate": (i32, [vp, i32, i32, P(i32), P(f64), i64, i64, i64, P(f64), P(f64)]),
+    "pgbp_simulate_device": (i32, [vp, i32, i32, P(i32), vp, i64, i64, i64, vp, vp]),
     "pgbp_calibrate": (i32, [vp, P(i32), i32, i32, u32, P(i32), P(i32), P(i32)]),
     "pgbp_calibrate_async": (i32, [vp, P(i32), i32, i32, u32]),
     "pgbp_propagate": (i32, [vp, i32, i32, i32, u32]),
@@ -105,6 +107,7 @@ SIGNATURES = {
 BATCH_FACTORS, BATCH_RESIDUALS = 1, 2
 CAL_POSTORDER, CAL_PREORDER, CAL_BOTH, CAL_RESIDNORM, CAL_RESIDKLDIV, CAL_AUTO, CAL_REFORDER = 1, 2, 3, 4, 8, 16, 32
 PAIR_ZIP, PAIR_PRODUCT = 0, 1
+MODEL_BM, MODEL_OU = 0, 1
 
 
 class Library:

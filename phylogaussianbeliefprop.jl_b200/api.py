@@ -200,7 +200,7 @@ def families_table(prenodes_info, node2cluster, node2family, node2fixed, beliefs
     n = len(node2cluster)
     taxa = list(taxa) if taxa is not None else None
     mem_off, mem_pos, mem_len, mem_gam, mem_col, datarow = [0], [], [], [], [], []
-    mem_tpos, partial = [], False
+    mem_tpos, mem_par, partial = [], [], False
     for v in range(n):
         ci = node2cluster[v] - 1
         be = beliefs[ci]
@@ -226,16 +226,16 @@ def families_table(prenodes_info, node2cluster, node2family, node2fixed, beliefs
                     else:
                         mem_tpos.append(-1)
             if k == 0:
-                mem_len.append(0.0); mem_gam.append(1.0); mem_col.append(0)
+                mem_len.append(0.0); mem_gam.append(1.0); mem_col.append(0); mem_par.append(-1)
             else:
                 par = next(p for p in info["parents"] if p[0] == q)
-                mem_len.append(float(par[1])); mem_gam.append(float(par[2]))
+                mem_len.append(float(par[1])); mem_gam.append(float(par[2])); mem_par.append(int(par[0]) - 1)
                 mem_col.append(int(edge_color(par[3])) if edge_color else 0)
         mem_off.append(len(mem_pos))
         datarow.append(taxa.index(info["name"]) if (info["leaf"] and taxa is not None) else -1)
     out = dict(nnodes=n, ntips=len(taxa) if taxa is not None else 0, root_fixed=int(bool(root_fixed)),
                node_cluster=[c - 1 for c in node2cluster], mem_off=mem_off, mem_pos=mem_pos,
-               mem_length=mem_len, mem_gamma=mem_gam, mem_color=mem_col, node_datarow=datarow)
+               mem_length=mem_len, mem_gamma=mem_gam, mem_color=mem_col, node_datarow=datarow, mem_parent=mem_par)
     tm = None if tip_missing is None else np.ascontiguousarray(np.asarray(tip_missing, dtype=bool).reshape(out["ntips"], ntraits))
     if partial or (tm is not None and tm.any()):
         out["mem_tpos"] = mem_tpos
@@ -420,6 +420,39 @@ class BatchedClusterGraphBelief:
         self.lib.check(self.lib.pgbp_assign_factors_device(
             self.handle, int(ncolors), C.c_void_p(int(d_params_ptr)), int(nparamsets),
             C.c_void_p(int(d_tip_ptr)) if d_tip_ptr else None, int(ndatasets), pr))
+
+    def _mem_parent(self):
+        if getattr(self, "_mp", None) is None:  # the family table is static: converted once per batch
+            fam = self.plan.families
+            if fam is None or fam.get("mem_parent") is None:
+                raise ValueError("simulate needs the key 'mem_parent' in the plan's node-family table (plan.families)")
+            self._mp = _ia(fam["mem_parent"])
+        return self._mp
+
+    def simulate(self, params, seed, first_replicate=0, model="bm", ncolors=1, nodes=False):
+        """Trait replicates simulated down the network on the device (pgbp_simulate): element e is replicate
+        first_replicate + e of `seed`.  params: (nparamsets, len) records of bm_params (model="bm") or (sigma2, alpha,
+        theta, mu, v) (model="ou"), nparamsets in {1, B}.  Returns tipdata[B, ntips, p] (NaN where the plan's tip is
+        missing), and nodes[B, nnodes, p] (every node, preorder) when nodes=True."""
+        mp = self._mem_parent()
+        pa = np.ascontiguousarray(np.atleast_2d(np.asarray(params, dtype=float)))
+        fam, p = self.plan.families, self.plan.ntraits
+        tip = np.empty((self.B, int(fam["ntips"]), p))
+        nd = np.empty((self.B, int(fam["nnodes"]), p)) if nodes else None
+        self.lib.check(self.lib.pgbp_simulate(self.handle, {"bm": L.MODEL_BM, "ou": L.MODEL_OU}[model], int(ncolors),
+                                              mp[1], _fptr(pa), pa.shape[0], int(np.int64(np.uint64(seed))),
+                                              int(first_replicate), _fptr(tip), _fptr(nd)))
+        return (tip, nd) if nodes else tip
+
+    def simulate_device(self, d_params_ptr, nparamsets, seed, d_tip_ptr, d_nodes_ptr=None, first_replicate=0,
+                        model="bm", ncolors=1):
+        """simulate with device records and outputs (d_tip [B][ntips][p], d_nodes [B][nnodes][p]; either may be
+        None, not both), enqueue only."""
+        mp = self._mem_parent()
+        self.lib.check(self.lib.pgbp_simulate_device(
+            self.handle, {"bm": L.MODEL_BM, "ou": L.MODEL_OU}[model], int(ncolors), mp[1], C.c_void_p(int(d_params_ptr)),
+            int(nparamsets), int(np.int64(np.uint64(seed))), int(first_replicate),
+            C.c_void_p(int(d_tip_ptr)) if d_tip_ptr else None, C.c_void_p(int(d_nodes_ptr)) if d_nodes_ptr else None))
 
     def init_beliefs_reset(self):
         self.lib.check(self.lib.pgbp_reset_beliefs(self.handle))

@@ -20,9 +20,10 @@ SOURCES = [("pgbp_plan.cu", [], "pgbp_plan"), ("pgbp_batch.cu", [], "pgbp_batch"
            ("pgbp_message_t0.cu", ["PGBP_T0_PART=0"], "pgbp_message_t0_0"),
            ("pgbp_message_t0.cu", ["PGBP_T0_PART=1"], "pgbp_message_t0_1"),
            ("pgbp_message_t0.cu", ["PGBP_T0_PART=2"], "pgbp_message_t0_2"),
-           ("pgbp_shared.cu", [], "pgbp_shared")]
+           ("pgbp_shared.cu", [], "pgbp_shared"), ("pgbp_simulate.cu", [], "pgbp_simulate")]
 HEADERS = ["pgbp_backend.h", "pgbp_internal.h", "pgbp_kernels.cuh", "pgbp_launch.h", "pgbp_shapes.h", "pgbp_msg_t0.cuh",
-           "pgbp_coop.cuh", "pgbp_bulk.cuh", "pgbp_factors.cuh", os.path.join("..", "..", "include", "pgbp_b200.h")]
+           "pgbp_coop.cuh", "pgbp_bulk.cuh", "pgbp_factors.cuh", "pgbp_philox.h",
+           os.path.join("..", "..", "include", "pgbp_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

@@ -358,7 +358,7 @@ int32_t pgbp_batch_destroy(pgbp_batch* b) {
   stream_sync(b->stream);
   dev_free(b->state); dev_free(b->factor); dev_free(b->resid); dev_free(b->kldiv);
   dev_free(b->calflag); dev_free(b->calflagJ); dev_free(b->done); dev_free(b->status); dev_free(b->iscal); dev_free(b->itertree);
-  dev_free(b->d_tab); dev_free(b->d_one); dev_free(b->scratch); dev_free(b->d_slot); free_tables(b);
+  dev_free(b->d_tab); dev_free(b->d_one); dev_free(b->scratch); dev_free(b->d_slot); free_tables(b); sim_free(b);
   shared_destroy(b);
   for (auto* p : b->d_msgs) dev_free(p);
   for (auto* p : b->d_walk) dev_free(p);

@@ -231,4 +231,5 @@ struct pgbp_batch {
   size_t h_pinned_bytes = 0;
   int32_t* d_slot = nullptr;  // device scratch for transpose slot tables
   size_t d_slot_len = 0;
+  void* d_sim = nullptr;  // pgbp_simulate: node descriptors of the last mem_parent table (pgbp_simulate.cu)
 };

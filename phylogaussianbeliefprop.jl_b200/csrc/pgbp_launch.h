@@ -14,6 +14,7 @@ int soa_to_aos(pgbp_batch* b, const double* d_soa, int64_t ld, double* d_aos, in
 int integrate_launch(pgbp_batch* b, int belief, double* d_mu_soa, double* d_norm, int64_t ld_out, double* d_cov_soa = nullptr);
 int launch_group(pgbp_batch* b, MsgArgs a, const MsgDesc* d_msgs, const LaunchGroup& g);
 void free_tables(pgbp_batch* b);
+void sim_free(pgbp_batch* b);  // pgbp_simulate's cached node descriptors
 // write the pending zeros of the sepset rows (no-op unless sepsets_lazy_zero)
 int batch_materialize_sepsets(pgbp_batch* b);
 // the sepsets become zero: lazily when `lazy`, else with a memset now

@@ -213,11 +213,12 @@ def cliquetree_plan(net, ntraits, root_fixed=True, edge_color=None, name="synthe
     # node families (same table as pgbp_b200.families_table)
     tips = [v for v in range(n) if leaf[v]]
     row = {v: i for i, v in enumerate(tips)}
-    mem_off, mem_pos, mem_len, mem_gam, mem_col, datarow = [0], [], [], [], [], []
+    mem_off, mem_pos, mem_len, mem_gam, mem_col, mem_par, datarow = [0], [], [], [], [], [], []
     for v in range(n):
         fam = [(v, 0.0, 1.0, 0)] + sorted(parents[v], key=lambda t: -t[0])
         off = cl_off[cl_of[v]]
         for k, (q, L, g, e) in enumerate(fam):
+            mem_par.append(q if k else -1)
             mem_pos.append(-1 if fixed[q] else off[q])
             mem_len.append(L if k else 0.0)
             mem_gam.append(g if k else 1.0)
@@ -226,7 +227,7 @@ def cliquetree_plan(net, ntraits, root_fixed=True, edge_color=None, name="synthe
         datarow.append(row.get(v, -1))
     families = dict(nnodes=n, ntips=len(tips), root_fixed=int(bool(root_fixed)), node_cluster=list(cl_of),
                     mem_off=mem_off, mem_pos=mem_pos, mem_length=mem_len, mem_gamma=mem_gam, mem_color=mem_col,
-                    node_datarow=datarow)
+                    node_datarow=datarow, mem_parent=mem_par)
     return dict(name=name, ntraits=p, nclusters=nc, belief_dim=belief_dim, sepset_clusters=sepset_clusters,
                 upind=upind, trees=[[tp, tc]], families=families, root_cluster=hub,
                 simulate=[[[q, L, g] for (q, L, g, _) in parents[v]] for v in range(n)], tip_nodes=tips,
