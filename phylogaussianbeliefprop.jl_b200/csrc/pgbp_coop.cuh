@@ -240,6 +240,25 @@ __global__ void __launch_bounds__(128) k_message_coop(MsgArgs a) {
 //      new = J_KK - z_r.z_c, delta = new - old, three stores.
 // Per-entry update order and operands equal message_thread_t0 / message_thread_rt: bit-identical.
 // =====================================================================================
+// doubles of shared memory per element
+PGBP_HD int smem_doubles(int I, int S) { return I * (I + 1) / 2 + I * S + I; }
+// 16-bit index tables of one message, staged in shared memory (+ 4 entries of slack)
+PGBP_HD size_t smem_table_bytes(int I, int S) {
+  const int M = I + S;
+  return sizeof(uint16_t) * (size_t)(M * (M + 1) / 2 + M + S * (S + 1) / 2 + S + 4);
+}
+// bytes of shared memory per block (one warp) of k_message_smem<I>: element data + index tables
+PGBP_HD size_t smem_block_bytes(int I, int S) {
+  return sizeof(double) * 32 * (size_t)smem_doubles(I, S) + smem_table_bytes(I, S);
+}
+// bytes of shared memory per tile of k_message_smem_mw<I, NW, TILE, .>: factor rows + 2 scalar rows (x TILE lanes x
+// 8 bytes), per-lane int32 flags (active, failed pivot, one non-zero flag per warp), index tables; 16 bytes of slack
+// on narrow tiles
+PGBP_HD size_t smem_tile_bytes(int I, int S, int NW, int TILE) {
+  return sizeof(double) * TILE * (size_t)(smem_doubles(I, S) + 2) + sizeof(int32_t) * TILE * (size_t)(2 + NW) +
+         smem_table_bytes(I, S) + (TILE < 32 ? 16 : 0);
+}
+
 #ifndef PGBP_HOST_EMUL
 
 __device__ __forceinline__ void cp_async8(double* smem_dst, const double* gsrc) {
@@ -247,14 +266,139 @@ __device__ __forceinline__ void cp_async8(double* smem_dst, const double* gsrc) 
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(sa), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p)); }
 
-// doubles of shared memory per element
-inline __host__ __device__ int smem_doubles(int I, int S) { return I * (I + 1) / 2 + I * S + I; }
-// bytes of shared memory per block (one warp) of k_message_smem<I>: element data + index tables
-inline __host__ __device__ size_t smem_block_bytes(int I, int S) {
-  const int M = I + S;
-  return sizeof(double) * 32 * (size_t)smem_doubles(I, S) + sizeof(uint16_t) * (size_t)(M * (M + 1) / 2 + M + S * (S + 1) / 2 + S + 4);
-}
+// Phase C of every shared-memory kernel below: the kept block streamed like in message_thread_t0.  For a chunk of CH
+// kept entries the sender's J_KK (h_K) entry, the old sepset value and the old receiver value are loaded together,
+// then  nv = J_KK - z_r.z_c  (h_K - Z'w) with nfma over i ascending,  d = nv - old sepset,  and three stores: the
+// sepset gets nv, the receiver old + d, the residual d.  Per entry the operands and their order are those of
+// message_thread_t0 / message_thread_rt, so each kernel that streams through here is bit-identical to them.
+//   LS  lane stride of the Z tile: Z(k, cc) = Z[(cc * I + k) * LS], column S holds w = U^-T h_I
+//   MI  compile-time bound on the integrated dimension I (MI == I where I is a template argument: the guards fold)
+//   MS  0: S is a runtime value, chunks of PGBP_CHUNK entries; > 0: S <= MS, a kept column or the h part is one chunk
+//   T   element type of the index tables (uint16_t staged in shared memory, or int32_t read from global memory)
+template <int LS, int MI, int MS, class T>
+struct KeptStream {
+  static constexpr int CH = MS > 0 ? MS : PGBP_CHUNK;
+  const double* Z;
+  int I, S;
+  const T* gat;  // sender slots in [I;K] order: J (tri(M) entries), then h
+  const T* sca;  // receiver slots at the sepset's positions: J (tri(S) entries), then h
+  char* st;
+  char* rs;      // may be null
+  uint32_t ld8, fJ, fh, sJ, sh, tJ, th, rJ, rh;
+  bool sz;       // PGBP_OPT_SEPZERO: the old sepset is zero and not loaded
+
+  __device__ __forceinline__ KeptStream(const double* Z_, int I_, const MsgDesc& md, const T* gat_, const T* sca_,
+                                        char* st_, char* rs_, uint32_t ld8_, bool sz_)
+      : Z(Z_), I(I_), S(md.s), gat(gat_), sca(sca_), st(st_), rs(rs_), ld8(ld8_), fJ((uint32_t)md.fJ),
+        fh((uint32_t)md.fh), sJ((uint32_t)md.sJ), sh((uint32_t)md.sh), tJ((uint32_t)md.tJ), th((uint32_t)md.th),
+        rJ((uint32_t)md.rJ), rh((uint32_t)md.rh), sz(sz_) {}
+
+  // kept column cc: entries (rr, cc), rr = 0..cc.  (MS > 0: z_c is read after the column's loads and reused for the
+  // diagonal entry -- the same values, in the order that keeps the unrolled kernels at their register budget.)
+  __device__ __forceinline__ void column(int cc, double& maxJ) const {
+    double zc[MI];
+    auto load_zc = [&] {
+#pragma unroll
+      for (int i = 0; i < MI; i++) zc[i] = i < I ? Z[(cc * I + i) * LS] : 0.0;
+    };
+    if (MS == 0) load_zc();
+    const T* gc = gat + tri(I + cc) + I;  // sender slots of (I+rr, I+cc), rr = 0..cc
+    const int qc = tri(cc);
+    for (int r0 = 0; r0 <= cc; r0 += CH) {
+      double jo[CH], so[CH], to[CH];
+      double* ta[CH];
+#pragma unroll
+      for (int u = 0; u < CH; u++) {
+        const int rr = r0 + u;
+        if (rr <= cc) {
+          ta[u] = slot_ptr(st, tJ + sca[qc + rr], ld8);
+          jo[u] = *slot_ptr(st, fJ + gc[rr], ld8);
+          so[u] = sz ? 0.0 : *slot_ptr(st, sJ + qc + rr, ld8);
+          to[u] = *ta[u];
+        }
+      }
+      if (MS > 0) load_zc();
+#pragma unroll
+      for (int u = 0; u < CH; u++) {
+        const int rr = r0 + u;
+        if (rr <= cc) {
+          double nv = jo[u];
+          const double* zr = Z + rr * I * LS;
+#pragma unroll
+          for (int i = 0; i < MI; i++)
+            if (i < I) nv = nfma(MS > 0 && rr == cc ? zc[i] : zr[i * LS], zc[i], nv);
+          const double d = nv - so[u];
+          *slot_ptr(st, sJ + qc + rr, ld8) = nv;
+          *ta[u] = to[u] + d;
+          if (rs) *slot_ptr(rs, rJ + qc + rr, ld8) = d;
+          absmax(maxJ, d);
+        }
+      }
+      if (MS > 0) break;  // cc < MS: one chunk
+    }
+  }
+
+  // h entries in chunks [k0, k0 + CH), [k0 + kstep, k0 + kstep + CH), ...
+  __device__ __forceinline__ void hpart(int k0, int kstep, double& maxh) const {
+    double w[MI];
+#pragma unroll
+    for (int i = 0; i < MI; i++) w[i] = i < I ? Z[(S * I + i) * LS] : 0.0;
+    const T* gh = gat + tri(I + S) + I;
+    const T* sh_ = sca + tri(S);
+    for (; k0 < S; k0 += kstep) {
+      double ho[CH], so[CH], to[CH];
+      double* ta[CH];
+#pragma unroll
+      for (int u = 0; u < CH; u++) {
+        const int k = k0 + u;
+        if (k < S) {
+          ta[u] = slot_ptr(st, th + sh_[k], ld8);
+          ho[u] = *slot_ptr(st, fh + gh[k], ld8);
+          so[u] = sz ? 0.0 : *slot_ptr(st, sh + k, ld8);
+          to[u] = *ta[u];
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < CH; u++) {
+        const int k = k0 + u;
+        if (k < S) {
+          double nv = ho[u];
+          const double* zr = Z + k * I * LS;
+#pragma unroll
+          for (int i = 0; i < MI; i++)
+            if (i < I) nv = nfma(zr[i * LS], w[i], nv);
+          const double d = nv - so[u];
+          *slot_ptr(st, sh + k, ld8) = nv;
+          *ta[u] = to[u] + d;
+          if (rs) *slot_ptr(rs, rh + k, ld8) = d;
+          absmax(maxh, d);
+        }
+      }
+      if (MS > 0) break;  // S <= MS: one chunk
+    }
+  }
+
+  // L2 prefetch of everything column(cc) and h entry cc read (kept block of the sender, old sepset, old receiver):
+  // issued before the factorisation, the HBM -> L2 transfers overlap it and phase C then waits on L2 only.  UNROLL:
+  // unroll count of the loop over the column's entries (the single-warp kernel keeps it rolled, the multi-warp kernel
+  // unrolls it 4 x: measured on C5, rolled there it was 0.4 % slower)
+  template <int UNROLL>
+  __device__ __forceinline__ void prefetch(int cc) const {
+    const T* gc = gat + tri(I + cc) + I;
+    const int qc = tri(cc);
+#pragma unroll(UNROLL)
+    for (int rr = 0; rr <= cc; rr++) {
+      prefetch_l2(slot_ptr(st, fJ + gc[rr], ld8));
+      if (!sz) prefetch_l2(slot_ptr(st, sJ + qc + rr, ld8));
+      prefetch_l2(slot_ptr(st, tJ + sca[qc + rr], ld8));
+    }
+    prefetch_l2(slot_ptr(st, fh + gat[tri(I + S) + I + cc], ld8));
+    if (!sz) prefetch_l2(slot_ptr(st, sh + cc, ld8));
+    prefetch_l2(slot_ptr(st, th + sca[tri(S) + cc], ld8));
+  }
+};
 
 // TILE < 32: narrow tiles for shapes whose 32-element factor exceeds the SM's shared memory (C5's (32,16)
 // messages: 274 KB at 32 lanes, 206 KB at 24): lanes >= TILE idle, rows of TILE doubles (whole 32-byte sectors
@@ -272,10 +416,8 @@ __global__ void __launch_bounds__(32) k_message_smem_rt(MsgArgs a) {
   const int I = md.mF - md.s, S = md.s, M = md.mF;
   const int64_t ld = a.ld;
   double* st = a.state + e;
-  double* rs = a.resid ? a.resid + e : nullptr;
   const int32_t* __restrict__ gat = a.tab + md.gat;
-  const int32_t* __restrict__ sca = a.tab + md.sca;
-  const int TI = tri(I), SMM = tri(M), SS = tri(S);
+  const int TI = tri(I), SMM = tri(M);
   const int ZB = TI, WB = TI + I * S;  // region bases: Z(k, cc) = ZB + cc*I + k, w(k) = WB + k
 #define PGBP_SM(ent) sm[(ent) * TILE + tid]
 
@@ -351,80 +493,11 @@ __global__ void __launch_bounds__(32) k_message_smem_rt(MsgArgs a) {
   }
 
   // ---- C: stream the kept block ---------------------------------------------------------------
+  const KeptStream<TILE, MAXI, 0, int32_t> ks(&PGBP_SM(ZB), I, md, gat, a.tab + md.sca, (char*)st,
+                                              a.resid ? (char*)(a.resid + e) : nullptr, (uint32_t)(ld * 8), sz);
   double maxJ = 0.0, maxh = 0.0;
-  for (int cc = 0; cc < S; cc++) {
-    double zc[MAXI];
-#pragma unroll
-    for (int i = 0; i < MAXI; i++) zc[i] = i < I ? PGBP_SM(ZB + cc * I + i) : 0.0;
-    const int32_t* gc = gat + tri(I + cc) + I;  // sender slots of (I+rr, I+cc), rr = 0..cc
-    const int qc = tri(cc);
-    for (int r0 = 0; r0 <= cc; r0 += PGBP_CHUNK) {
-      double jo[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-      int64_t ta[PGBP_CHUNK];
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int rr = r0 + u;
-        if (rr <= cc) {
-          ta[u] = (md.tJ + sca[qc + rr]) * ld;
-          jo[u] = st[(md.fJ + gc[rr]) * ld];
-          so[u] = sz ? 0.0 : st[(md.sJ + qc + rr) * ld];
-          to[u] = st[ta[u]];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int rr = r0 + u;
-        if (rr <= cc) {
-          double nv = jo[u];
-          const int zb = ZB + rr * I;
-#pragma unroll
-          for (int i = 0; i < MAXI; i++)
-            if (i < I) nv = nfma(PGBP_SM(zb + i), zc[i], nv);
-          const double d = nv - so[u];
-          st[(md.sJ + qc + rr) * ld] = nv;
-          st[ta[u]] = to[u] + d;
-          if (rs) rs[(md.rJ + qc + rr) * ld] = d;
-          absmax(maxJ, d);
-        }
-      }
-    }
-  }
-  {
-    double w[MAXI];
-#pragma unroll
-    for (int i = 0; i < MAXI; i++) w[i] = i < I ? PGBP_SM(WB + i) : 0.0;
-    const int32_t* gh = gat + SMM + I;
-    for (int k0 = 0; k0 < S; k0 += PGBP_CHUNK) {
-      double ho[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-      int64_t ta[PGBP_CHUNK];
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          ta[u] = (md.th + sca[SS + k]) * ld;
-          ho[u] = st[(md.fh + gh[k]) * ld];
-          so[u] = sz ? 0.0 : st[(md.sh + k) * ld];
-          to[u] = st[ta[u]];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          double nv = ho[u];
-          const int zb = ZB + k * I;
-#pragma unroll
-          for (int i = 0; i < MAXI; i++)
-            if (i < I) nv = nfma(PGBP_SM(zb + i), w[i], nv);
-          const double d = nv - so[u];
-          st[(md.sh + k) * ld] = nv;
-          st[ta[u]] = to[u] + d;
-          if (rs) rs[(md.rh + k) * ld] = d;
-          absmax(maxh, d);
-        }
-      }
-    }
-  }
+  for (int cc = 0; cc < S; cc++) ks.column(cc, maxJ);
+  ks.hpart(0, PGBP_CHUNK, maxh);
   st[md.sg * ld] = g;
   st[md.tg * ld] = tg_old + (g - sg_old);
   store_flag(a, md.dmsg, e, S, maxJ, maxh);
@@ -443,12 +516,6 @@ __global__ void __launch_bounds__(32) k_message_smem_rt(MsgArgs a) {
 // The "all zero" test of src/beliefupdates.jl:62-66 is folded into the loads of phase B; a failed
 // pivot is only reported once the whole I-part has been seen to be non-zero.
 // -------------------------------------------------------------------------------------
-__device__ __forceinline__ double* gaddr(char* base, uint32_t slot, uint32_t ld8) {
-  return (double*)(base + (uint64_t)slot * (uint64_t)ld8);  // IMAD.WIDE.U32
-}
-
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p)); }
-
 // MS = 0: kept dimension S is a runtime value (loops over kept columns stay loops);
 // MS > 0: S <= MS and every loop over kept columns / rows is fully unrolled with uniform early exits --
 // straight-line code whose table offsets and shared-memory offsets are immediates and whose loads the
@@ -457,7 +524,7 @@ template <int I, int MS>
 __global__ void __launch_bounds__(32) k_message_smem(MsgArgs a) {
   extern __shared__ double sm[];
   const int tid = threadIdx.x;
-  const int64_t e0 = a.e0 + (int64_t)blockIdx.x * 32 + tid;
+  const int64_t e = a.e0 + (int64_t)blockIdx.x * 32 + tid;
   const MsgDesc md = a.msgs[blockIdx.y];
   const int S = md.s, M = md.mF;
   constexpr int TI = I * (I + 1) / 2;
@@ -475,25 +542,22 @@ __global__ void __launch_bounds__(32) k_message_smem(MsgArgs a) {
     for (int q = tid; q < nsca; q += 32) tsca[q] = (uint16_t)s0[q];
   }
   __syncwarp();
-  const int64_t e = e0;
   if (e >= a.B) return;  // (no warp-level synchronisation below this point)
   if (a.status[e] != 0) return;
   if (a.done && a.done[e]) return;
   const uint32_t ld8 = (uint32_t)(a.ld * 8);
   char* stb = (char*)(a.state + e);
-  char* rsb = a.resid ? (char*)(a.resid + e) : nullptr;
   const uint16_t* gat = tgat;
-  const uint16_t* sca = tsca;
-  const uint32_t fJ = (uint32_t)md.fJ, fh = (uint32_t)md.fh, sJ = (uint32_t)md.sJ, sh = (uint32_t)md.sh,
-                 tJ = (uint32_t)md.tJ, th = (uint32_t)md.th, rJ = (uint32_t)md.rJ, rh = (uint32_t)md.rh;
   double* smt = sm + tid;             // entry n of this thread: smt[n * 32]
   double* Z = smt + TI * 32;          // Z(k, cc) = Z[(cc * I + k) * 32]; column S holds h_I / w
+  const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
+  const KeptStream<32, I, MS, uint16_t> ks(Z, I, md, tgat, tsca, stb, a.resid ? (char*)(a.resid + e) : nullptr, ld8, sz);
 
   // ---- A: I-rows of the sender -> shared (asynchronous) ---------------------------------
 #pragma unroll
   for (int c = 0; c < I; c++) {
 #pragma unroll
-    for (int k = 0; k <= c; k++) cp_async8(smt + pk(k, c) * 32, gaddr(stb, fJ + gat[pk(k, c)], ld8));
+    for (int k = 0; k <= c; k++) cp_async8(smt + pk(k, c) * 32, slot_ptr(stb, ks.fJ + gat[pk(k, c)], ld8));
   }
 #pragma unroll(MS > 0 ? MS : 1)
   for (int cc = 0; cc < (MS > 0 ? MS : S); cc++) {
@@ -501,32 +565,19 @@ __global__ void __launch_bounds__(32) k_message_smem(MsgArgs a) {
     const uint16_t* gc = gat + tri(I + cc);
     double* zc = Z + cc * I * 32;
 #pragma unroll
-    for (int k = 0; k < I; k++) cp_async8(zc + k * 32, gaddr(stb, fJ + gc[k], ld8));
+    for (int k = 0; k < I; k++) cp_async8(zc + k * 32, slot_ptr(stb, ks.fJ + gc[k], ld8));
   }
   {
     double* zc = Z + S * I * 32;
 #pragma unroll
-    for (int k = 0; k < I; k++) cp_async8(zc + k * 32, gaddr(stb, fh + gat[SMM + k], ld8));
+    for (int k = 0; k < I; k++) cp_async8(zc + k * 32, slot_ptr(stb, ks.fh + gat[SMM + k], ld8));
   }
-  double g = *gaddr(stb, (uint32_t)md.fg, ld8);
-  const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
-  const double sg_old = sz ? 0.0 : *gaddr(stb, (uint32_t)md.sg, ld8), tg_old = *gaddr(stb, (uint32_t)md.tg, ld8);
-  // ---- L2 prefetch of everything phase C will read (kept block of the sender, old sepset, old
-  //      receiver): the HBM -> L2 transfers overlap phases A and B, phase C then waits on L2 only
+  double g = *slot_ptr(stb, (uint32_t)md.fg, ld8);
+  const double sg_old = sz ? 0.0 : *slot_ptr(stb, (uint32_t)md.sg, ld8), tg_old = *slot_ptr(stb, (uint32_t)md.tg, ld8);
 #pragma unroll(MS > 0 ? MS : 1)
   for (int cc = 0; cc < (MS > 0 ? MS : S); cc++) {
     if (MS > 0 && cc >= S) break;
-    const uint16_t* gc = gat + tri(I + cc) + I;
-    const int qc = tri(cc);
-#pragma unroll(MS > 0 ? MS : 1)
-    for (int rr = 0; rr <= cc; rr++) {
-      prefetch_l2(gaddr(stb, fJ + gc[rr], ld8));
-      if (!sz) prefetch_l2(gaddr(stb, sJ + qc + rr, ld8));
-      prefetch_l2(gaddr(stb, tJ + sca[qc + rr], ld8));
-    }
-    prefetch_l2(gaddr(stb, fh + gat[SMM + I + cc], ld8));
-    if (!sz) prefetch_l2(gaddr(stb, sh + cc, ld8));
-    prefetch_l2(gaddr(stb, th + sca[SS + cc], ld8));
+    ks.template prefetch<(MS > 0 ? MS : 1)>(cc);
   }
   cp_async_wait_all();
 
@@ -606,461 +657,65 @@ __global__ void __launch_bounds__(32) k_message_smem(MsgArgs a) {
 
   // ---- C: stream the kept block ---------------------------------------------------------------
   double maxJ = 0.0, maxh = 0.0;
-  if constexpr (MS > 0) {
 #pragma unroll
-    for (int cc = 0; cc < MS; cc++) {
-      if (cc >= S) break;
-      const uint16_t* gc = gat + tri(I + cc) + I;  // sender slots of (I+rr, I+cc), rr = 0..cc
-      const int qc = tri(cc);
-      double jo[MS], so[MS], to[MS];
-      double* ta[MS];
-#pragma unroll
-      for (int rr = 0; rr <= cc; rr++) {
-        ta[rr] = gaddr(stb, tJ + sca[qc + rr], ld8);
-        jo[rr] = *gaddr(stb, fJ + gc[rr], ld8);
-        so[rr] = sz ? 0.0 : *gaddr(stb, sJ + qc + rr, ld8);
-        to[rr] = *ta[rr];
-      }
-      double zc[I];
-#pragma unroll
-      for (int i = 0; i < I; i++) zc[i] = Z[(cc * I + i) * 32];
-#pragma unroll
-      for (int rr = 0; rr <= cc; rr++) {
-        double nv = jo[rr];
-#pragma unroll
-        for (int i = 0; i < I; i++) nv = nfma(rr == cc ? zc[i] : Z[(rr * I + i) * 32], zc[i], nv);
-        const double d = nv - so[rr];
-        *gaddr(stb, sJ + qc + rr, ld8) = nv;
-        *ta[rr] = to[rr] + d;
-        if (rsb) *gaddr(rsb, rJ + qc + rr, ld8) = d;
-        absmax(maxJ, d);
-      }
-    }
-    {
-      double w[I];
-#pragma unroll
-      for (int i = 0; i < I; i++) w[i] = Z[(S * I + i) * 32];
-      const uint16_t* gh = gat + SMM + I;
-      double ho[MS], so[MS], to[MS];
-      double* ta[MS];
-#pragma unroll
-      for (int k = 0; k < MS; k++) {
-        if (k < S) {
-          ta[k] = gaddr(stb, th + sca[SS + k], ld8);
-          ho[k] = *gaddr(stb, fh + gh[k], ld8);
-          so[k] = sz ? 0.0 : *gaddr(stb, sh + k, ld8);
-          to[k] = *ta[k];
-        }
-      }
-#pragma unroll
-      for (int k = 0; k < MS; k++) {
-        if (k < S) {
-          double nv = ho[k];
-#pragma unroll
-          for (int i = 0; i < I; i++) nv = nfma(Z[(k * I + i) * 32], w[i], nv);
-          const double d = nv - so[k];
-          *gaddr(stb, sh + k, ld8) = nv;
-          *ta[k] = to[k] + d;
-          if (rsb) *gaddr(rsb, rh + k, ld8) = d;
-          absmax(maxh, d);
-        }
-      }
-    }
-  } else {
-  for (int cc = 0; cc < S; cc++) {
-    double zc[I];
-#pragma unroll
-    for (int i = 0; i < I; i++) zc[i] = Z[(cc * I + i) * 32];
-    const uint16_t* gc = gat + tri(I + cc) + I;  // sender slots of (I+rr, I+cc), rr = 0..cc
-    const int qc = tri(cc);
-    for (int r0 = 0; r0 <= cc; r0 += PGBP_CHUNK) {
-      double jo[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-      double* ta[PGBP_CHUNK];
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int rr = r0 + u;
-        if (rr <= cc) {
-          ta[u] = gaddr(stb, tJ + sca[qc + rr], ld8);
-          jo[u] = *gaddr(stb, fJ + gc[rr], ld8);
-          so[u] = sz ? 0.0 : *gaddr(stb, sJ + qc + rr, ld8);
-          to[u] = *ta[u];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int rr = r0 + u;
-        if (rr <= cc) {
-          double nv = jo[u];
-          const double* zr = Z + rr * I * 32;
-#pragma unroll
-          for (int i = 0; i < I; i++) nv = nfma(zr[i * 32], zc[i], nv);
-          const double d = nv - so[u];
-          *gaddr(stb, sJ + qc + rr, ld8) = nv;
-          *ta[u] = to[u] + d;
-          if (rsb) *gaddr(rsb, rJ + qc + rr, ld8) = d;
-          absmax(maxJ, d);
-        }
-      }
-    }
+  for (int cc = 0; cc < (MS > 0 ? MS : S); cc++) {
+    if (MS > 0 && cc >= S) break;
+    ks.column(cc, maxJ);
   }
-  {
-    double w[I];
-#pragma unroll
-    for (int i = 0; i < I; i++) w[i] = Z[(S * I + i) * 32];
-    const uint16_t* gh = gat + SMM + I;
-    for (int k0 = 0; k0 < S; k0 += PGBP_CHUNK) {
-      double ho[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-      double* ta[PGBP_CHUNK];
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          ta[u] = gaddr(stb, th + sca[SS + k], ld8);
-          ho[u] = *gaddr(stb, fh + gh[k], ld8);
-          so[u] = sz ? 0.0 : *gaddr(stb, sh + k, ld8);
-          to[u] = *ta[u];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          double nv = ho[u];
-          const double* zr = Z + k * I * 32;
-#pragma unroll
-          for (int i = 0; i < I; i++) nv = nfma(zr[i * 32], w[i], nv);
-          const double d = nv - so[u];
-          *gaddr(stb, sh + k, ld8) = nv;
-          *ta[u] = to[u] + d;
-          if (rsb) *gaddr(rsb, rh + k, ld8) = d;
-          absmax(maxh, d);
-        }
-      }
-    }
-  }
-  }
-  *gaddr(stb, (uint32_t)md.sg, ld8) = g;
-  *gaddr(stb, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
+  ks.hpart(0, ks.CH, maxh);
+  *slot_ptr(stb, (uint32_t)md.sg, ld8) = g;
+  *slot_ptr(stb, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
   store_flag(a, md.dmsg, e, S, maxJ, maxh);
 }
 
 // -------------------------------------------------------------------------------------
 // Multi-warp version of k_message_smem for LARGE integrated dimensions (I >= 12: C5's (16,16) and (16,32)
-// messages).  There the factor of 32 elements fills 100-175 KB of shared memory, so only one or two
-// single-warp blocks fit an SM and every phase runs at the latency of its own dependent chain
-// (profiles/r1_c5_launches.txt: 49 % of the C5 step).  Here NW warps share ONE tile of 32 elements (lane =
-// element, as before) and split the work by COLUMN: the asynchronous staging (phase A) by entry, the
-// right-hand sides of Z = U^-T [J_IK | h_I] (phase B2) and the kept columns of the streamed Schur
-// complement (phase C, paired cc / S-1-cc for balance) by warp; only the Cholesky of J_II (phase B1,
-// ~12 % of the flops) stays on warp 0.  Same shared-memory footprint, NW x the warps per SM.
-// NW = 4 (two tiles per SM, full register budget) when two tiles fit the SM's shared memory, else NW = 8
-// (one tile per SM).  Measured on C5 (B200): single-warp tiles 490 ms per calibration step, 8 warps at
-// 128 registers 389 ms, 4 warps at 255 registers 356 ms.
+// messages, C4's (16,8); I = 32: C5's (32,16)).  There the factor of 32 elements fills 100-175 KB of shared memory
+// (274 KB at I = 32), so only one or two single-warp blocks fit an SM and every phase runs at the latency of its own
+// dependent chain (profiles/r1_c5_launches.txt: 49 % of the C5 step).  Here NW warps share ONE tile of TILE elements
+// (lane = element, as before) and split the work by COLUMN: the asynchronous staging (phase A) by entry, the
+// right-hand sides of Z = U^-T [J_IK | h_I] (phase B2) and the kept columns of the streamed Schur complement
+// (phase C, paired cc / S-1-cc for balance) by warp.  Same shared-memory footprint, NW x the warps per SM.
+// The Cholesky of J_II (phase B1) comes in two forms:
+//   COLPAR = false  on warp 0, left-looking and fully unrolled as in k_message_smem (~12 % of the flops at I = 16);
+//                   1/U_cc is kept in the (otherwise unused) diagonal slot of U for the other warps
+//   COLPAR = true   right-looking, one block barrier per pivot: the owner of column c (c mod NW) applies pivot k to
+//                   its column, A[r,c] -= u_kr u_kc with u_k. = A[k,.] / sqrt(A[k,k]) formed on the fly (row k is not
+//                   written during step k); rows are scaled in place afterwards.  For I = 32, where B1 is 29 % of
+//                   the flops and would otherwise serialise the tile on one warp.  Per entry the updates arrive in
+//                   ascending k with the same operands as in the left-looking form.
+// Used as <I, 4 or 8, 32, false> for I = 12..16: NW = 4 (two tiles per SM, full register budget) when two tiles fit
+// the SM's shared memory, else NW = 8 (one tile per SM); measured on C5 (B200): single-warp tiles 490 ms per
+// calibration step, 8 warps at 128 registers 389 ms, 4 warps at 255 registers 356 ms.  And as <32, 8, 24, true>:
+// the 32-element factor does not fit, tiles of 24 elements (lanes 24..31 idle; rows of 24 doubles = six whole
+// 32-byte sectors) and ONE tile of 206 KB per SM, so all the parallelism has to come from inside the tile.
 // Every entry is still produced by one thread with the same operands in the same order: bit-identical.
 // -------------------------------------------------------------------------------------
-// shared memory of one tile: factor rows + 2 scalar rows (x 32 lanes x 8 bytes), per-lane flags, index tables
-inline __host__ __device__ size_t smem_mw_block_bytes(int I, int S, int NW) {
-  const int M = I + S;
-  return sizeof(double) * 32 * (size_t)(smem_doubles(I, S) + 2) + sizeof(int32_t) * 32 * (size_t)(2 + NW) +
-         sizeof(uint16_t) * (size_t)(M * (M + 1) / 2 + M + S * (S + 1) / 2 + S + 4);
-}
-
-template <int I, int NW, int MINB = (NW <= 4 ? 2 : 1)>
-__global__ void __launch_bounds__(32 * NW, MINB) k_message_smem_mw(MsgArgs a) {
+template <int I, int NW, int TILE, bool COLPAR>
+__global__ void __launch_bounds__(32 * NW, NW <= 4 ? 2 : 1) k_message_smem_mw(MsgArgs a) {
+  constexpr int TI = I * (I + 1) / 2;
+  static_assert(2 * NW <= TI, "the flag reduction reuses rows [0, 2 NW) of U");
   extern __shared__ __align__(128) double sm[];  // bulk-copy destinations need 16-byte alignment
   __shared__ __align__(8) unsigned long long mbar;
   const int tid = threadIdx.x, wid = threadIdx.y;
   if (wid == 0 && tid == 0) mbar_init(&mbar, 1);  // (made visible to the other threads by the barrier after the tables)
-  const int64_t e = a.e0 + (int64_t)blockIdx.x * 32 + tid;
+  const bool lane_ok = TILE == 32 || tid < TILE;
+  const int lane = lane_ok ? tid : 0;      // idle lanes never touch shared memory (all accesses are guarded)
+  const int64_t tile0 = a.e0 + (int64_t)blockIdx.x * TILE, e = tile0 + lane;
   const MsgDesc md = a.msgs[blockIdx.y];
   const int S = md.s, M = md.mF;
-  constexpr int TI = I * (I + 1) / 2;
   const int SMM = tri(M), SS = tri(S);
   const int nrhs = S + 1;
   const int NE = TI + I * nrhs;            // staged entries per element
-  // shared layout: rows of 32 lanes: [0, NE) factor | ww | logdet; then per-lane int32 flags
-  // ([tid] active, [32 + tid] failed pivot, [64 + 32 w + tid] warp w saw a non-zero), then the index tables.
-  // 1/U_cc is kept in the (otherwise unused) diagonal slot of U; the flag reduction of phase C reuses
-  // rows of U, which is dead by then.
-  double* smt = sm + tid;
-  double* Z = smt + TI * 32;               // Z(k, cc) = Z[(cc * I + k) * 32]; column S holds h_I / w
-  double* s_ww = smt + NE * 32;
-  double* s_logdet = s_ww + 32;
-  double* s_redJ = smt;                    // rows [0, NW) and [NW, 2 NW) of U (2 NW <= TI)
-  double* s_redh = smt + NW * 32;
-  int32_t* s_flag = (int32_t*)(sm + 32 * (NE + 2));
-  uint16_t* tgat = (uint16_t*)(s_flag + 32 * (2 + NW));
-  const int ngat = SMM + M, nsca = SS + S;
-  uint16_t* tsca = tgat + ngat;
-  {
-    const int32_t* __restrict__ g0 = a.tab + md.gat;
-    const int32_t* __restrict__ s0 = a.tab + md.sca;
-    for (int q = wid * 32 + tid; q < ngat; q += 32 * NW) tgat[q] = (uint16_t)g0[q];
-    for (int q = wid * 32 + tid; q < nsca; q += 32 * NW) tsca[q] = (uint16_t)s0[q];
-    if (wid == 0) {
-      int act = e < a.B;
-      if (act && a.status[e] != 0) act = 0;
-      if (act && a.done && a.done[e]) act = 0;
-      s_flag[tid] = act;
-      s_flag[32 + tid] = 0;
-    }
-  }
-  __syncthreads();
-  const bool active = s_flag[tid] != 0;    // same answer in every warp of the tile
-  const int64_t ee = active ? e : a.e0 + (int64_t)blockIdx.x * 32;  // inactive lanes shadow a valid element, never store
-  const uint32_t ld8 = (uint32_t)(a.ld * 8);
-  char* stb = (char*)(a.state + ee);
-  char* rsb = a.resid ? (char*)(a.resid + ee) : nullptr;
-  const uint16_t* gat = tgat;
-  const uint16_t* sca = tsca;
-  const uint32_t fJ = (uint32_t)md.fJ, fh = (uint32_t)md.fh, sJ = (uint32_t)md.sJ, sh = (uint32_t)md.sh,
-                 tJ = (uint32_t)md.tJ, th = (uint32_t)md.th, rJ = (uint32_t)md.rJ, rh = (uint32_t)md.rh;
-  const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
-
-  // ---- A: staging with bulk asynchronous copies: one 256-byte row (32 elements of one slot) per instruction,
-  //      rows dealt to the threads of the tile, completion counted in bytes on the tile's mbarrier ----------
-  {
-    const char* tileb = (const char*)(a.state + a.e0 + (int64_t)blockIdx.x * 32);
-    if (wid == 0 && tid == 0) mbar_expect_tx(&mbar, (unsigned)NE * 256u);
-    for (int n = wid * 32 + tid; n < NE; n += 32 * NW) {
-      uint32_t slot;
-      if (n < TI) slot = fJ + gat[n];
-      else {
-        const int idx = n - TI, cc = idx / I, k = idx - cc * I;
-        slot = cc < S ? fJ + gat[tri(I + cc) + k] : fh + gat[SMM + k];
-      }
-      bulk_g2s(sm + n * 32, tileb + (uint64_t)slot * (uint64_t)ld8, 256u, &mbar);
-    }
-  }
-  double g = 0.0, sg_old = 0.0, tg_old = 0.0;
-  if (wid == 0) {
-    g = *gaddr(stb, (uint32_t)md.fg, ld8);
-    sg_old = sz ? 0.0 : *gaddr(stb, (uint32_t)md.sg, ld8);
-    tg_old = *gaddr(stb, (uint32_t)md.tg, ld8);
-  }
-  // L2 prefetch of what phase C reads, by kept column
-  for (int cc = wid; cc < S; cc += NW) {
-    const uint16_t* gc = gat + tri(I + cc) + I;
-    const int qc = tri(cc);
-    for (int rr = 0; rr <= cc; rr++) {
-      prefetch_l2(gaddr(stb, fJ + gc[rr], ld8));
-      if (!sz) prefetch_l2(gaddr(stb, sJ + qc + rr, ld8));
-      prefetch_l2(gaddr(stb, tJ + sca[qc + rr], ld8));
-    }
-    prefetch_l2(gaddr(stb, fh + gat[SMM + I + cc], ld8));
-    if (!sz) prefetch_l2(gaddr(stb, sh + cc, ld8));
-    prefetch_l2(gaddr(stb, th + sca[SS + cc], ld8));
-  }
-  mbar_wait(&mbar, 0);  // every staged row has landed (async-proxy writes are visible after the wait)
-  __syncthreads();
-
-  // ---- B1: U'U = J_II on warp 0 (left-looking, fully unrolled; as k_message_smem) ----------------
-  bool nz = false;
-  if (wid == 0) {
-    double rinv[I];
-    double logdet = 0.0;
-    int fail = 0;
-#pragma unroll
-    for (int c = 0; c < I; c++) {
-      double v[I];
-#pragma unroll
-      for (int k = 0; k <= c; k++) {
-        v[k] = smt[pk(k, c) * 32];
-        if (!(fabs(v[k]) <= PGBP_EPS)) nz = true;
-      }
-#pragma unroll
-      for (int k = 0; k < c; k++) {
-        const double u = v[k] * rinv[k];
-        v[k] = u;
-        smt[pk(k, c) * 32] = u;
-#pragma unroll
-        for (int r = k + 1; r <= c; r++) v[r] = nfma(r == c ? u : smt[pk(k, r) * 32], u, v[r]);
-      }
-      const double d = v[c];
-      if (!(d > 0.0) && fail == 0) fail = c + 1;
-      logdet += log(d);
-      rinv[c] = 1.0 / sqrt(d);
-      smt[pk(c, c) * 32] = rinv[c];
-    }
-    s_logdet[0] = logdet;
-    s_flag[32 + tid] = fail;
-  }
-  __syncthreads();
-
-  // ---- B2: Z = U^-T [J_IK | h_I], right-hand sides dealt to the warps ---------------------------
-  {
-    double rinv[I];
-#pragma unroll
-    for (int k = 0; k < I; k++) rinv[k] = smt[pk(k, k) * 32];
-    for (int c0 = wid; c0 < nrhs; c0 += NW) {
-      double* z0 = Z + c0 * I * 32;
-      double v0[I];
-#pragma unroll
-      for (int k = 0; k < I; k++) {
-        v0[k] = z0[k * 32];
-        if (!(fabs(v0[k]) <= PGBP_EPS)) nz = true;
-      }
-#pragma unroll
-      for (int k = 0; k < I; k++) {
-        const double u0 = v0[k] * rinv[k];
-        v0[k] = u0;
-#pragma unroll
-        for (int r = k + 1; r < I; r++) v0[r] = nfma(smt[pk(k, r) * 32], u0, v0[r]);
-      }
-#pragma unroll
-      for (int k = 0; k < I; k++) z0[k * 32] = v0[k];
-      if (c0 == S) {  // the h column: w = U^-T h_I
-        double ww = 0.0;
-#pragma unroll
-        for (int k = 0; k < I; k++) ww = fma(v0[k], v0[k], ww);
-        s_ww[0] = ww;
-      }
-    }
-  }
-  s_flag[64 + wid * 32 + tid] = nz ? 1 : 0;
-  __syncthreads();
-  bool nzall = false;
-#pragma unroll
-  for (int w = 0; w < NW; w++) nzall = nzall || s_flag[64 + w * 32 + tid] != 0;
-  const int fail = s_flag[32 + tid];
-  const bool dead = !active || (nzall && fail != 0);
-  if (nzall) {
-    if (fail && active && wid == 0) status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, fail));
-    if (wid == 0) g += 0.5 * ((double)I * PGBP_LOG2PI - s_logdet[0] + s_ww[0]);
-  } else {  // "missing data" shortcut: message = (h_K, J_KK, g) unchanged
-    for (int q = wid; q < nrhs * I; q += NW) Z[q * 32] = 0.0;
-  }
-  __syncthreads();
-
-  // ---- C: stream the kept block, kept columns paired (j, S-1-j) and dealt to the warps ------------
-  double maxJ = 0.0, maxh = 0.0;
-  const int half = (S + 1) / 2;
-  for (int j = wid; j < half && !dead; j += NW) {
-    for (int side = 0; side < 2; side++) {
-      const int cc = side == 0 ? j : S - 1 - j;
-      if (side == 1 && cc == j) break;
-      double zc[I];
-#pragma unroll
-      for (int i = 0; i < I; i++) zc[i] = Z[(cc * I + i) * 32];
-      const uint16_t* gc = gat + tri(I + cc) + I;
-      const int qc = tri(cc);
-      for (int r0 = 0; r0 <= cc; r0 += PGBP_CHUNK) {
-        double jo[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-        double* ta[PGBP_CHUNK];
-#pragma unroll
-        for (int u = 0; u < PGBP_CHUNK; u++) {
-          const int rr = r0 + u;
-          if (rr <= cc) {
-            ta[u] = gaddr(stb, tJ + sca[qc + rr], ld8);
-            jo[u] = *gaddr(stb, fJ + gc[rr], ld8);
-            so[u] = sz ? 0.0 : *gaddr(stb, sJ + qc + rr, ld8);
-            to[u] = *ta[u];
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < PGBP_CHUNK; u++) {
-          const int rr = r0 + u;
-          if (rr <= cc) {
-            double nv = jo[u];
-            const double* zr = Z + rr * I * 32;
-#pragma unroll
-            for (int i = 0; i < I; i++) nv = nfma(zr[i * 32], zc[i], nv);
-            const double d = nv - so[u];
-            *gaddr(stb, sJ + qc + rr, ld8) = nv;
-            *ta[u] = to[u] + d;
-            if (rsb) *gaddr(rsb, rJ + qc + rr, ld8) = d;
-            absmax(maxJ, d);
-          }
-        }
-      }
-    }
-  }
-  if (!dead) {  // h part: chunks of kept entries dealt to the warps, last warp first (it has the lightest J share)
-    double w[I];
-#pragma unroll
-    for (int i = 0; i < I; i++) w[i] = Z[(S * I + i) * 32];
-    const uint16_t* gh = gat + SMM + I;
-    for (int k0 = (NW - 1 - wid) * PGBP_CHUNK; k0 < S; k0 += NW * PGBP_CHUNK) {
-      double ho[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-      double* ta[PGBP_CHUNK];
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          ta[u] = gaddr(stb, th + sca[SS + k], ld8);
-          ho[u] = *gaddr(stb, fh + gh[k], ld8);
-          so[u] = sz ? 0.0 : *gaddr(stb, sh + k, ld8);
-          to[u] = *ta[u];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          double nv = ho[u];
-          const double* zr = Z + k * I * 32;
-#pragma unroll
-          for (int i = 0; i < I; i++) nv = nfma(zr[i * 32], w[i], nv);
-          const double d = nv - so[u];
-          *gaddr(stb, sh + k, ld8) = nv;
-          *ta[u] = to[u] + d;
-          if (rsb) *gaddr(rsb, rh + k, ld8) = d;
-          absmax(maxh, d);
-        }
-      }
-    }
-  }
-  s_redJ[wid * 32] = maxJ;
-  s_redh[wid * 32] = maxh;
-  __syncthreads();
-  if (wid == 0 && !dead) {
-    double mJ = 0.0, mh = 0.0;
-#pragma unroll
-    for (int w = 0; w < NW; w++) {  // NaN-propagating maximum, like absmax
-      const double xj = s_redJ[w * 32], xh = s_redh[w * 32];
-      if (xj > mJ || xj != xj) mJ = xj;
-      if (xh > mh || xh != xh) mh = xh;
-    }
-    *gaddr(stb, (uint32_t)md.sg, ld8) = g;
-    *gaddr(stb, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
-    store_flag(a, md.dmsg, e, S, mJ, mh);
-  }
-}
-
-// -------------------------------------------------------------------------------------
-// Multi-warp kernel for integrated dimension 32 (C5's (32,16) messages: sender dimension 48).  The factor of
-// 32 elements needs 274 KB of shared memory, so the tile is TILE = 24 elements (lanes 24..31 idle; rows of
-// 24 doubles = six whole 32-byte sectors) and ONE tile of 206 KB occupies the SM: all the parallelism has to
-// come from inside the tile.  NW = 8 warps split every phase by column -- including the Cholesky of J_II,
-// which at I = 32 is 29 % of the flops and would otherwise serialise the tile on one warp:
-//   B1  right-looking, one block barrier per pivot: the owner of column c (c mod NW) applies pivot k to its
-//       column, A[r,c] -= u_kr u_kc with u_k. = A[k,.] / sqrt(A[k,k]) formed on the fly (row k is not
-//       written during step k); rows are scaled in place afterwards.  Per entry the updates arrive in
-//       ascending k with the same operands as in the left-looking form: bit-identical to every other kernel.
-//   B2 / C  as in k_message_smem_mw.
-// -------------------------------------------------------------------------------------
-template <int I, int NW, int TILE>
-__global__ void __launch_bounds__(32 * NW, 1) k_message_smem_mwp(MsgArgs a) {
-  extern __shared__ __align__(128) double sm[];  // bulk-copy destinations need 16-byte alignment
-  __shared__ __align__(8) unsigned long long mbar;
-  const int tid = threadIdx.x, wid = threadIdx.y;
-  if (wid == 0 && tid == 0) mbar_init(&mbar, 1);  // (made visible to the other threads by the barrier after the tables)
-  const bool lane_ok = tid < TILE;
-  const int lane = lane_ok ? tid : 0;      // idle lanes never touch shared memory (all accesses are guarded)
-  const int64_t e = a.e0 + (int64_t)blockIdx.x * TILE + lane;
-  const MsgDesc md = a.msgs[blockIdx.y];
-  const int S = md.s, M = md.mF;
-  constexpr int TI = I * (I + 1) / 2;
-  const int SMM = tri(M), SS = tri(S);
-  const int nrhs = S + 1;
-  const int NE = TI + I * nrhs;
+  // shared layout (smem_tile_bytes): rows of TILE lanes: [0, NE) factor | ww | logdet; then per-lane int32 flags
+  // ([lane] active, [TILE + lane] failed pivot, [(2 + w) TILE + lane] warp w saw a non-zero), then the index tables.
   double* smt = sm + lane;                 // entry n of this lane: smt[n * TILE]
   double* Z = smt + TI * TILE;             // Z(k, cc) = Z[(cc * I + k) * TILE]; column S holds h_I / w
   double* s_ww = smt + NE * TILE;
   double* s_logdet = s_ww + TILE;
-  double* s_redJ = smt;                    // rows [0, NW) / [NW, 2 NW) of U, dead by the end of phase C
+  double* s_redJ = smt;                    // rows [0, NW) and [NW, 2 NW) of U, dead in phase C
   double* s_redh = smt + NW * TILE;
-  int32_t* s_flag = (int32_t*)(sm + TILE * (NE + 2));  // [lane] active, [TILE + lane] failed pivot, [(2 + w) TILE + lane] nz
+  int32_t* s_flag = (int32_t*)(sm + TILE * (NE + 2));
   uint16_t* tgat = (uint16_t*)(s_flag + TILE * (2 + NW));
   const int ngat = SMM + M, nsca = SS + S;
   uint16_t* tsca = tgat + ngat;
@@ -1078,115 +733,138 @@ __global__ void __launch_bounds__(32 * NW, 1) k_message_smem_mwp(MsgArgs a) {
     }
   }
   __syncthreads();
-  const bool active = lane_ok && s_flag[lane] != 0;
-  const int64_t ee = active ? e : a.e0 + (int64_t)blockIdx.x * TILE;  // inactive lanes shadow a valid element, never store
+  const bool active = lane_ok && s_flag[lane] != 0;  // same answer in every warp of the tile
+  const int64_t ee = active ? e : tile0;   // inactive lanes shadow a valid element, never store
   const uint32_t ld8 = (uint32_t)(a.ld * 8);
   char* stb = (char*)(a.state + ee);
-  char* rsb = a.resid ? (char*)(a.resid + ee) : nullptr;
-  const uint16_t* gat = tgat;
-  const uint16_t* sca = tsca;
-  const uint32_t fJ = (uint32_t)md.fJ, fh = (uint32_t)md.fh, sJ = (uint32_t)md.sJ, sh = (uint32_t)md.sh,
-                 tJ = (uint32_t)md.tJ, th = (uint32_t)md.th, rJ = (uint32_t)md.rJ, rh = (uint32_t)md.rh;
   const bool sz = (a.opts & PGBP_OPT_SEPZERO) != 0;
+  const KeptStream<TILE, I, 0, uint16_t> ks(Z, I, md, tgat, tsca, stb, a.resid ? (char*)(a.resid + ee) : nullptr, ld8, sz);
 
-  // ---- A: staging with bulk asynchronous copies: one row of TILE elements (8 TILE bytes, 16-byte aligned) per
-  //      instruction, rows dealt to the threads of the tile, completion counted in bytes on the tile's mbarrier -----
-  double g = 0.0, sg_old = 0.0, tg_old = 0.0;
+  // ---- A: staging with bulk asynchronous copies: one row of the tile (TILE elements of one slot) per instruction,
+  //      rows dealt to the threads of the tile, completion counted in bytes on the tile's mbarrier ----------
   {
-    const int64_t tile0 = a.e0 + (int64_t)blockIdx.x * TILE;
     const char* tileb = (const char*)(a.state + tile0);
-    const int64_t room = a.ld - tile0;  // the last tile of a row may be cut by the row pitch
-    const unsigned rowbytes = (unsigned)((room < TILE ? room : TILE) * 8);
+    unsigned rowbytes = 8u * TILE;
+    if (TILE < 32) {  // the last narrow tile of a row may be cut by the row pitch (a multiple of 32 elements)
+      const int64_t room = a.ld - tile0;
+      if (room < TILE) rowbytes = (unsigned)(room * 8);
+    }
     if (wid == 0 && tid == 0) mbar_expect_tx(&mbar, (unsigned)NE * rowbytes);
     for (int n = wid * 32 + tid; n < NE; n += 32 * NW) {
       uint32_t slot;
-      if (n < TI) slot = fJ + gat[n];
+      if (n < TI) slot = ks.fJ + tgat[n];
       else {
         const int idx = n - TI, cc = idx / I, k = idx - cc * I;
-        slot = cc < S ? fJ + gat[tri(I + cc) + k] : fh + gat[SMM + k];
+        slot = cc < S ? ks.fJ + tgat[tri(I + cc) + k] : ks.fh + tgat[SMM + k];
       }
       bulk_g2s(sm + n * TILE, tileb + (uint64_t)slot * (uint64_t)ld8, rowbytes, &mbar);
     }
   }
+  double g = 0.0, sg_old = 0.0, tg_old = 0.0;
   if (lane_ok) {
     if (wid == 0) {
-      g = *gaddr(stb, (uint32_t)md.fg, ld8);
-      sg_old = sz ? 0.0 : *gaddr(stb, (uint32_t)md.sg, ld8);
-      tg_old = *gaddr(stb, (uint32_t)md.tg, ld8);
+      g = *slot_ptr(stb, (uint32_t)md.fg, ld8);
+      sg_old = sz ? 0.0 : *slot_ptr(stb, (uint32_t)md.sg, ld8);
+      tg_old = *slot_ptr(stb, (uint32_t)md.tg, ld8);
     }
-    for (int cc = wid; cc < S; cc += NW) {  // L2 prefetch of what phase C reads
-      const uint16_t* gc = gat + tri(I + cc) + I;
-      const int qc = tri(cc);
-      for (int rr = 0; rr <= cc; rr++) {
-        prefetch_l2(gaddr(stb, fJ + gc[rr], ld8));
-        if (!sz) prefetch_l2(gaddr(stb, sJ + qc + rr, ld8));
-        prefetch_l2(gaddr(stb, tJ + sca[qc + rr], ld8));
-      }
-      prefetch_l2(gaddr(stb, fh + gat[SMM + I + cc], ld8));
-      if (!sz) prefetch_l2(gaddr(stb, sh + cc, ld8));
-      prefetch_l2(gaddr(stb, th + sca[SS + cc], ld8));
-    }
+    for (int cc = wid; cc < S; cc += NW) ks.template prefetch<4>(cc);
   }
-  mbar_wait(&mbar, 0);  // every staged row has landed
+  mbar_wait(&mbar, 0);  // every staged row has landed (async-proxy writes are visible after the wait)
   __syncthreads();
 
-  // ---- B1: U'U = J_II, right-looking, columns dealt to the warps, one barrier per pivot ----------
+  // ---- B1: U'U = J_II; afterwards every warp holds 1/U_kk in rinv --------------------------------
   bool nz = false;
   double rinv[I];
-  double logdet = 0.0;
-  int fail = 0;
-  if (lane_ok)  // "all zero" test on the original entries of this warp's columns (src/beliefupdates.jl:62-66)
-    for (int c = wid; c < I; c += NW)
-      for (int k = 0; k <= c; k++)
-        if (!(fabs(smt[(tri(c) + k) * TILE]) <= PGBP_EPS)) nz = true;
+  if constexpr (!COLPAR) {
+    if (wid == 0 && lane_ok) {
+      double logdet = 0.0;
+      int fail = 0;
 #pragma unroll
-  for (int k = 0; k < I; k++) {
-    double d = 1.0;
-    if (lane_ok) d = smt[pk(k, k) * TILE];  // final: every update of steps < k is behind the barrier
-    if (!(d > 0.0) && fail == 0) fail = k + 1;  // LAPACK potrf info (also NaN); reported below
-    if (wid == 0) logdet += log(d);
-    const double ri = 1.0 / sqrt(d);
-    rinv[k] = ri;
+      for (int c = 0; c < I; c++) {
+        double v[I];
+#pragma unroll
+        for (int k = 0; k <= c; k++) {
+          v[k] = smt[pk(k, c) * TILE];
+          if (!(fabs(v[k]) <= PGBP_EPS)) nz = true;
+        }
+#pragma unroll
+        for (int k = 0; k < c; k++) {
+          const double u = v[k] * rinv[k];
+          v[k] = u;
+          smt[pk(k, c) * TILE] = u;
+#pragma unroll
+          for (int r = k + 1; r <= c; r++) v[r] = nfma(r == c ? u : smt[pk(k, r) * TILE], u, v[r]);
+        }
+        const double d = v[c];
+        if (!(d > 0.0) && fail == 0) fail = c + 1;  // LAPACK potrf info (also NaN); reported below
+        logdet += log(d);
+        rinv[c] = 1.0 / sqrt(d);
+        smt[pk(c, c) * TILE] = rinv[c];
+      }
+      s_logdet[0] = logdet;
+      s_flag[TILE + tid] = fail;
+    }
+    __syncthreads();
     if (lane_ok) {
-      const int c0 = k + 1 + ((wid - (k + 1)) % NW + NW) % NW;  // first column > k owned by this warp
-      for (int c = c0; c < I; c += NW) {
-        const int tc = tri(c);
-        const double ukc = smt[(tc + k) * TILE] * ri;
-        // operands of 8 rows loaded before the first store: the compiler cannot move a shared-memory load above
-        // a store it cannot disambiguate, and one row per iteration exposed the full LDS latency every time
-        for (int r0 = k + 1; r0 <= c; r0 += 8) {
-          double ur[8], av[8];
 #pragma unroll
-          for (int u = 0; u < 8; u++) {
-            const int r = r0 + u;
-            if (r <= c) {
-              ur[u] = smt[(tri(r) + k) * TILE];
-              av[u] = smt[(tc + r) * TILE];
+      for (int k = 0; k < I; k++) rinv[k] = smt[pk(k, k) * TILE];
+    }
+  } else {
+    double logdet = 0.0;
+    int fail = 0;
+    if (lane_ok)  // "all zero" test on the original entries of this warp's columns (src/beliefupdates.jl:62-66)
+      for (int c = wid; c < I; c += NW)
+        for (int k = 0; k <= c; k++)
+          if (!(fabs(smt[(tri(c) + k) * TILE]) <= PGBP_EPS)) nz = true;
+#pragma unroll
+    for (int k = 0; k < I; k++) {
+      double d = 1.0;
+      if (lane_ok) d = smt[pk(k, k) * TILE];  // final: every update of steps < k is behind the barrier
+      if (!(d > 0.0) && fail == 0) fail = k + 1;  // LAPACK potrf info (also NaN); reported below
+      if (wid == 0) logdet += log(d);
+      const double ri = 1.0 / sqrt(d);
+      rinv[k] = ri;
+      if (lane_ok) {
+        const int c0 = k + 1 + ((wid - (k + 1)) % NW + NW) % NW;  // first column > k owned by this warp
+        for (int c = c0; c < I; c += NW) {
+          const int tc = tri(c);
+          const double ukc = smt[(tc + k) * TILE] * ri;
+          // operands of 8 rows loaded before the first store: the compiler cannot move a shared-memory load above
+          // a store it cannot disambiguate, and one row per iteration exposed the full LDS latency every time
+          for (int r0 = k + 1; r0 <= c; r0 += 8) {
+            double ur[8], av[8];
+#pragma unroll
+            for (int u = 0; u < 8; u++) {
+              const int r = r0 + u;
+              if (r <= c) {
+                ur[u] = smt[(tri(r) + k) * TILE];
+                av[u] = smt[(tc + r) * TILE];
+              }
+            }
+#pragma unroll
+            for (int u = 0; u < 8; u++) {
+              const int r = r0 + u;
+              if (r <= c) smt[(tc + r) * TILE] = nfma(ur[u] * ri, ukc, av[u]);
             }
           }
-#pragma unroll
-          for (int u = 0; u < 8; u++) {
-            const int r = r0 + u;
-            if (r <= c) smt[(tc + r) * TILE] = nfma(ur[u] * ri, ukc, av[u]);
-          }
         }
+      }
+      __syncthreads();
+    }
+    if (lane_ok) {  // scale the rows in place: U(k,c) = A(k,c) / sqrt(A(k,k))
+      for (int c = wid; c < I; c += NW) {
+        const int tc = tri(c);
+#pragma unroll
+        for (int k = 0; k < I; k++)
+          if (k < c) smt[(tc + k) * TILE] *= rinv[k];
+      }
+      if (wid == 0) {
+        s_logdet[0] = logdet;
+        s_flag[TILE + tid] = fail;
       }
     }
     __syncthreads();
   }
-  if (lane_ok) {  // scale the rows in place: U(k,c) = A(k,c) / sqrt(A(k,k)) (every warp keeps 1/U_kk in registers)
-    for (int c = wid; c < I; c += NW) {
-      const int tc = tri(c);
-#pragma unroll
-      for (int k = 0; k < I; k++)
-        if (k < c) smt[(tc + k) * TILE] *= rinv[k];
-    }
-    if (wid == 0) {
-      s_logdet[0] = logdet;
-      s_flag[TILE + tid] = fail;
-    }
-  }
-  __syncthreads();
 
   // ---- B2: Z = U^-T [J_IK | h_I], right-hand sides dealt to the warps ---------------------------
   if (lane_ok) {
@@ -1218,22 +896,22 @@ __global__ void __launch_bounds__(32 * NW, 1) k_message_smem_mwp(MsgArgs a) {
   }
   __syncthreads();
   bool nzall = false;
-  int failp = 0;
+  int fail = 0;
   if (lane_ok) {
 #pragma unroll
     for (int w = 0; w < NW; w++) nzall = nzall || s_flag[(2 + w) * TILE + tid] != 0;
-    failp = s_flag[TILE + tid];
+    fail = s_flag[TILE + tid];
   }
-  const bool dead = !active || (nzall && failp != 0);
+  const bool dead = !active || (nzall && fail != 0);
   if (lane_ok) {
     if (nzall) {
-      if (failp && active && wid == 0) status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, failp));
+      if (fail && active && wid == 0) status_fail(a.status, e, PGBP_STATUS(a.ref_base + md.ref, fail));
       if (wid == 0) g += 0.5 * ((double)I * PGBP_LOG2PI - s_logdet[0] + s_ww[0]);
     } else {  // "missing data" shortcut: message = (h_K, J_KK, g) unchanged
       for (int q = wid; q < nrhs * I; q += NW) Z[q * TILE] = 0.0;
     }
   }
-  __syncthreads();
+  __syncthreads();  // the last read of U (B2) is behind this barrier: phase C reads Z only
 
   // ---- C: stream the kept block, kept columns paired (j, S-1-j) and dealt to the warps ------------
   double maxJ = 0.0, maxh = 0.0;
@@ -1242,78 +920,11 @@ __global__ void __launch_bounds__(32 * NW, 1) k_message_smem_mwp(MsgArgs a) {
     for (int side = 0; side < 2; side++) {
       const int cc = side == 0 ? j : S - 1 - j;
       if (side == 1 && cc == j) break;
-      double zc[I];
-#pragma unroll
-      for (int i = 0; i < I; i++) zc[i] = Z[(cc * I + i) * TILE];
-      const uint16_t* gc = gat + tri(I + cc) + I;
-      const int qc = tri(cc);
-      for (int r0 = 0; r0 <= cc; r0 += PGBP_CHUNK) {
-        double jo[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-        double* ta[PGBP_CHUNK];
-#pragma unroll
-        for (int u = 0; u < PGBP_CHUNK; u++) {
-          const int rr = r0 + u;
-          if (rr <= cc) {
-            ta[u] = gaddr(stb, tJ + sca[qc + rr], ld8);
-            jo[u] = *gaddr(stb, fJ + gc[rr], ld8);
-            so[u] = sz ? 0.0 : *gaddr(stb, sJ + qc + rr, ld8);
-            to[u] = *ta[u];
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < PGBP_CHUNK; u++) {
-          const int rr = r0 + u;
-          if (rr <= cc) {
-            double nv = jo[u];
-            const double* zr = Z + rr * I * TILE;
-#pragma unroll
-            for (int i = 0; i < I; i++) nv = nfma(zr[i * TILE], zc[i], nv);
-            const double d = nv - so[u];
-            *gaddr(stb, sJ + qc + rr, ld8) = nv;
-            *ta[u] = to[u] + d;
-            if (rsb) *gaddr(rsb, rJ + qc + rr, ld8) = d;
-            absmax(maxJ, d);
-          }
-        }
-      }
+      ks.column(cc, maxJ);
     }
   }
-  if (!dead) {  // h part: chunks of kept entries dealt to the warps, last warp first
-    double w[I];
-#pragma unroll
-    for (int i = 0; i < I; i++) w[i] = Z[(S * I + i) * TILE];
-    const uint16_t* gh = gat + SMM + I;
-    for (int k0 = (NW - 1 - wid) * PGBP_CHUNK; k0 < S; k0 += NW * PGBP_CHUNK) {
-      double ho[PGBP_CHUNK], so[PGBP_CHUNK], to[PGBP_CHUNK];
-      double* ta[PGBP_CHUNK];
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          ta[u] = gaddr(stb, th + sca[SS + k], ld8);
-          ho[u] = *gaddr(stb, fh + gh[k], ld8);
-          so[u] = sz ? 0.0 : *gaddr(stb, sh + k, ld8);
-          to[u] = *ta[u];
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < PGBP_CHUNK; u++) {
-        const int k = k0 + u;
-        if (k < S) {
-          double nv = ho[u];
-          const double* zr = Z + k * I * TILE;
-#pragma unroll
-          for (int i = 0; i < I; i++) nv = nfma(zr[i * TILE], w[i], nv);
-          const double d = nv - so[u];
-          *gaddr(stb, sh + k, ld8) = nv;
-          *ta[u] = to[u] + d;
-          if (rsb) *gaddr(rsb, rh + k, ld8) = d;
-          absmax(maxh, d);
-        }
-      }
-    }
-  }
-  __syncthreads();  // phase C of every warp is done with Z ... and nobody reads U any more: reuse its rows
+  // h part: chunks of kept entries dealt to the warps, last warp first (it has the lightest J share)
+  if (!dead) ks.hpart((NW - 1 - wid) * PGBP_CHUNK, NW * PGBP_CHUNK, maxh);
   if (lane_ok) {
     s_redJ[wid * TILE] = maxJ;
     s_redh[wid * TILE] = maxh;
@@ -1327,8 +938,8 @@ __global__ void __launch_bounds__(32 * NW, 1) k_message_smem_mwp(MsgArgs a) {
       if (xj > mJ || xj != xj) mJ = xj;
       if (xh > mh || xh != xh) mh = xh;
     }
-    *gaddr(stb, (uint32_t)md.sg, ld8) = g;
-    *gaddr(stb, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
+    *slot_ptr(stb, (uint32_t)md.sg, ld8) = g;
+    *slot_ptr(stb, (uint32_t)md.tg, ld8) = tg_old + (g - sg_old);
     store_flag(a, md.dmsg, e, S, mJ, mh);
   }
 }

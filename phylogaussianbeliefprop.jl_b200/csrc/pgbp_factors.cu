@@ -667,10 +667,6 @@ struct AssignOU {
   }
 };
 
-PGBP_HD double* kaddr(char* base, uint32_t slot, uint32_t ld8) {
-  return (double*)(base + (uint64_t)slot * (uint64_t)ld8);  // one IMAD.WIDE.U32
-}
-
 template <int P, bool SH = false>
 struct AssignFast {
   AssignBody gen;
@@ -816,7 +812,7 @@ struct AssignFast {
 #pragma unroll
             for (int cc = 0; cc < P; cc++) s += PGBP_JU(r, cc) * z[cc];
             quad += z[r] * s;
-            double* dh = kaddr(stb, (uint32_t)(hs + pa + r), ld8);
+            double* dh = slot_ptr(stb, (uint32_t)(hs + pa + r), ld8);
             if (first) *dh = 0.0 - (-1.0) * s;
             else *dh = *dh - (-1.0) * s;
 #if defined(__CUDA_ARCH__)
@@ -842,7 +838,7 @@ struct AssignFast {
             if (!((fh >> a) & 1)) continue;
             const int pa = F.mem_pos[k0 + a];
 #pragma unroll
-            for (int t = 0; t < P; t++) *kaddr(stb, (uint32_t)(hs + pa + t), ld8) = 0.0;
+            for (int t = 0; t < P; t++) *slot_ptr(stb, (uint32_t)(hs + pa + t), ld8) = 0.0;
           }
           continue;
         }
@@ -888,13 +884,13 @@ struct AssignFast {
         const double ca = a == 0 ? 1.0 : (nm == 2 ? -1.0 : -F.mem_gamma[k0 + a]);
         if ((fh >> a) & 1) {
 #pragma unroll
-          for (int t = 0; t < P; t++) *kaddr(stb, (uint32_t)(hs + pa + t), ld8) = anyfixed ? 0.0 - ca * jz[t] : 0.0;
+          for (int t = 0; t < P; t++) *slot_ptr(stb, (uint32_t)(hs + pa + t), ld8) = anyfixed ? 0.0 - ca * jz[t] : 0.0;
         } else if (anyfixed) {
           double oldh[P];
 #pragma unroll
-          for (int t = 0; t < P; t++) oldh[t] = *kaddr(stb, (uint32_t)(hs + pa + t), ld8);
+          for (int t = 0; t < P; t++) oldh[t] = *slot_ptr(stb, (uint32_t)(hs + pa + t), ld8);
 #pragma unroll
-          for (int t = 0; t < P; t++) *kaddr(stb, (uint32_t)(hs + pa + t), ld8) = oldh[t] - ca * jz[t];
+          for (int t = 0; t < P; t++) *slot_ptr(stb, (uint32_t)(hs + pa + t), ld8) = oldh[t] - ca * jz[t];
         }
         for (int bq = a; lead && bq < nm; bq++) {
           const int pb = F.mem_pos[k0 + bq];
@@ -909,7 +905,7 @@ struct AssignFast {
               const uint32_t colslot = (uint32_t)js + (uint32_t)tri(pb + tb) + (uint32_t)pa;  // pk(pa + ta, pb + tb)
 #pragma unroll
               for (int ta = 0; ta < P; ta++)
-                if (!diag || ta <= tb) *kaddr(stb, colslot + ta, ld8) = cab * PGBP_JU(ta, tb);
+                if (!diag || ta <= tb) *slot_ptr(stb, colslot + ta, ld8) = cab * PGBP_JU(ta, tb);
             }
           } else {
             // read-modify-write of a block another family wrote first: the P loads of a column are issued
@@ -921,10 +917,10 @@ struct AssignFast {
               double old[P];
 #pragma unroll
               for (int ta = 0; ta < P; ta++)
-                if (!diag || ta <= tb) old[ta] = *kaddr(stb, colslot + ta, ld8);
+                if (!diag || ta <= tb) old[ta] = *slot_ptr(stb, colslot + ta, ld8);
 #pragma unroll
               for (int ta = 0; ta < P; ta++)
-                if (!diag || ta <= tb) *kaddr(stb, colslot + ta, ld8) = old[ta] + cab * PGBP_JU(ta, tb);
+                if (!diag || ta <= tb) *slot_ptr(stb, colslot + ta, ld8) = old[ta] + cab * PGBP_JU(ta, tb);
             }
           }
         }

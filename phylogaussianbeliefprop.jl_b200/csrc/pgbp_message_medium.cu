@@ -52,14 +52,9 @@ static int launch_smem(pgbp_batch* b, const MsgArgs& a, int nmsg, int I, int S) 
 }
 
 
-// multi-warp shared-memory kernel (large I): NW warps per tile of 32 elements
+// multi-warp shared-memory kernel: NW warps per tile of TILE elements, column-parallel Cholesky if COLPAR
 #define PGBP_SMEM_MW_LIMIT (225 * 1024)
-static size_t mw_bytes(int I, int S, int NW) {  // == smem_mw_block_bytes (pgbp_coop.cuh, device build only)
-  const int M = I + S;
-  return sizeof(double) * 32 * (size_t)(I * (I + 1) / 2 + I * S + I + 2) + sizeof(int32_t) * 32 * (size_t)(2 + NW) +
-         sizeof(uint16_t) * (size_t)(M * (M + 1) / 2 + M + S * (S + 1) / 2 + S + 4);
-}
-template <int I, int NW, int MINB = (NW <= 4 ? 2 : 1)>
+template <int I, int NW, int TILE, bool COLPAR>
 static int launch_smem_mw(pgbp_batch* b, const MsgArgs& a, int nmsg, int S) {
 #ifdef PGBP_HOST_EMUL
   (void)S;
@@ -68,39 +63,14 @@ static int launch_smem_mw(pgbp_batch* b, const MsgArgs& a, int nmsg, int S) {
 #else
   static AttrOnce attr_done;  // per instantiation and device
   if (attr_done.first()) {
-    PGBP_CUDA(cudaFuncSetAttribute((const void*)k_message_smem_mw<I, NW, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, PGBP_SMEM_MW_LIMIT));
-  }
-  if (a.ld * 8 >= ((int64_t)1 << 32)) PGBP_FAIL(PGBP_ESTATE, "batch too large for 32-bit row pitch");
-  dim3 grid((unsigned)((a.B - a.e0 + 31) / 32), (unsigned)nmsg), block(32, NW);
-  k_message_smem_mw<I, NW, MINB><<<grid, block, mw_bytes(I, S, NW), b->stream>>>(a);
-#endif
-  b->launches++;
-  return check_launch("k_message_smem_mw");
-}
-
-// multi-warp kernel with the column-parallel Cholesky, tiles of TILE <= 32 elements (C5's (32,16) messages)
-static size_t mwp_bytes(int I, int S, int NW, int TILE) {
-  const int M = I + S;
-  return sizeof(double) * TILE * (size_t)(I * (I + 1) / 2 + I * S + I + 2) + sizeof(int32_t) * TILE * (size_t)(2 + NW) +
-         sizeof(uint16_t) * (size_t)(M * (M + 1) / 2 + M + S * (S + 1) / 2 + S + 4) + 16;
-}
-template <int I, int NW, int TILE>
-static int launch_smem_mwp(pgbp_batch* b, const MsgArgs& a, int nmsg, int S) {
-#ifdef PGBP_HOST_EMUL
-  (void)S;
-  for (int m = 0; m < nmsg; m++)
-    for (int64_t e = a.e0; e < a.B; e++) message_thread_rt<PGBP_MAX_DIM>(a, m, e);
-#else
-  static AttrOnce attr_done;
-  if (attr_done.first()) {
-    PGBP_CUDA(cudaFuncSetAttribute((const void*)k_message_smem_mwp<I, NW, TILE>, cudaFuncAttributeMaxDynamicSharedMemorySize, PGBP_SMEM_MW_LIMIT));
+    PGBP_CUDA(cudaFuncSetAttribute((const void*)k_message_smem_mw<I, NW, TILE, COLPAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, PGBP_SMEM_MW_LIMIT));
   }
   if (a.ld * 8 >= ((int64_t)1 << 32)) PGBP_FAIL(PGBP_ESTATE, "batch too large for 32-bit row pitch");
   dim3 grid((unsigned)((a.B - a.e0 + TILE - 1) / TILE), (unsigned)nmsg), block(32, NW);
-  k_message_smem_mwp<I, NW, TILE><<<grid, block, mwp_bytes(I, S, NW, TILE), b->stream>>>(a);
+  k_message_smem_mw<I, NW, TILE, COLPAR><<<grid, block, smem_tile_bytes(I, S, NW, TILE), b->stream>>>(a);
 #endif
   b->launches++;
-  return check_launch("k_message_smem_mwp");
+  return check_launch("k_message_smem_mw");
 }
 
 // narrow tiles (TILE = 24 or 16 elements per single-warp block) for I <= 32 when the 32-lane factor does not fit
@@ -115,6 +85,7 @@ static int launch_smem_tile(pgbp_batch* b, const MsgArgs& a, int nmsg, int I, in
   if (attr_done.first()) {
     PGBP_CUDA(cudaFuncSetAttribute((const void*)k_message_smem_rt<32, TILE>, cudaFuncAttributeMaxDynamicSharedMemorySize, PGBP_SMEM_MW_LIMIT));
   }
+  if (a.ld * 8 >= ((int64_t)1 << 32)) PGBP_FAIL(PGBP_ESTATE, "batch too large for 32-bit row pitch");
   const size_t bytes = sizeof(double) * TILE * (size_t)(I * (I + 1) / 2 + I * S + I);
   dim3 grid((unsigned)((a.B - a.e0 + TILE - 1) / TILE), (unsigned)nmsg);
   k_message_smem_rt<32, TILE><<<grid, 32, bytes, b->stream>>>(a);
@@ -129,7 +100,7 @@ int launch_medium(pgbp_batch* b, const MsgArgs& a, int n, int I, int S) {
   const int mode = b->coop_mode;
   const bool fits = I <= 32 && sizeof(double) * 32 * (size_t)(I * (I + 1) / 2 + I * S + I) + 4 * (size_t)(M * (M + 3) / 2 + S * (S + 3) / 2 + 2) <= PGBP_SMEM_LIMIT;
   // large I (C5: p = 16): one or two single-warp tiles per SM are latency-bound; share the tile among warps
-  const bool fits_mw = I >= 12 && I <= 16 && mw_bytes(I, S, 8) <= PGBP_SMEM_MW_LIMIT;
+  const bool fits_mw = I >= 12 && I <= 16 && smem_tile_bytes(I, S, 8, 32) <= PGBP_SMEM_MW_LIMIT;
   // (measured on C4: the multi-warp form for I = 8 -- 4 warps x 4 tiles or 2 warps x 8 tiles per SM at 128
   // registers -- is SLOWER than the single-warp kernel with its unrolled S <= 8 variant: 70.6 / 68.5 ms per
   // step against 60.3 ms; it stays reserved for I >= 12.)
@@ -137,7 +108,7 @@ int launch_medium(pgbp_batch* b, const MsgArgs& a, int n, int I, int S) {
     switch (I) {
     // two tiles per SM with 4 warps each when they fit (233,472 bytes per SM, 1 KB reserved per block), else
     // one tile with 8 warps
-#define PGBP_MW_CASE(I_) case I_: rc = (mode == 2 || 2 * (mw_bytes(I, S, 4) + 1024) <= 233472) ? launch_smem_mw<I_, 4>(b, a, n, S) : launch_smem_mw<I_, 8>(b, a, n, S); break;
+#define PGBP_MW_CASE(I_) case I_: rc = (mode == 2 || 2 * (smem_tile_bytes(I, S, 4, 32) + 1024) <= 233472) ? launch_smem_mw<I_, 4, 32, false>(b, a, n, S) : launch_smem_mw<I_, 8, 32, false>(b, a, n, S); break;
       PGBP_MW_CASE(12) PGBP_MW_CASE(13) PGBP_MW_CASE(14) PGBP_MW_CASE(15) PGBP_MW_CASE(16)
 #undef PGBP_MW_CASE
     }
@@ -158,8 +129,8 @@ int launch_medium(pgbp_batch* b, const MsgArgs& a, int n, int I, int S) {
     if (mode == 1) {  // single-warp narrow tiles: measured 880 ms per C5 step (one warp per SM), kept for comparison
       if (sizeof(double) * 24 * (size_t)(I * (I + 1) / 2 + I * S + I) <= PGBP_SMEM_MW_LIMIT) rc = launch_smem_tile<24>(b, a, n, I, S);
       else rc = launch_smem_tile<16>(b, a, n, I, S);
-    } else if (I == 32 && mwp_bytes(I, S, 8, 24) <= PGBP_SMEM_MW_LIMIT) {
-      rc = launch_smem_mwp<32, 8, 24>(b, a, n, S);
+    } else if (I == 32 && smem_tile_bytes(I, S, 8, 24) <= PGBP_SMEM_MW_LIMIT) {
+      rc = launch_smem_mw<32, 8, 24, true>(b, a, n, S);
     } else if (M <= PGBP_COOP_MAX) {
       rc = launch_coop<48, 16>(b, a, n);
     } else {

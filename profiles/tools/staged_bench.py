@@ -15,6 +15,8 @@ here.  The first --lib is the baseline.  Written to DIR:
   default_<lib>.json        (--default-runs) the default bench.py run: other_workloads block and CPU check
   summary.json              per workload: medians, spreads, ratios against the baseline and whether each median lies
                             within the baseline's min..max; byte-identity of every dump
+  kernels_<w>_<lib>.txt     (--profiles w:K,...) torch.profiler per-kernel device time of bench.py --workload w --steps K
+                            --warmup 1, set-up included, own process per library
 Run `--profile-c2 FILE` alone to profile one C2 step with the library PGBP_B200_LIB selects.
 """
 import argparse
@@ -76,6 +78,23 @@ def profile_c2(path):
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         step()
         torch.cuda.synchronize()
+    write_kernel_table(prof, path, "kernel device time of one C2 step (B = %d)" % B, {"B": B})
+    assert np.isfinite(norm[:B].cpu().numpy()).all()
+
+
+def profile_workload(w, steps, path):
+    """bench.py --workload w --steps steps --warmup 1 (set-up included) under torch.profiler."""
+    from torch.profiler import ProfilerActivity, profile
+
+    import bench
+    sys.argv = ["bench.py", "--workload", w, "--steps", str(steps), "--warmup", "1", "--no-others", "--no-cpu"]
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        bench.main()
+    write_kernel_table(prof, path, "kernel device time of bench.py --workload %s --steps %d --warmup 1 (set-up, warm-up "
+                       "and timed steps)" % (w, steps), {"workload": w, "steps": steps})
+
+
+def write_kernel_table(prof, path, title, extra):
     rows = {}
     for ev in prof.key_averages():
         us = getattr(ev, "self_device_time_total", 0.0)
@@ -83,15 +102,16 @@ def profile_c2(path):
             rows[ev.key] = [ev.count, us]
     total = sum(r[1] for r in rows.values())
     table = sorted(([n, c, us] for n, (c, us) in rows.items()), key=lambda x: -x[2])
+    lib = os.environ.get("PGBP_B200_LIB")
+    lib = os.path.relpath(lib, ROOT) if lib else "default"
     with open(path, "w") as f:
-        f.write("library: %s\nkernel device time of one C2 step (B = %d), sum %.1f us\n" % (os.environ.get("PGBP_B200_LIB", "default"), B, total))
+        f.write("library: %s\n%s, sum %.1f us\n" % (lib, title, total))
         f.write("%10s %6s %7s  %s\n" % ("us", "calls", "share", "kernel"))
         for n, c, us in table:
             f.write("%10.1f %6d %6.1f%%  %s\n" % (us, c, 100.0 * us / total if total else 0.0, n))
-    json.dump({"library": os.environ.get("PGBP_B200_LIB", "default"), "B": B, "sum_us": total,
-               "kernels": [{"name": n, "calls": c, "us": us} for n, c, us in table]},
+    json.dump(dict(extra, library=lib, sum_us=total,
+                   kernels=[{"name": n, "calls": c, "us": us} for n, c, us in table]),
               open(os.path.splitext(path)[0] + ".json", "w"), indent=1)
-    assert np.isfinite(norm[:B].cpu().numpy()).all()
 
 
 def main():
@@ -104,9 +124,16 @@ def main():
     ap.add_argument("--dumps", default="c2,c4,c3", help="workloads whose outputs are dumped and compared")
     ap.add_argument("--no-profile", action="store_true", help="skip the per-kernel profile of one C2 step")
     ap.add_argument("--profile-c2")
+    ap.add_argument("--profile-workload", nargs=3, metavar=("W", "STEPS", "FILE"))
+    ap.add_argument("--profiles", default="", help="name:steps, comma-separated: per-kernel table of each workload and "
+                    "library, own process each (kernels_<w>_<lib>.txt)")
     args = ap.parse_args()
     if args.profile_c2:
         profile_c2(args.profile_c2)
+        return
+    if args.profile_workload:
+        w, k, f = args.profile_workload
+        profile_workload(w, int(k), f)
         return
     libs = [tuple(x.split("=", 1)) for x in args.lib]
     libs = [(n, os.path.abspath(p)) for n, p in libs]
@@ -146,7 +173,7 @@ def main():
                 s["median_over_baseline"] = s["median"] / b["median"]
                 s["min_over_baseline_max"] = s["min"] / b["max"]
                 s["median_within_baseline_spread"] = b["min"] <= s["median"] <= b["max"]
-    steps = {"c2": 20, "c4": 3, "c3": 2, "c3l": 2, "c2s": 20, "c5s": 1}
+    steps = {"c2": 20, "c4": 3, "c3": 2, "c3l": 2, "c2s": 20, "c5": 1, "c5s": 1}
     for w in filter(None, args.dumps.split(",")):
         st = steps[w]
         for n, p in libs:
@@ -166,6 +193,10 @@ def main():
             break
         f = os.path.join(out, "kernels_%s.txt" % n)
         run([py, os.path.abspath(__file__), "--profile-c2", f], p, f + ".log", f + ".err")
+    for w, k in (x.split(":") for x in args.profiles.split(",") if x):
+        for n, p in libs:
+            f = os.path.join(out, "kernels_%s_%s.txt" % (w, n))
+            run([py, os.path.abspath(__file__), "--profile-workload", w, k, f], p, f + ".log", f + ".err", timeout=1800)
     if args.default_runs:
         for n, p in libs:
             f = os.path.join(out, "default_%s.json" % n)
